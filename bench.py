@@ -12,6 +12,12 @@ number (1M strings per GPU) is measured in the same run and reported under the k
   python bench.py [--gpus N] [--steps K] [--warmup W]          our arm (one JSON line on stdout)
   python bench.py --impl reference ...                           the reference's CPU implementation
   torchrun ... bench.py --gpus N ...                             one rank per GPU
+  python bench.py ... --dump-outputs DIR                         also write what the last timed step returned, DIR/<name>.npy
+
+`--dump-outputs DIR` writes, in float64, the log-likelihood (loglik.npy), the gradient (grad.npy) and log q of every string
+in corpus order (logq.npy, the ranks' strings one after another) that the timed evaluations returned in their last step.
+The inputs are seeded, so two builds run with the same arguments can be compared output for output.  Above DUMP_BYTES in
+all, logq.npy holds a fixed, seeded sample of the strings, in corpus order.
 
 `value`  : kernel-resident throughput -- x already on the device, K evaluations timed with CUDA
            events on the library's own stream, max over ranks.
@@ -38,6 +44,7 @@ METRIC = "fwd-bwd+grad symbols/sec"
 UNIT = "symbols/s"
 C4 = dict(n_states=256, n_sym=64, n_succ=8, n_emis=4, seed=1234)
 C5 = dict(n_states=4096, n_sym=256, n_succ=64, n_emis=16, seed=4321)    # config 5 (dense, CTA-per-string kernel)
+DUMP_BYTES = 64 * 10**6                   # --dump-outputs: at most this much in all, .npy headers included
 
 
 def peaks():
@@ -204,6 +211,16 @@ def _trim_all_used(used):
     return trimmed, n
 
 
+def dump_outputs(out_dir, loglik, grad, logq):
+    grad, logq = np.asarray(grad, dtype=np.float64), np.asarray(logq, dtype=np.float64)
+    room = (DUMP_BYTES - 3 * 256 - 8 - grad.nbytes) // 8
+    if len(logq) > room:
+        logq = logq[np.sort(np.random.RandomState(0).choice(len(logq), room, replace=False))]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in (("loglik", np.array([loglik], dtype=np.float64)), ("grad", grad), ("logq", logq)):
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def measure(dev, x, args, barrier, want_e2e=True):
     """Device-timed steps (one event pair per evaluation, L2 flushed between evaluations), then the host-buffer call."""
     dev.upload_x(x)
@@ -350,6 +367,11 @@ def run_ours(args, rank, world, local):
     lq_ms = lq_s * 1e3 / min(args.steps, 5)
     barrier()
     assert ll_q == M["ll"] and np.array_equal(g_q, M["grad"])
+    logq_all = lq
+    if args.dump_outputs and world > 1:
+        parts = [None] * world
+        dist.all_gather_object(parts, lq)
+        logq_all = np.concatenate(parts)
     # self check on every run, any number of ranks: the log-likelihood never went through the per-string values, and with
     # N > 1 it went through the exchange over peer memory -- compare it with sum_s p_s log q_s over all ranks
     ll_strings = all_sum([float(np.dot(w / total_w, lq))])[0]
@@ -491,6 +513,8 @@ def run_ours(args, rank, world, local):
         }
         if world == 1 and not args.no_cpu and args.config == "c4":
             line["cpu_baseline"] = cpu_baseline(model)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, M["ll"], M["grad"], logq_all)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
@@ -518,7 +542,11 @@ def main():
     ap.add_argument("--ref-strings", type=int, default=8000, help="--impl reference: strings in the bounded sample")
     ap.add_argument("--cpu-strings", type=int, default=20000)
     ap.add_argument("--cpu-port", action="store_true", help="--impl reference: time the CPU port instead of oracle/_ref")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write loglik, grad and log q per string of the last timed step as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs: only the GPU arm (--impl ours) has outputs to write")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank, world, local = dist_env()
     if world == 1 and args.gpus > 1 and args.impl == "ours":

@@ -9,7 +9,7 @@ import numpy as np
 import pytest
 
 import wfsa_b200 as W
-from helpers import all_cases, fnum, key
+from helpers import all_cases, fnum, key, load_cases
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -116,21 +116,24 @@ def test_descriptor_validation():
 @pytest.mark.parametrize("fsa,corpus", [("test3.wfsa", "test.corpus"), ("talk.wfsa", "talk.corpus"), ("test5.wfsa", "test5.corpus"),
                                         ("test.list.wfsa", "test.corpus"), ("test.loop.wfsa", "test.corpus")])
 @pytest.mark.parametrize("order", ["0", "1"])
-def test_path_listing_matches_reference_binary(fsa, corpus, order):
+def test_path_listing_matches_reference_binary(fsa, corpus, order, tmp_path):
     """-pr lists every accepting path of every corpus string (src/main.cpp:178-203).  The listing happens before the
-    device is touched, so it can be compared here, without a GPU, against the unmodified reference build
-    (oracle/_ref/wfsa_ref) -- as a set of lines: the reference's order follows its hash-map iteration."""
-    import os
+    device is touched, so it can be compared here, without a GPU, against the reference binary's listing of the same
+    data fixture (tests/golden/path_listing.json) -- as a set of lines: the reference's order follows its hash-map
+    iteration -- and, string by string, against the reference's path counts (tests/golden/fixtures.json)."""
     import subprocess
-    ref = os.path.join(ROOT, "oracle", "_ref", "wfsa_ref")
-    data = "/root/reference/data"
+    from collections import Counter
+    name = fsa + "+" + corpus
+    case = [c for c in load_cases("fixtures") if c["name"] == name][0]
+    (tmp_path / fsa).write_bytes(case["fsa_text"].encode())
+    (tmp_path / corpus).write_bytes(case["corpus_text"].encode())
     ours = os.path.join(ROOT, "w-fsa_b200", "_build", "wfsa")
-    if not (os.path.exists(ref) and os.path.isdir(data)):
-        pytest.skip("needs the reference build and its data (build container only)")
-    args = ["-a", os.path.join(data, fsa), "-c", os.path.join(data, corpus), "-pr", "-r", order, "-e", "0", "-s"]
-    want = sorted(ln for ln in subprocess.run([ref] + args, capture_output=True, text=True).stderr.splitlines() if " -> " in ln)
+    args = ["-a", str(tmp_path / fsa), "-c", str(tmp_path / corpus), "-pr", "-r", order, "-e", "0", "-s"]
     got = sorted(ln for ln in subprocess.run([ours] + args, capture_output=True, text=True).stderr.splitlines() if " -> " in ln)
+    want = load_cases("path_listing")[name]
     assert want and got == want
+    paths = Counter(ln.split(": ", 1)[0] for ln in got)
+    assert {w["word"]: paths[w["word"]] for w in case["corpus"]} == {w["word"]: w["paths"] for w in case["corpus"]}
 
 
 def test_cli_gpus_option_without_a_device(tmp_path):

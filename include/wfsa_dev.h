@@ -195,6 +195,13 @@ typedef struct {
        instances / of the distinct types (what one evaluation walks), host milliseconds of the compile */
     int64_t seg_types, seg_region_instances, seg_region_edges, seg_type_edges;
     double  seg_host_ms;
+    /* schedule of the region phase of k_eval6 (segmented kernel 6, 0 otherwise), as the next launch would run it:
+       big DAG groups (dealt out statically, big group b to warp b / grid of CTA b % grid); 1 if the CTAs that own a big group
+       are dedicated to it (the environment as it is now); staging areas per CTA and word rows each (0 slots: every big group is
+       streamed from HBM); rows of the longest big group; big groups the two-warp chain takes (at most one per CTA, when
+       e6_big_groups <= grid, the group is staged and at least two staging areas exist) */
+    int64_t e6_big_groups;
+    int32_t e6_big_dedicate, e6_big_slots, e6_big_rows, e6_max_big_rows, e6_two_warp_eligible;
 } wfsa_dev_info;
 int wfsa_dev_get_info(wfsa_dev* h, wfsa_dev_info* info);
 
@@ -219,9 +226,12 @@ int wfsa_lattice_stats(const wfsa_fsa_desc* fsa, const wfsa_corpus_desc* corpus,
  * (1..16), plus 64 to keep every region in DAG form (no path lists).
  * which: 0 rwords(u32) 1 rgoff(i64) 2 rgrows(i32) 3 typeW(f64) 4 swords(u32) 5 sgoff(i64) 6 sgref(i32)
  *        7 ksid(i32) 8 kp(f64) 9 overflow(i32) 10 rejected(i32) 11 const_acc(i64)
- *        12 stats(i64): types, region instances, instance edges, type edges, bridges, strings, host microseconds
+ *        12 stats(i64): types, region instances, instance edges, type edges, bridges, strings, host microseconds,
+ *           path blocks omitted (1: a region type has more than 2^20 paths, so arrays 13-19 describe zero blocks)
  *        13 path_off(i64) 14 col_off(i64) 15 val_off(i64) 16 cols(i32) 17 counts(f64) 18 p(f64) 19 type slot(i32): the path blocks
- *           wfsa_dev_hessian derives from the region types (layout of wfsa_path_blocks, p = weight of the type) */
+ *           wfsa_dev_hessian derives from the region types (layout of wfsa_path_blocks, p = weight of the type).  The
+ *           evaluation does not need them: a shard whose blocks cannot be built still compiles (wfsa_dev_hessian of such
+ *           a shard returns WFSA_ERR_LIMIT). */
 typedef struct wfsa_segmented wfsa_segmented;
 int wfsa_segmented_compile(const wfsa_fsa_desc* fsa, const wfsa_corpus_desc* corpus, const int32_t* trimmed,
                            int32_t n_slots, double fx_scale, wfsa_segmented** out);

@@ -214,6 +214,7 @@ def test_config4_shape_bridges_regions_and_type_merging():
     st = seg["stats"]
     assert len(seg["overflow"]) == 0 and len(handled) == 600
     assert st[4] > 0 and st[1] > st[0] > 0, "expected bridges and merged region types"
+    assert st[7] == 0 and len(seg["hb_p"]) > 0, "the H_f path blocks fit"
     assert interpret.counts[0] > 0 and interpret.counts[1] > 0, "expected regions in path form and in DAG form"
     # DAG form only (bit 6 of n_slots): the same numbers, small and big DAG regions
     seg_d, ee_d, _, _, handled_d = check(low, trimmed, x, n_slots=16 | 64)
@@ -238,6 +239,24 @@ def test_trimmed_arcs_are_removed_from_segments():
     seg, _, _, olq, handled = check(low, trimmed, x)
     for s in range(80):
         assert (s in handled) == bool(np.isfinite(olq[s]))
+
+
+def test_region_types_beyond_the_path_limit_of_the_hessian_blocks():
+    """Eight emissions per state: some region types have more than 2^20 paths, too many for the H_f path blocks.  The
+    evaluation does not need those blocks, so the shard still compiles: the region arrays as always, zero path blocks and
+    the flag in stats[7].  The region arrays still reproduce the oracle's log q of every string (check)."""
+    model = synth.make_model(256, 64, 8, 8, seed=1)
+    low = model.lowered()
+    offs, toks, w = model.corpus(5000, 32, 128, seed=2)
+    low.set_tokens(offs, toks, w / w.sum())
+    zt, ze = np.zeros(low.n_trans), np.zeros(low.n_emis)
+    _, _, ee0 = O.dp_eval(low, zt, ze, nthreads=O.max_threads())
+    trimmed, n, _ = O.trim(low, ee0 > 0)
+    x = np.random.RandomState(3).normal(-1.0, 0.3, size=n)
+    seg, ee, oee, olq, handled = check(low, trimmed, x)
+    assert seg["stats"][7] == 1 and len(handled) > 4000
+    assert seg["hb_path_off"].tolist() == [0] and seg["hb_col_off"].tolist() == [0] and seg["hb_val_off"].tolist() == [0]
+    assert len(seg["hb_cols"]) == len(seg["hb_counts"]) == len(seg["hb_p"]) == len(seg["hb_slot"]) == 0
 
 
 def _hessian_from_blocks(seg, x, n):

@@ -451,6 +451,9 @@ static int setup_kl(wfsa_dev* h)
         smem = (awg ? 0 : ((size_t)h->larcs.n_arcs + 1) * 8) + (size_t)nt * K * 8;
     }
     h->kl_K = K; h->kl_block = nt; h->kl_grid = h->sm_count; h->kl_smem = smem;
+    // experiment / test knob: a smaller persistent grid, so that a small shard reaches the schedules of a large one (more big DAG
+    // groups than CTAs, several per warp).  Read here, before the per-warp x stacks are sized from kl_grid.
+    if (const char* g = getenv("WFSA_E6_GRID")) h->kl_grid = std::min(h->sm_count, std::max(1, atoi(g)));
     h->kl_bridges = !(h->opt.reserved & 4);
     const LatticeArcs& A = h->larcs;
     CK(h->d_kl_arc_tid.upload(A.arc_tid, h->stream)); CK(h->d_kl_arc_eid.upload(A.arc_eid, h->stream));
@@ -872,6 +875,13 @@ static void launch_main(wfsa_dev* h, int kernel, int mode, const CorpusD& C, con
     }
 }
 
+// CTAs that own a big DAG group wait for it before they take regular groups: few big groups (up to grid / 4 by default)
+static int eval6_big_dedicate(const wfsa_dev* h)
+{
+    const int ded_div = getenv("WFSA_E6_DED_DIV") ? std::max(1, atoi(getenv("WFSA_E6_DED_DIV"))) : 4;
+    return (h->kr_big_groups > 0 && h->kr_big_groups * ded_div <= h->kl_grid && !getenv("WFSA_E6_NO_DEDICATE")) ? 1 : 0;
+}
+
 // The whole evaluation of the segmented path in one launch (kernels_eval6.cuh).  All launch parameters are constant per
 // parameter map: x, the scale of loglik and the epoch are read from device memory.
 static void fill_eval6_params(wfsa_dev* h, Eval6Params& P)
@@ -895,8 +905,7 @@ static void fill_eval6_params(wfsa_dev* h, Eval6Params& P)
     P.stamps = h->d_e6stamps.p;
     P.debug = getenv("WFSA_E6_DEBUG") ? atoi(getenv("WFSA_E6_DEBUG")) : 0;
     P.pool_slots = h->kl_K; P.big_slots = h->e6_big_slots; P.big_rows = h->e6_big_rows;
-    const int ded_div = getenv("WFSA_E6_DED_DIV") ? std::max(1, atoi(getenv("WFSA_E6_DED_DIV"))) : 4;      // dedicate CTAs up to grid / 4 big groups
-    P.big_dedicate = (h->kr_big_groups > 0 && h->kr_big_groups * ded_div <= h->kl_grid && !getenv("WFSA_E6_NO_DEDICATE")) ? 1 : 0;
+    P.big_dedicate = eval6_big_dedicate(h);
     // dedicated CTAs: the shard is small (a few regular groups per warp): everything static among the free CTAs; one global
     // ticket counter for ~3.5 k groups costs ~3 ns per ticket in the L2, i.e. ~10 us of a ~14 us phase
     if (P.big_dedicate && !getenv("WFSA_E6_STATIC")) P.static_pct = 100;
@@ -2267,15 +2276,17 @@ extern "C" int wfsa_segmented_compile(const wfsa_fsa_desc* fd, const wfsa_corpus
         return (cd->offsets[a + 1] - cd->offsets[a]) > (cd->offsets[b + 1] - cd->offsets[b]);
     });
     compile_corpus_segmented(f, A, alive.data(), cd->tokens, cd->offsets, cd->p, ids, n_slots, fx_scale, s->sc);
-    s->stats = {s->sc.n_types, s->sc.n_region_instances, s->sc.n_region_edges, s->sc.n_type_edges, s->sc.n_bridge, s->sc.n_strings,
-                (int64_t)(s->sc.host_ms * 1000.0)};
+    int64_t blocks_omitted = 0;
     {   // H_f blocks in the numbering of `trimmed` (raw parameter ids when trimmed is NULL)
         std::vector<int32_t> ttp(f.n_trans()), etp(f.n_emis());
         for (int t = 0; t < f.n_trans(); ++t) ttp[t] = f.trans_param[t] < 0 ? -1 : (trimmed ? trimmed[f.trans_param[t]] : f.trans_param[t]);
         for (int e = 0; e < f.n_emis(); ++e) etp[e] = f.emis_param[e] < 0 ? -1 : (trimmed ? trimmed[f.emis_param[e]] : f.emis_param[e]);
         make_type_blocks(A, ttp, etp, s->sc.rwords, s->sc.rgoff, s->sc.rgrows, s->sc.typeW, s->blocks);
-        if (!s->blocks.fail.empty()) { g_create_error = s->blocks.fail; delete s; return WFSA_ERR_LIMIT; }
+        // the evaluation does not need the blocks: a region type with too many paths leaves them out (zero blocks), not the shard
+        if (!s->blocks.fail.empty()) { s->blocks = TypeBlocks(); blocks_omitted = 1; }
     }
+    s->stats = {s->sc.n_types, s->sc.n_region_instances, s->sc.n_region_edges, s->sc.n_type_edges, s->sc.n_bridge, s->sc.n_strings,
+                (int64_t)(s->sc.host_ms * 1000.0), blocks_omitted};
     *out = s;
     return WFSA_OK;
 }
@@ -2325,6 +2336,15 @@ extern "C" int wfsa_dev_get_info(wfsa_dev* h, wfsa_dev_info* info)
         info->lattice_bridge_edges = h->seg_bridges; info->n_overflow_strings = h->n_active_w; info->pool_slots = h->kl_K;
         info->seg_types = h->seg_types; info->seg_region_instances = h->seg_instances; info->seg_region_edges = h->seg_region_edges;
         info->seg_type_edges = h->seg_type_edges; info->seg_host_ms = h->seg_host_ms;
+        if (h->n >= 0) {                                           // the conditions of k_eval6's P1 (kernels_eval6.cuh)
+            info->e6_big_groups = h->kr_big_groups; info->e6_big_dedicate = eval6_big_dedicate(h);
+            info->e6_big_slots = h->e6_big_slots; info->e6_big_rows = h->e6_big_rows; info->e6_max_big_rows = (int32_t)h->kl_max_words;
+            int two = 0;
+            if (h->kr_big_groups <= h->kl_grid && h->e6_big_slots >= 2)
+                for (int64_t b = 0; b < h->kr_big_groups; ++b)
+                    two += (h->hrgoff[b + 1] - h->hrgoff[b]) >> 5 <= h->e6_big_rows && !(h->hrgrows[b] & 0x10000);
+            info->e6_two_warp_eligible = two;
+        }
     }
     info->n_active_strings = h->n_active + h->n_active_w; info->table_bytes = (int64_t)h->table_bytes;
     info->kernels_launched = h->launches; info->fixed_point_scale_log2 = h->fx_log2;

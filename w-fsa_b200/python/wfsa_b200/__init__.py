@@ -59,7 +59,9 @@ class DevInfo(C.Structure):
                 ("lattice_words", C.c_int64), ("lattice_edges", C.c_int64), ("lattice_bridge_edges", C.c_int64),
                 ("n_overflow_strings", C.c_int64), ("pool_slots", C.c_int32), ("eval_path", C.c_int32),
                 ("seg_types", C.c_int64), ("seg_region_instances", C.c_int64), ("seg_region_edges", C.c_int64),
-                ("seg_type_edges", C.c_int64), ("seg_host_ms", C.c_double)]
+                ("seg_type_edges", C.c_int64), ("seg_host_ms", C.c_double), ("e6_big_groups", C.c_int64),
+                ("e6_big_dedicate", C.c_int32), ("e6_big_slots", C.c_int32), ("e6_big_rows", C.c_int32),
+                ("e6_max_big_rows", C.c_int32), ("e6_two_warp_eligible", C.c_int32)]
 
 
 class PathBlocks(C.Structure):

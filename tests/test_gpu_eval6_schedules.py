@@ -3,15 +3,15 @@ w-fsa_b200/csrc/kernels_eval6.cuh) and through the host-buffer (graph) call, aga
 
 How a big DAG group is walked depends on the number of big groups (n_big, 32 distinct region types each) against the
 persistent grid (one CTA per SM unless WFSA_E6_GRID caps it):
-  A  n_big * 4 <= grid: two warps per group (kr_big_fwd2 / _bwd2 / _red2), the owning CTA dedicated to it;
+  A  n_big * 4 <= grid: two warps per group (big_fwd / big_bwd<false> / big_red<true>), the owning CTA dedicated to it;
   B  grid / 4 < n_big <= grid: the same two-warp chain, its CTA also taking regular groups;
-  C  n_big > grid: one warp per group staged in shared memory (kr_big_t<ACC_GLOBAL, true>); with n_big > 16 * grid a warp
+  C  n_big > grid: one warp per group staged in shared memory (big_one<BigSmem>); with n_big > 16 * grid a warp
      owns several groups and re-stages the later ones;
-  D  no staging area (WFSA_E6_NO_STAGING=1): one warp per group, streamed from HBM (kr_big_t<ACC_GLOBAL, false>).
+  D  no staging area (WFSA_E6_NO_STAGING=1): one warp per group, streamed from HBM (big_one<BigGmem>, as kr_regions).
 A group longer than the staging area is streamed while the others are staged ("mixed").  Every posterior and every
 log-likelihood term is rounded once to 64-bit fixed point and the rounded values are summed as integers, and the two-warp
-chain forms kr_big_t's posteriors bitwise, so every schedule must return the same bits; each must also meet the oracle
-tolerances of test_gpu_parity.py.  Each schedule asserts, through wfsa_dev_info, the regime it claims to run."""
+chain forms the one-warp chain's posteriors bitwise (kernels_seg.cuh, big_sc), so every schedule must return the same bits;
+each must also meet the oracle tolerances of test_gpu_parity.py.  Each schedule asserts, through wfsa_dev_info, the regime it claims to run."""
 import time
 
 import numpy as np

@@ -11,7 +11,7 @@
 //       shapes are fully unrolled: all rows of a group are loaded in one round trip and stay in registers for the REDs;
 //       group descriptors of the regular classes come from a class table in shared memory, not from HBM; big DAG groups are
 //       staged in shared memory and, when a CTA owns one, walked by two warps (forward chain on warp 0, backward chain on
-//       warp 1, kernels_seg.cuh kr_big_fwd2 / _bwd2 / _red2);
+//       warp 1, REDs on warp 0: kernels_seg.cuh big_fwd / big_bwd<false> / big_red<true>), else by one (big_one);
 //   P2  grid barrier (arrival counter in HBM);
 //   P3  fold: one warp per edge gathers the (arc, replica) cells of the edge; with several ranks the per-edge sums are
 //       exchanged through NVLink peer memory as self-validating packets (ll_exchange, kernels_seg.cuh) and the warp
@@ -86,67 +86,6 @@ __device__ __forceinline__ unsigned int e6_ld_acquire(const unsigned int* p)
     return v;
 }
 
-// Path form of any length in batches of LB = 24 / PP levels: every batch is ONE round trip (LB*PP loads in flight), for
-// the products and again for the REDs (the arc ids of a long type do not fit the registers; the second pass finds them
-// in the L1/L2).  The rolled loop of kr_paths pays a round trip per level.  One instance per PP serves every length:
-// fully unrolled instances per (PP, L) made the kernel 26 k instructions, and a warp that runs a rarely used instance
-// waits for instruction fetches from the L2 (cold after the flush) far longer than for data -- measured 15-40 us for ONE
-// group.  Same arithmetic, in the same order, as kr_paths.
-template <int PP>
-__device__ __forceinline__ void e6_paths_long(const KRParams& P, const double* aw, int L, long long g, long long off, int lane,
-                                              unsigned long long* acc_g, long long& ll)
-{
-    constexpr int LB = 24 / PP;
-    const uint32_t* wp = P.words + off + lane;
-    // more than one batch: ask for all rows of the group now (one 128-byte row per lane and round), so that the later
-    // batches find them in the L2 instead of paying a DRAM round trip each (an 8 x 16 group took 26 us: twelve batches)
-    if (L > LB)
-        for (int i = lane; i < L * PP; i += 32) asm volatile("prefetch.global.L2 [%0];" :: "l"(P.words + off + (size_t)i * 32));
-    const double W = P.typeW[g * 32 + lane];
-    double r[PP];
-#pragma unroll
-    for (int p = 0; p < PP; ++p) r[p] = 1.0;
-    for (int l0 = 0; l0 < L; l0 += LB) {
-        uint32_t a[LB * PP];
-#pragma unroll
-        for (int i = 0; i < LB * PP; ++i) a[i] = l0 * PP + i < L * PP ? __ldg(wp + (size_t)(l0 * PP + i) * 32) : (uint32_t)P.n_arcs;
-#pragma unroll
-        for (int l = 0; l < LB; ++l)
-            if (l0 + l < L) {
-#pragma unroll
-                for (int p = 0; p < PP; ++p) r[p] *= aw[a[l * PP + p]];
-            }
-    }
-    double q = 0.0;
-#pragma unroll
-    for (int p = 0; p < PP; ++p) q += r[p];
-    const bool ok = W > 0.0 && q > 0.0 && isfinite(q);
-    if (W > 0.0) {
-        const double lq = ok ? log(q) : -INFINITY;
-        P.lq[g * 32 + lane] = lq;
-        kr_loglik(P, W, ok, lq, ll);
-    }
-    const double sc = ok ? W * P.fx_scale / q : 0.0;
-    long long v[PP];
-#pragma unroll
-    for (int p = 0; p < PP; ++p) v[p] = __double2ll_rn(r[p] * sc);
-    if (P.no_long_reds) return;                                          // timing experiment (debug bit 3): no REDs from long path-form types
-    for (int l0 = 0; l0 < L; l0 += LB) {
-        uint32_t a[LB * PP];
-#pragma unroll
-        for (int i = 0; i < LB * PP; ++i) a[i] = l0 * PP + i < L * PP ? __ldg(wp + (size_t)(l0 * PP + i) * 32) : (uint32_t)P.n_arcs;
-#pragma unroll
-        for (int l = 0; l < LB; ++l)
-            if (l0 + l < L) {
-#pragma unroll
-                for (int p = 0; p < PP; ++p) {
-                    if (l0 + l == 0 && p < 2) red_uniform(acc_g, v[p] ? (int)a[p] : -1, v[p], lane);
-                    else if (v[p]) red_add64(acc_g + a[l * PP + p], (unsigned long long)v[p]);
-                }
-            }
-    }
-}
-
 // Sum of the (arc, replica) cells of one edge by a HALF-warp (hl = lane in the half, hmask = its lanes).  The first
 // (up to 16) arc ids of the edge are already in `first`, one per lane.
 __device__ __forceinline__ unsigned long long e6_fold_edge(const unsigned long long* __restrict__ acc, int n_arcs, int replicas,
@@ -218,7 +157,7 @@ __global__ void __launch_bounds__(NT, 1) k_eval6(const Eval6Params P)
     __shared__ long long s_part[NT / 32][2];
     __shared__ unsigned int s_ticket;                         // next entry of this CTA's static share of the regular groups
     __shared__ int s_bigleft;                                 // warps of this CTA still busy with big DAG groups
-    __shared__ double s_trash[NT];                            // where the lanes without an edge store (kr_big_t)
+    __shared__ double s_trash[NT];                            // where the lanes without an edge store (big_fwd, big_bwd)
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     double* aw = AWG ? P.aw_g : reinterpret_cast<double*>(smem);   // [n_arcs + 1]; the last entry is the zero weight of padding
     double* const sbase = AWG ? reinterpret_cast<double*>(smem) : aw + P.n_arcs + 1;    // shared memory behind the weight table
@@ -327,7 +266,9 @@ __global__ void __launch_bounds__(NT, 1) k_eval6(const Eval6Params P)
     // ---- P1: region types -------------------------------------------------------------------------------------
     KRParams R{};
     R.words = P.words; R.goff = P.goff; R.typeW = P.typeW; R.lq = P.lq; R.xs = P.xs; R.xs_rows = P.xs_rows;
-    R.fx_scale = P.fx_scale; R.ll_scale = ll_scale; R.red = P.red; R.n_arcs = P.n_arcs; R.no_long_reds = (P.debug & 8) ? 1 : 0;
+    R.fx_scale = P.fx_scale; R.ll_scale = ll_scale; R.red = P.red; R.n_arcs = P.n_arcs;
+    const bool path_reds = !(P.debug & 8);                     // timing experiment (debug bit 3): no REDs from path-form types
+    const BigPool pl{(unsigned int)__cvta_generic_to_shared(pool), (unsigned int)NT * 8u, (unsigned int)__cvta_generic_to_shared(&s_trash[tid])};
     unsigned int* const counter = P.ctl + par;
     unsigned long long* const acc_g = P.acc + (size_t)par * acc_words + (size_t)(blockIdx.x % P.replicas) * (size_t)P.n_arcs;
     const long long gwarp = (long long)blockIdx.x * (NT / 32) + warp;
@@ -361,8 +302,8 @@ __global__ void __launch_bounds__(NT, 1) k_eval6(const Eval6Params P)
     long long big = big0;
     long long g = 0;
     // At most one big group per CTA (n_big <= grid: group blockIdx.x on warp 0): the CTA walks the two chains of the group on
-    // two warps, warp 0 forward, warp 1 backward (kernels_seg.cuh, kr_big_fwd2 / _bwd2 / _red2); warp 1 joins the regular groups
-    // afterwards.
+    // two warps, warp 0 forward, warp 1 backward (kernels_seg.cuh, big_fwd / big_bwd<false> / big_red<true>); warp 1 joins
+    // the regular groups afterwards.
     bool two = false;
     int two_nw = 0;
     if (P.n_big <= (long long)gridDim.x && warp < 2 && (long long)blockIdx.x < P.n_big && P.big_slots >= 2 && !(P.debug & (4 | 128))) {
@@ -373,8 +314,7 @@ __global__ void __launch_bounds__(NT, 1) k_eval6(const Eval6Params P)
         double* const xs0 = sxs - (size_t)P.big_rows * 48;                                  // warp 0's staging area
         const unsigned int w0_sa = (unsigned int)__cvta_generic_to_shared(reinterpret_cast<uint32_t*>(xs0 - lane + (size_t)P.big_rows * 32) + lane);
         asm volatile("bar.sync 1, 64;" ::: "memory");                                        // warp 0 has the words in place
-        kr_big_bwd2(aw, (unsigned int)__cvta_generic_to_shared(pool), (unsigned int)NT * 8u, (unsigned int)__cvta_generic_to_shared(&s_trash[tid]),
-                    w0_sa, two_nw, (unsigned int)__cvta_generic_to_shared(sxs));
+        big_bwd<false>(aw, pl, BigSmem{w0_sa, (unsigned int)__cvta_generic_to_shared(sxs)}, two_nw, false, 0.0, 0);
         asm volatile("bar.sync 1, 64;" ::: "memory");                                        // the y stack is complete
     }
     if (big >= P.n_big) {
@@ -400,11 +340,11 @@ __global__ void __launch_bounds__(NT, 1) k_eval6(const Eval6Params P)
         if (rows & 0x10000) {                                  // path form: paths << 8 | length
             const int L = rows & 0xff;
             switch ((rows >> 8) & 0xff) {
-                case 2: e6_paths_long<2>(R, aw, L, g, off, lane, acc_g, ll); break;
-                case 3: e6_paths_long<3>(R, aw, L, g, off, lane, acc_g, ll); break;
-                case 4: e6_paths_long<4>(R, aw, L, g, off, lane, acc_g, ll); break;
-                case 6: e6_paths_long<6>(R, aw, L, g, off, lane, acc_g, ll); break;
-                default: e6_paths_long<8>(R, aw, L, g, off, lane, acc_g, ll); break;
+                case 2: kr_paths<2>(R, aw, L, g, off, lane, acc_g, ll, path_reds); break;
+                case 3: kr_paths<3>(R, aw, L, g, off, lane, acc_g, ll, path_reds); break;
+                case 4: kr_paths<4>(R, aw, L, g, off, lane, acc_g, ll, path_reds); break;
+                case 6: kr_paths<6>(R, aw, L, g, off, lane, acc_g, ll, path_reds); break;
+                default: kr_paths<8>(R, aw, L, g, off, lane, acc_g, ll, path_reds); break;
             }
         } else {
             {
@@ -418,24 +358,18 @@ __global__ void __launch_bounds__(NT, 1) k_eval6(const Eval6Params P)
                 }
                 if (two && warp == 0 && g == big0) {
                     // (stage_big succeeded for this group: two == the same conditions)
-                    const unsigned int wp_sa = (unsigned int)__cvta_generic_to_shared(sw), xs_sa = (unsigned int)__cvta_generic_to_shared(sxs);
-                    const unsigned int ys_sa = (unsigned int)__cvta_generic_to_shared(sxs + (size_t)P.big_rows * 48);      // warp 1's x-stack area
+                    const unsigned int wp_sa = (unsigned int)__cvta_generic_to_shared(sw);
+                    const BigSmem mx{wp_sa, (unsigned int)__cvta_generic_to_shared(sxs)};
+                    const BigSmem my{wp_sa, (unsigned int)__cvta_generic_to_shared(sxs + (size_t)P.big_rows * 48)};   // warp 1's x-stack area
                     asm volatile("bar.sync 1, 64;" ::: "memory");
-                    double qh; int EQ; bool any;
-                    kr_big_fwd2(aw, (unsigned int)__cvta_generic_to_shared(pool), (unsigned int)NT * 8u, (unsigned int)__cvta_generic_to_shared(&s_trash[tid]),
-                                wp_sa, nw, xs_sa, qh, EQ, any);
-                    const double W = R.typeW[g * 32 + lane];
-                    const bool ok = any && qh > 0.0 && isfinite(qh);
-                    if (any) {
-                        const double lq = ok ? log(qh) + (double)EQ * 0.69314718055994530942 : -INFINITY;
-                        R.lq[g * 32 + lane] = lq;
-                        kr_loglik(R, W, ok, lq, ll);
-                    }
+                    double qh, sc0; int EQ; bool any;
+                    big_fwd(aw, pl, mx, nw, qh, EQ, any);
+                    const bool ok = big_lq(R, R.typeW[g * 32 + lane], g, lane, qh, EQ, any, ll, sc0);
                     asm volatile("bar.sync 1, 64;" ::: "memory");
-                    kr_big_red2(wp_sa, nw, xs_sa, ys_sa, ok, ok ? W * R.fx_scale / qh : 0.0, EQ, acc_g);
+                    big_red<true>(mx, my, nw, ok, sc0, EQ, acc_g);
                 } else if (!(P.debug & 4)) {
-                    if (staged) kr_big_t<ACC_GLOBAL, true>(R, aw, pool, NT, g, lane, sw, nw, sxs, acc_g, ll, &s_trash[tid]);
-                    else kr_big_t<ACC_GLOBAL, false>(R, aw, pool, NT, g, lane, P.words + off + lane, nw, xs, acc_g, ll, &s_trash[tid]);
+                    if (staged) big_one(R, aw, pl, BigSmem{(unsigned int)__cvta_generic_to_shared(sw), (unsigned int)__cvta_generic_to_shared(sxs)}, nw, g, lane, acc_g, ll, true);
+                    else big_one(R, aw, pl, BigGmem{P.words + off + lane, xs}, nw, g, lane, acc_g, ll, true);
                 }
                 __syncwarp();
             }

@@ -9,6 +9,7 @@
 //   KR  kr_regions : forward-backward over every distinct region TYPE once (thread per type):
 //                    lq[type] = log q_type,  acc[arc] += W_type * posterior   (64-bit fixed-point REDs),
 //                    loglik += W_type * lq[type]
+//                    (path form: kr_paths; DAG form: big_fwd / big_bwd / big_red; all shared with k_eval6)
 // The bridges need no per-string work: with c[arc] = sum_s p_s * (times arc is a bridge of s), computed when the
 // lattices are compiled, their part of the gradient is the constant c and their part of the log-likelihood is
 // sum_arc c[arc] * log w[arc] (k_prep6).  Only a caller that wants log q_s of every string runs
@@ -33,7 +34,6 @@ struct KRParams {
     unsigned long long* acc;              // [replicas][n_arcs]
     double fx_scale;
     int n_arcs, replicas;
-    int no_long_reds;                     // timing experiment of k_eval6 (debug bit 3): long path-form types skip their REDs
     // log-likelihood: sum_s p_s log q_s = sum_types W_type * lq_type + sum_arcs (bridge count of the arc) * log w[arc].
     // The first sum is accumulated here (fixed point, one RED per CTA), the second one arrives as per-CTA partials of
     // the weight kernel in llpart[n_llpart][2] = (value, non-finite terms) and is added by CTA 0.
@@ -74,25 +74,38 @@ __device__ __forceinline__ void red_uniform(unsigned long long* acc_g, int key, 
     } else if (key >= 0 && v) red_add64(acc_g + key, (unsigned long long)v);
 }
 
-// One region in PATH FORM per thread: PP paths (padded with zero-weight paths) of L edges each, arc of edge l of
-// path p at row l*PP + p.  q = sum_p prod_l w[arc]; every edge of path p gets the posterior r_p / q.  Registers
-// only: PP independent multiply chains, no pool, no flags (the reference's P.x / exp / M algebra,
-// src/Learner.cpp:530-545, for one small segment).
-template <int PP, int ACC>
+// One region in PATH FORM per thread: PP paths (padded with zero-weight paths) of L edges each, arc of edge l of path p at
+// row l*PP + p.  q = sum_p prod_l w[arc]; every edge of path p gets the posterior r_p / q.  Registers only: PP independent
+// multiply chains, no pool, no flags (the reference's P.x / exp / M algebra, src/Learner.cpp:530-545, for one small segment).
+// Levels go in batches of LB = 24 / PP: every batch is ONE round trip (LB*PP loads in flight), for the products and again for
+// the REDs (the arc ids of a long type do not fit the registers; the second pass finds them in the L1/L2); a rolled loop pays
+// a round trip per level.  One instance per PP serves every length: fully unrolled instances per (PP, L) made k_eval6 26 k
+// instructions, and a warp that runs a rarely used instance waits for instruction fetches from the L2 (cold after the flush)
+// far longer than for data -- measured 15-40 us for ONE group.  reds = false: no REDs (timing experiments).
+template <int PP>
 __device__ __forceinline__ void kr_paths(const KRParams& P, const double* aw, int L, long long g, long long off, int lane,
-                                         unsigned long long* acc_g, long long& ll)
+                                         unsigned long long* acc_g, long long& ll, bool reds)
 {
+    constexpr int LB = 24 / PP;
     const uint32_t* wp = P.words + off + lane;
+    // more than one batch: ask for all rows of the group now (one 128-byte row per lane and round), so that the later
+    // batches find them in the L2 instead of paying a DRAM round trip each (an 8 x 16 group took 26 us: twelve batches)
+    if (L > LB)
+        for (int i = lane; i < L * PP; i += 32) asm volatile("prefetch.global.L2 [%0];" :: "l"(P.words + off + (size_t)i * 32));
     const double W = P.typeW[g * 32 + lane];
     double r[PP];
 #pragma unroll
     for (int p = 0; p < PP; ++p) r[p] = 1.0;
-    for (int l = 0; l < L; ++l) {
-        uint32_t a[PP];
+    for (int l0 = 0; l0 < L; l0 += LB) {
+        uint32_t a[LB * PP];
 #pragma unroll
-        for (int p = 0; p < PP; ++p) a[p] = __ldg(wp + (size_t)(l * PP + p) * 32);
+        for (int i = 0; i < LB * PP; ++i) a[i] = l0 * PP + i < L * PP ? __ldg(wp + (size_t)(l0 * PP + i) * 32) : (uint32_t)P.n_arcs;
 #pragma unroll
-        for (int p = 0; p < PP; ++p) r[p] *= aw[a[p]];
+        for (int l = 0; l < LB; ++l)
+            if (l0 + l < L) {
+#pragma unroll
+                for (int p = 0; p < PP; ++p) r[p] *= aw[a[l * PP + p]];
+            }
     }
     double q = 0.0;
 #pragma unroll
@@ -103,208 +116,110 @@ __device__ __forceinline__ void kr_paths(const KRParams& P, const double* aw, in
         P.lq[g * 32 + lane] = lq;
         kr_loglik(P, W, ok, lq, ll);
     }
-    if (ACC == ACC_NONE) return;
     const double sc = ok ? W * P.fx_scale / q : 0.0;
     long long v[PP];
 #pragma unroll
     for (int p = 0; p < PP; ++p) v[p] = __double2ll_rn(r[p] * sc);
-    for (int l = 0; l < L; ++l) {
-        uint32_t a[PP];
+    if (!reds) return;
+    for (int l0 = 0; l0 < L; l0 += LB) {
+        uint32_t a[LB * PP];
 #pragma unroll
-        for (int p = 0; p < PP; ++p) a[p] = __ldg(wp + (size_t)(l * PP + p) * 32);
+        for (int i = 0; i < LB * PP; ++i) a[i] = l0 * PP + i < L * PP ? __ldg(wp + (size_t)(l0 * PP + i) * 32) : (uint32_t)P.n_arcs;
 #pragma unroll
-        for (int p = 0; p < PP; ++p) {
-            if (ACC == ACC_GLOBAL && l == 0 && p < 2) red_uniform(acc_g, v[p] ? (int)a[p] : -1, v[p], lane);
-            else if (v[p]) red_add64(acc_g + a[p], (unsigned long long)v[p]);
-        }
+        for (int l = 0; l < LB; ++l)
+            if (l0 + l < L) {
+#pragma unroll
+                for (int p = 0; p < PP; ++p) {
+                    if (l0 + l == 0 && p < 2) red_uniform(acc_g, v[p] ? (int)a[p] : -1, v[p], lane);
+                    else if (v[p]) red_add64(acc_g + a[l * PP + p], (unsigned long long)v[p]);
+                }
+            }
     }
 }
 
-// One big region per thread: the KL stream loop (CHECK words rescale, x values on a stack).  STAGED = false: words
-// streamed from HBM (wp = P.words + goff[g] + lane), stack in HBM (one slab per warp).  STAGED = true (k_eval6): the
-// caller copied the nw word rows of the group to shared memory (wp) and the stack lives there as well, so that the serial
-// chain of a region (up to ~100 dependent steps, twice) runs at shared-memory latency.
-template <int ACC, bool STAGED>
-__device__ __forceinline__ void kr_big_t(const KRParams& P, const double* aw, double* pool, int NT, long long g, int lane,
-                                         const uint32_t* wp, int nw, double* xs, unsigned long long* acc_g, long long& ll, double* trash)
+// ---- big DAG regions: the KL stream loop (CHECK words rescale, x values on a stack), one thread per region -------------
+// A group is walked by three blocks: big_fwd (forward chain), big_bwd (backward chain) and big_red (the REDs).  One warp
+// runs all three (k_eval6 with one warp per group, kr_regions), or two warps split them (k_eval6, a CTA that owns one
+// staged group): warp 0 big_fwd, warp 1 big_bwd<false> on its own pool at the same time, then warp 0 big_red<true>.
+//
+// The chain of a region is serial (every step reads the node value the previous step wrote): what a step costs is the
+// latency of its dependent instructions.  Both chain loops are therefore free of branches inside a batch of eight words:
+// every lane does the same loads, arithmetic and stores, and a lane whose word is padding, FIN or belongs to a shorter region
+// works on slot 0 / arc 0 and stores into `trash` (one double per thread).  The decode and the weight loads of step k + 1
+// then overlap the chain of step k.  Measured before (45 instructions with four branches per step): ~300 cycles per step,
+// the 96-row group of a 125 k-string shard alone took 31 us of a 37 us region phase.  A lone warp still gets ~4 cycles per
+// instruction whatever is done about its dependencies (interleaving the two chains in one instruction stream was measured
+// twice: slower), but the chains are independent until the posteriors, so two warps -- two schedulers -- can walk them.
+//
+// The pool lives in shared memory and is addressed as such: node value of slot s of the lane at byte address p + s * ps.
+// (A generic store to the shared window sits in the same in-order LSU queue as the chain's LDS/STS and takes longer to
+// resolve.)  No memory clobbers: the pool and the staging area are touched by these volatile statements only, which keep
+// their order among themselves; a clobber would pin every other memory access around each of them.
+struct BigPool { unsigned int p, ps, trash; };
+__device__ __forceinline__ double lds_f64(unsigned int a) { double v; asm volatile("ld.shared.f64 %0, [%1];" : "=d"(v) : "r"(a)); return v; }
+__device__ __forceinline__ void sts_f64(unsigned int a, double v) { asm volatile("st.shared.f64 [%0], %1;" :: "r"(a), "d"(v)); }
+__device__ __forceinline__ int lds_exp(unsigned int a) { int hi; asm volatile("ld.shared.u32 %0, [%1];" : "=r"(hi) : "r"(a + 4u)); return (hi >> 20) & 0x7ff; }
+
+// Where the words (row i: word of the lane) and the x stack (row i: 64 bits of the lane) of a group live.  BigSmem: the
+// staging area of shared memory (k_eval6), byte addresses of the lane's column, so that the chain runs at shared-memory
+// latency.  BigGmem: streamed from HBM, the stack in HBM, one slab per warp (kr_regions, k_eval6 without staging).
+struct BigSmem {
+    unsigned int w, x;
+    __device__ __forceinline__ uint32_t word(int i) const { uint32_t v; asm volatile("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(w + (unsigned int)i * 128u)); return v; }
+    __device__ __forceinline__ long long ld(int i) const { long long v; asm volatile("ld.shared.b64 %0, [%1];" : "=l"(v) : "r"(x + (unsigned int)i * 256u)); return v; }
+    __device__ __forceinline__ void st(int i, long long v) const { asm volatile("st.shared.b64 [%0], %1;" :: "r"(x + (unsigned int)i * 256u), "l"(v)); }
+};
+struct BigGmem {
+    const uint32_t* w; double* x;
+    __device__ __forceinline__ uint32_t word(int i) const { return __ldcs(w + (size_t)i * 32); }
+    __device__ __forceinline__ long long ld(int i) const { return reinterpret_cast<const long long*>(x)[(size_t)i * 32]; }
+    __device__ __forceinline__ void st(int i, long long v) const { reinterpret_cast<long long*>(x)[(size_t)i * 32] = v; }
+};
+
+// A CHECK word with pool slot mask m0: when the largest exponent among those slots has left the band 1023 +- kLBand, they
+// are scaled back to exponent 0.  Returns the shift (0: nothing to do), which the chain subtracts from its exponent.
+__device__ __forceinline__ int big_rescale(const BigPool& pl, uint32_t m0)
 {
-    // The chain of a region is serial (every step reads the node value the previous step wrote), and ONE warp walks it:
-    // what a step costs is the latency of its dependent instructions.  Both chain loops are therefore free of branches
-    // inside a batch of eight words: every lane does the same loads, arithmetic and stores, and a lane whose word is
-    // padding, FIN or belongs to a shorter region works on slot 0 / arc 0 and stores into `trash` (one double per
-    // thread).  The decode and the weight loads of step k + 1 then overlap the chain of step k.  The posteriors are
-    // rounded inside the backward chain and parked in the x stack; a third loop without dependencies issues the REDs.
-    // Measured before (45 instructions with four branches per step): ~300 cycles per step, the 96-row group of a
-    // 125 k-string shard alone took 31 us of a 37 us region phase.
-    // STAGED: words and x stack are in shared memory; address them as such (a generic store to the shared window sits in the
-    // same in-order LSU queue as the chain's LDS/STS and takes longer to resolve)
-    const unsigned int wp_sa = STAGED ? (unsigned int)__cvta_generic_to_shared(wp) : 0u;
-    const unsigned int xs_sa = STAGED ? (unsigned int)__cvta_generic_to_shared(xs) : 0u;
-    auto ldw = [&](int i) -> uint32_t {
-        if (STAGED) { uint32_t v; asm volatile("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(wp_sa + (unsigned int)i * 128u)); return v; }
-        return __ldcs(wp + (size_t)i * 32);
-    };
-    auto xs_ld = [&](int i) -> long long {
-        if (STAGED) { long long v; asm volatile("ld.shared.b64 %0, [%1];" : "=l"(v) : "r"(xs_sa + (unsigned int)i * 256u)); return v; }
-        return reinterpret_cast<const long long*>(xs)[(size_t)i * 32];
-    };
-    auto xs_st = [&](int i, long long v) {
-        // (no memory clobber: the x stack is touched by these volatile statements only, which keep their order among themselves;
-        //  a clobber would pin the chain's pool accesses around every store)
-        if (STAGED) asm volatile("st.shared.b64 [%0], %1;" :: "r"(xs_sa + (unsigned int)i * 256u), "l"(v));
-        else reinterpret_cast<long long*>(xs)[(size_t)i * 32] = v;
-    };
-    const double W = P.typeW[g * 32 + lane];
-    pool[0] = 1.0;
-    int E = 0, EQ = 0;
-    double qh = 0.0;
-    bool any = false;
-    for (int i0 = 0; i0 < nw; i0 += 8) {
-        uint32_t w[8];
-#pragma unroll
-        for (int j = 0; j < 8; ++j) w[j] = ldw(i0 + j);
-        const bool has_chk = (i0 & 8) != 0;                   // word 7 of every second batch is a CHECK word (same index in all lanes)
-        if (has_chk) w[7] = 0u;
-        // decode first (addresses and weights of the eight steps are independent of the chain), then the chain itself:
-        // per step  LDS node -> DMUL -> DADD -> select -> STS  and nothing else
-        const double* ps[8]; double* pd[8]; double wv[8];
-#pragma unroll
-        for (int j = 0; j < 8; ++j) {
-            const uint32_t wj = w[j];
-            const bool edge = (wj & kLEdge) != 0;
-            const int src = edge ? (wj >> 19) & 15 : (wj & 15), arc = edge ? (int)(wj & 0xffff) : 0;
-            ps[j] = pool + src * NT;                          // (FIN: the exit node)
-            pd[j] = edge ? pool + ((wj >> 23) & 15) * NT : trash;
-            wv[j] = aw[arc];
-            any |= edge;
-        }
-#pragma unroll
-        for (int j = 0; j < 8; ++j) {
-            const uint32_t wj = w[j];
-            const bool fin = (wj & (kLEdge | kLFin)) == kLFin;
-            const double a = *ps[j];
-            const double xv = a * wv[j];
-            const double sum = *pd[j] + xv;
-            *pd[j] = (wj & kLFirstIn) ? xv : sum;
-            xs_st(i0 + j, __double_as_longlong(xv));
-            qh = fin ? a : qh;
-            EQ = fin ? E : EQ;
-        }
-        if (has_chk) {
-            const uint32_t m0 = ldw(i0 + 7) & 0xffffu;
-            xs_st(i0 + 7, (long long)E);
-            if (m0) {
-                int emax = 0;
-                for (uint32_t m = m0; m; m &= m - 1) emax = max(emax, pool_exp(pool + (__ffs(m) - 1) * NT));
-                if (emax != 0 && (emax < 1023 - kLBand || emax > 1023 + kLBand)) {
-                    const int shift = 1023 - emax;
-                    for (uint32_t m = m0; m; m &= m - 1) { double* q = pool + (__ffs(m) - 1) * NT; *q = scalbn(*q, shift); }
-                    E -= shift;
-                }
-            }
-        }
-    }
-    const bool ok = any && qh > 0.0 && isfinite(qh);
-    if (any) {
-        const double lq = ok ? log(qh) + (double)EQ * 0.69314718055994530942 : -INFINITY;
-        P.lq[g * 32 + lane] = lq;
-        kr_loglik(P, W, ok, lq, ll);
-    }
-    const double sc0 = ok ? W * P.fx_scale / qh : 0.0;
-    double sc = sc0;
-    int F = 0;
-    for (int i0 = nw - 8; i0 >= 0; i0 -= 8) {
-        uint32_t w[8];
-        double xv[8];
-#pragma unroll
-        for (int j = 0; j < 8; ++j) { w[j] = ldw(i0 + j); xv[j] = __longlong_as_double(xs_ld(i0 + j)); }
-        const bool has_chk = (i0 & 8) != 0;
-        if (has_chk) {
-            const uint32_t m0 = w[7] & 0xffffu;
-            if (m0) {
-                const int Et = (int)__double_as_longlong(xv[7]);
-                int emax = 0;
-                for (uint32_t m = m0; m; m &= m - 1) emax = max(emax, pool_exp(pool + (__ffs(m) - 1) * NT));
-                if (emax != 0 && (emax < 1023 - kLBand || emax > 1023 + kLBand)) {
-                    const int shift = 1023 - emax;
-                    for (uint32_t m = m0; m; m &= m - 1) { double* q = pool + (__ffs(m) - 1) * NT; *q = scalbn(*q, shift); }
-                    F -= shift;
-                }
-                sc = scalbn(sc0, Et + F - EQ);
-            }
-            w[7] = 0u;
-        }
-        const double* pdst[8]; double* psrc[8]; double wv[8];
-#pragma unroll
-        for (int j = 0; j < 8; ++j) {
-            const uint32_t wj = w[j];
-            const bool edge = (wj & kLEdge) != 0;
-            const int slot = edge ? (wj >> 19) & 15 : (wj & 15), arc = edge ? (int)(wj & 0xffff) : 0;   // (FIN: the exit node, beta = 1)
-            pdst[j] = pool + ((wj >> 23) & 15) * NT;
-            psrc[j] = (wj & (kLEdge | kLFin)) ? pool + slot * NT : trash;
-            wv[j] = aw[arc];
-        }
-#pragma unroll
-        for (int j = 7; j >= 0; --j) {
-            const uint32_t wj = w[j];
-            const bool edge = (wj & kLEdge) != 0;
-            const bool fin = (wj & (kLEdge | kLFin)) == kLFin;
-            const double bd = *pdst[j];
-            const double c = wv[j] * bd;
-            const double sum = *psrc[j] + c;
-            *psrc[j] = fin ? 1.0 : ((wj & kLLastOut) ? c : sum);
-            const long long v = __double2ll_rn(xv[j] * bd * sc);
-            xs_st(i0 + j, (edge && ok) ? v : 0ll);
-        }
-    }
-    if (ACC == ACC_NONE) return;
-    for (int i0 = 0; i0 < nw; i0 += 8) {                      // the REDs: no dependencies between the steps
-        uint32_t w[8];
-        long long v[8];
-#pragma unroll
-        for (int j = 0; j < 8; ++j) { w[j] = ldw(i0 + j); v[j] = xs_ld(i0 + j); }
-#pragma unroll
-        for (int j = 0; j < 8; ++j) if (v[j]) red_add64(acc_g + (w[j] & 0xffff), (unsigned long long)v[j]);
-    }
+    if (!m0) return 0;
+    int emax = 0;
+    for (uint32_t m = m0; m; m &= m - 1) emax = max(emax, lds_exp(pl.p + (unsigned int)(__ffs(m) - 1) * pl.ps));
+    if (emax == 0 || (emax >= 1023 - kLBand && emax <= 1023 + kLBand)) return 0;
+    const int shift = 1023 - emax;
+    for (uint32_t m = m0; m; m &= m - 1) { const unsigned int a = pl.p + (unsigned int)(__ffs(m) - 1) * pl.ps; sts_f64(a, scalbn(lds_f64(a), shift)); }
+    return shift;
 }
 
-// ---- one big DAG group on TWO warps (k_eval6, a staged group on a dedicated CTA) ---------------------------------------
-// The chain of a region costs a lone warp ~4 cycles per instruction whatever is done about its dependencies (interleaving
-// the forward with the backward chain in one instruction stream was measured twice: slower).  But the two chains are
-// independent until the posteriors -- alpha needs the weights only, beta as well -- so they can run on two warps, i.e. two
-// schedulers: warp 0 walks the words forward (x stack: alpha_src * w per edge, E at the CHECK words), warp 1 backward on its own
-// pool (y stack: beta_dst per edge, F at the CHECK words), and warp 0 then forms (x * y) * sc in the order and with the scale
-// factors of kr_big_t -- bitwise the same posteriors -- and issues the REDs.  All addresses are shared-memory byte addresses of
-// the calling lane's column: wp_sa words [rows][32] u32, xs_sa / ys_sa stacks [rows][32] f64, pool at stride NT doubles.
-__device__ __forceinline__ double bg_lds(unsigned int a) { double v; asm volatile("ld.shared.f64 %0, [%1];" : "=d"(v) : "r"(a)); return v; }
-__device__ __forceinline__ void bg_sts(unsigned int a, double v) { asm volatile("st.shared.f64 [%0], %1;" :: "r"(a), "d"(v)); }
-__device__ __forceinline__ uint32_t bg_ldw(unsigned int wp_sa, int i) { uint32_t v; asm volatile("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(wp_sa + (unsigned int)i * 128u)); return v; }
-__device__ __forceinline__ void bg_st64(unsigned int base, int i, long long v) { asm volatile("st.shared.b64 [%0], %1;" :: "r"(base + (unsigned int)i * 256u), "l"(v)); }
-__device__ __forceinline__ long long bg_ld64(unsigned int base, int i) { long long v; asm volatile("ld.shared.b64 %0, [%1];" : "=l"(v) : "r"(base + (unsigned int)i * 256u)); return v; }
-__device__ __forceinline__ int bg_exp(unsigned int a) { int hi; asm volatile("ld.shared.u32 %0, [%1];" : "=r"(hi) : "r"(a + 4u)); return (hi >> 20) & 0x7ff; }
+// The posterior scale below a CHECK word.  x = alpha_src * w carries the forward scale 2^E (E from the x stack), beta_dst
+// the backward scale 2^F and q the scale 2^EQ, so posterior = (x * beta_dst) * sc with sc = sc0 * 2^(E + F - EQ),
+// sc0 = W * fx_scale / q.  The one-warp backward chain (big_bwd<true>) and the two-warp RED pass (big_red<true>) both round
+// (x * beta_dst) * sc once, with sc from here and from the same E, F and EQ: every schedule returns the same bits.
+__device__ __forceinline__ double big_sc(double sc0, int E, int F, int EQ) { return scalbn(sc0, E + F - EQ); }
 
-// forward chain; returns q (its exponent in EQ) and whether the lane holds a region at all
-__device__ __forceinline__ void kr_big_fwd2(const double* aw, unsigned int p_sa, unsigned int ps, unsigned int tr_sa, unsigned int wp_sa, int nw,
-                                            unsigned int xs_sa, double& qh, int& EQ, bool& any)
+// Forward chain: alpha_src * w of every edge to the x stack, E to the CHECK slots; returns q (its exponent in EQ) and whether
+// the lane holds a region at all.
+template <class M>
+__device__ __forceinline__ void big_fwd(const double* aw, const BigPool& pl, const M& m, int nw, double& qh, int& EQ, bool& any)
 {
-    bg_sts(p_sa, 1.0);
+    sts_f64(pl.p, 1.0);
     int E = 0;
     EQ = 0; qh = 0.0; any = false;
     for (int i0 = 0; i0 < nw; i0 += 8) {
         uint32_t w[8];
 #pragma unroll
-        for (int j = 0; j < 8; ++j) w[j] = bg_ldw(wp_sa, i0 + j);
-        const bool chk = (i0 & 8) != 0;
+        for (int j = 0; j < 8; ++j) w[j] = m.word(i0 + j);
+        const bool chk = (i0 & 8) != 0;                       // word 7 of every second batch is a CHECK word (same index in all lanes)
         const uint32_t m0 = chk ? w[7] & 0xffffu : 0u;
         if (chk) w[7] = 0u;
+        // decode first (addresses and weights of the eight steps are independent of the chain), then the chain itself:
+        // per step  LDS node -> DMUL -> DADD -> select -> STS  and nothing else
         unsigned int fs[8], fd[8];
         double fw[8];
 #pragma unroll
         for (int j = 0; j < 8; ++j) {
             const uint32_t wj = w[j];
             const bool edge = (wj & kLEdge) != 0;
-            fs[j] = p_sa + (edge ? (wj >> 19) & 15u : (wj & 15u)) * ps;
-            fd[j] = edge ? p_sa + ((wj >> 23) & 15u) * ps : tr_sa;
+            fs[j] = pl.p + (edge ? (wj >> 19) & 15u : (wj & 15u)) * pl.ps;   // (FIN: the exit node)
+            fd[j] = edge ? pl.p + ((wj >> 23) & 15u) * pl.ps : pl.trash;
             fw[j] = aw[edge ? (wj & 0xffffu) : 0u];
             any |= edge;
         }
@@ -312,51 +227,41 @@ __device__ __forceinline__ void kr_big_fwd2(const double* aw, unsigned int p_sa,
         for (int j = 0; j < 8; ++j) {
             const uint32_t wj = w[j];
             const bool fin = (wj & (kLEdge | kLFin)) == kLFin;
-            const double a = bg_lds(fs[j]);
+            const double a = lds_f64(fs[j]);
             const double xv = a * fw[j];
-            const double old = bg_lds(fd[j]);
-            bg_sts(fd[j], (wj & kLFirstIn) ? xv : old + xv);
-            bg_st64(xs_sa, i0 + j, __double_as_longlong(xv));
+            const double old = lds_f64(fd[j]);
+            sts_f64(fd[j], (wj & kLFirstIn) ? xv : old + xv);
+            m.st(i0 + j, __double_as_longlong(xv));
             qh = fin ? a : qh;
             EQ = fin ? E : EQ;
         }
         if (chk) {
-            bg_st64(xs_sa, i0 + 7, (long long)E);
-            if (m0) {
-                int emax = 0;
-                for (uint32_t m = m0; m; m &= m - 1) emax = max(emax, bg_exp(p_sa + (unsigned int)(__ffs(m) - 1) * ps));
-                if (emax != 0 && (emax < 1023 - kLBand || emax > 1023 + kLBand)) {
-                    const int shift = 1023 - emax;
-                    for (uint32_t m = m0; m; m &= m - 1) { const unsigned int a = p_sa + (unsigned int)(__ffs(m) - 1) * ps; bg_sts(a, scalbn(bg_lds(a), shift)); }
-                    E -= shift;
-                }
-            }
+            m.st(i0 + 7, (long long)E);
+            E -= big_rescale(pl, m0);
         }
     }
 }
 
-// backward chain on the caller's own pool: beta of the target node of every edge to the y stack, F to the CHECK slots
-__device__ __forceinline__ void kr_big_bwd2(const double* aw, unsigned int p_sa, unsigned int ps, unsigned int tr_sa, unsigned int wp_sa, int nw,
-                                            unsigned int ys_sa)
+// Backward chain, beta_dst of every edge, F at the CHECK words.  ROUND (one warp, after big_fwd on the same stack): the
+// posterior of every edge, rounded to fixed point, replaces x in the stack (0 for every other word); sc0 = 0 when !ok.
+// !ROUND (two warps): beta_dst of every edge and F at the CHECK words go to the stack of m -- the y stack, while the
+// partner warp fills the x stack with big_fwd -- and big_red<true> forms the posteriors (ok, sc0, EQ unused).
+template <bool ROUND, class M>
+__device__ __forceinline__ void big_bwd(const double* aw, const BigPool& pl, const M& m, int nw, bool ok, double sc0, int EQ)
 {
+    double sc = sc0;
     int F = 0;
     for (int i0 = nw - 8; i0 >= 0; i0 -= 8) {
         uint32_t w[8];
+        double xv[8];
 #pragma unroll
-        for (int j = 0; j < 8; ++j) w[j] = bg_ldw(wp_sa, i0 + j);
+        for (int j = 0; j < 8; ++j) { w[j] = m.word(i0 + j); if (ROUND) xv[j] = __longlong_as_double(m.ld(i0 + j)); }
         const bool chk = (i0 & 8) != 0;
         if (chk) {                                             // the CHECK word comes first in backward order
             const uint32_t m0 = w[7] & 0xffffu;
-            if (m0) {
-                int emax = 0;
-                for (uint32_t m = m0; m; m &= m - 1) emax = max(emax, bg_exp(p_sa + (unsigned int)(__ffs(m) - 1) * ps));
-                if (emax != 0 && (emax < 1023 - kLBand || emax > 1023 + kLBand)) {
-                    const int shift = 1023 - emax;
-                    for (uint32_t m = m0; m; m &= m - 1) { const unsigned int a = p_sa + (unsigned int)(__ffs(m) - 1) * ps; bg_sts(a, scalbn(bg_lds(a), shift)); }
-                    F -= shift;
-                }
-            }
-            bg_st64(ys_sa, i0 + 7, (long long)F);
+            F -= big_rescale(pl, m0);
+            if (!ROUND) m.st(i0 + 7, (long long)F);
+            else if (m0) sc = big_sc(sc0, (int)__double_as_longlong(xv[7]), F, EQ);
             w[7] = 0u;
         }
         unsigned int bd_[8], bs[8];
@@ -365,59 +270,88 @@ __device__ __forceinline__ void kr_big_bwd2(const double* aw, unsigned int p_sa,
         for (int j = 0; j < 8; ++j) {
             const uint32_t wj = w[j];
             const bool edge = (wj & kLEdge) != 0;
-            bd_[j] = p_sa + ((wj >> 23) & 15u) * ps;
-            bs[j] = (wj & (kLEdge | kLFin)) ? p_sa + (edge ? (wj >> 19) & 15u : (wj & 15u)) * ps : tr_sa;
+            bd_[j] = pl.p + ((wj >> 23) & 15u) * pl.ps;
+            bs[j] = (wj & (kLEdge | kLFin)) ? pl.p + (edge ? (wj >> 19) & 15u : (wj & 15u)) * pl.ps : pl.trash;   // (FIN: the exit node, beta = 1)
             bw[j] = aw[edge ? (wj & 0xffffu) : 0u];
         }
 #pragma unroll
         for (int j = 7; j >= 0; --j) {
             const uint32_t wj = w[j];
+            const bool edge = (wj & kLEdge) != 0;
             const bool fin = (wj & (kLEdge | kLFin)) == kLFin;
-            const double bd = bg_lds(bd_[j]);
+            const double bd = lds_f64(bd_[j]);
             const double c = bw[j] * bd;
-            const double old = bg_lds(bs[j]);
-            bg_sts(bs[j], fin ? 1.0 : ((wj & kLLastOut) ? c : old + c));
-            if (!(j == 7 && chk)) bg_st64(ys_sa, i0 + j, __double_as_longlong(bd));
+            const double old = lds_f64(bs[j]);
+            sts_f64(bs[j], fin ? 1.0 : ((wj & kLLastOut) ? c : old + c));
+            if (ROUND) m.st(i0 + j, (edge && ok) ? __double2ll_rn(xv[j] * bd * sc) : 0ll);
+            else if (!(j == 7 && chk)) m.st(i0 + j, __double_as_longlong(bd));
         }
     }
 }
 
-// posteriors (x * y) * sc and their REDs; sc follows the CHECK words exactly as in kr_big_t
-__device__ __forceinline__ void kr_big_red2(unsigned int wp_sa, int nw, unsigned int xs_sa, unsigned int ys_sa, bool ok, double sc0, int EQ,
-                                            unsigned long long* acc_g)
+// The REDs, without dependencies between the steps.  XY = false: the posteriors the one-warp big_bwd left rounded in the
+// stack of x, in word order.  XY = true: formed here as (x * y) * sc from the x stack of big_fwd and the y stack of
+// big_bwd<false>, backward, because sc changes at the CHECK words.
+template <bool XY, class M>
+__device__ __forceinline__ void big_red(const M& x, const M& y, int nw, bool ok, double sc0, int EQ, unsigned long long* acc_g)
 {
     double sc = sc0;
-    for (int i0 = nw - 8; i0 >= 0; i0 -= 8) {
+    for (int k = 0; k < nw; k += 8) {
+        const int i0 = XY ? nw - 8 - k : k;
         uint32_t w[8];
-        long long x[8], y[8];
+        long long xv[8], yv[8];
 #pragma unroll
-        for (int j = 0; j < 8; ++j) { w[j] = bg_ldw(wp_sa, i0 + j); x[j] = bg_ld64(xs_sa, i0 + j); y[j] = bg_ld64(ys_sa, i0 + j); }
-        if (i0 & 8) {
-            if (w[7] & 0xffffu) sc = scalbn(sc0, (int)x[7] + (int)y[7] - EQ);
+        for (int j = 0; j < 8; ++j) { w[j] = x.word(i0 + j); xv[j] = x.ld(i0 + j); if (XY) yv[j] = y.ld(i0 + j); }
+        if (XY && (i0 & 8)) {
+            if (w[7] & 0xffffu) sc = big_sc(sc0, (int)xv[7], (int)yv[7], EQ);
             w[7] = 0u;
         }
 #pragma unroll
         for (int j = 7; j >= 0; --j) {
-            if (!(w[j] & kLEdge) || !ok) continue;
-            const long long v = __double2ll_rn(__longlong_as_double(x[j]) * __longlong_as_double(y[j]) * sc);
+            long long v = xv[j];
+            if (XY) {
+                if (!(w[j] & kLEdge) || !ok) continue;
+                v = __double2ll_rn(__longlong_as_double(xv[j]) * __longlong_as_double(yv[j]) * sc);
+            }
             if (v) red_add64(acc_g + (w[j] & 0xffff), (unsigned long long)v);
         }
     }
 }
 
-template <int ACC>
-__device__ __forceinline__ void kr_big(const KRParams& P, const double* aw, double* pool, int NT, long long g, int lane,
-                                       double* xs, unsigned long long* acc_g, long long& ll, double* trash)
+// log q of the lane's region from the forward chain into lq[] and the log-likelihood; returns whether q is usable and in
+// sc0 the posterior scale W * fx_scale / q (0 if not)
+__device__ __forceinline__ bool big_lq(const KRParams& P, double W, long long g, int lane, double qh, int EQ, bool any, long long& ll, double& sc0)
 {
-    const long long o = P.goff[g];
-    kr_big_t<ACC, false>(P, aw, pool, NT, g, lane, P.words + o + lane, (int)((P.goff[g + 1] - o) >> 5), xs, acc_g, ll, trash);
+    const bool ok = any && qh > 0.0 && isfinite(qh);
+    if (any) {
+        const double lq = ok ? log(qh) + (double)EQ * 0.69314718055994530942 : -INFINITY;
+        P.lq[g * 32 + lane] = lq;
+        kr_loglik(P, W, ok, lq, ll);
+    }
+    sc0 = ok ? W * P.fx_scale / qh : 0.0;
+    return ok;
+}
+
+// One big group on one warp: forward chain, log q, backward chain rounding the posteriors, REDs (reds = false: none).
+template <class M>
+__device__ __forceinline__ void big_one(const KRParams& P, const double* aw, const BigPool& pl, const M& m, int nw, long long g, int lane,
+                                        unsigned long long* acc_g, long long& ll, bool reds)
+{
+    const double W = P.typeW[g * 32 + lane];
+    double qh, sc0;
+    int EQ;
+    bool any;
+    big_fwd(aw, pl, m, nw, qh, EQ, any);
+    const bool ok = big_lq(P, W, g, lane, qh, EQ, any, ll, sc0);
+    big_bwd<true>(aw, pl, m, nw, ok, sc0, EQ);
+    if (reds) big_red<false>(m, m, nw, ok, sc0, EQ, acc_g);
 }
 
 template <int ACC, int MAXNT, bool AWG = false>
 __global__ void __launch_bounds__(MAXNT, 1) kr_regions(const KRParams P)
 {
     extern __shared__ unsigned long long smem[];
-    __shared__ double s_trash[MAXNT];                         // where the lanes without an edge store (kr_big_t)
+    __shared__ double s_trash[MAXNT];                         // where the lanes without an edge store (big_fwd, big_bwd)
     const int tid = threadIdx.x, NT = blockDim.x, lane = tid & 31;
     // [n_arcs + 1] arc weights, the last entry the zero weight of padding: a copy in shared memory, or (AWG: the table does not
     // fit) P.aw itself, which then has the zero entry behind it
@@ -428,6 +362,8 @@ __global__ void __launch_bounds__(MAXNT, 1) kr_regions(const KRParams P)
     const long long gwarp = ((long long)blockIdx.x * NT + tid) >> 5;
     double* const xs = P.xs + (size_t)gwarp * P.xs_rows * 32 + lane;
     unsigned long long* const acc_g = P.acc + (size_t)(blockIdx.x % P.replicas) * (size_t)P.n_arcs;
+    const bool reds = ACC != ACC_NONE;                        // ACC_NONE: no REDs at all (timing experiment)
+    const BigPool pl{(unsigned int)__cvta_generic_to_shared(pool), (unsigned int)NT * 8u, (unsigned int)__cvta_generic_to_shared(&s_trash[tid])};
     // groups are sorted by cost (DAG regions first, then path form by paths and length) and handed out dynamically, one
     // at a time; the id of the next group is requested while the current one is processed
     long long g = 0, ll = 0;
@@ -441,13 +377,13 @@ __global__ void __launch_bounds__(MAXNT, 1) kr_regions(const KRParams P)
         if (rows & 0x10000) {                                  // path form: paths << 8 | length
             const int L = rows & 0xff;
             switch ((rows >> 8) & 0xff) {
-                case 2: kr_paths<2, ACC>(P, aw, L, g, off, lane, acc_g, ll); break;
-                case 3: kr_paths<3, ACC>(P, aw, L, g, off, lane, acc_g, ll); break;
-                case 4: kr_paths<4, ACC>(P, aw, L, g, off, lane, acc_g, ll); break;
-                case 6: kr_paths<6, ACC>(P, aw, L, g, off, lane, acc_g, ll); break;
-                default: kr_paths<8, ACC>(P, aw, L, g, off, lane, acc_g, ll); break;
+                case 2: kr_paths<2>(P, aw, L, g, off, lane, acc_g, ll, reds); break;
+                case 3: kr_paths<3>(P, aw, L, g, off, lane, acc_g, ll, reds); break;
+                case 4: kr_paths<4>(P, aw, L, g, off, lane, acc_g, ll, reds); break;
+                case 6: kr_paths<6>(P, aw, L, g, off, lane, acc_g, ll, reds); break;
+                default: kr_paths<8>(P, aw, L, g, off, lane, acc_g, ll, reds); break;
             }
-        } else kr_big<ACC>(P, aw, pool, NT, g, lane, xs, acc_g, ll, &s_trash[tid]);
+        } else big_one(P, aw, pl, BigGmem{P.words + off + lane, xs}, (int)((P.goff[g + 1] - off) >> 5), g, lane, acc_g, ll, reds);
         g = __shfl_sync(FULL, gn, 0);
     }
     // the CTA's share of the log-likelihood: integer sums (exact, order independent), one RED per CTA

@@ -239,6 +239,10 @@ int wfsa_segmented_get(const wfsa_segmented* s, int which, const void** data, in
 void wfsa_segmented_free(wfsa_segmented* s);
 
 void wfsa_dev_destroy(wfsa_dev* h);
+/* Bytes of device and pinned host memory held by all handles of this process, for leak tests: a handle that is
+ * destroyed, or a parameter map that is replaced, must give back all it took.  (cudaMemGetInfo would see every
+ * process on the device.) */
+int64_t wfsa_dev_held_bytes(void);
 const char* wfsa_dev_last_error(const wfsa_dev* h);   /* h may be NULL: last create() error */
 const char* wfsa_dev_version(void);
 

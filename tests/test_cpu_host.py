@@ -98,6 +98,7 @@ def test_no_cpu_fallback_without_gpu():
         assert e.code == 3 and "no CPU fallback" in e.message
         with pytest.raises(W.WfsaError):
             W.Session(case["fsa_text"], case["corpus_text"])
+        assert W.lib().wfsa_dev_held_bytes() == 0
     else:
         dev.close()
         pytest.skip("a GPU is present")

@@ -9,6 +9,7 @@
 #include <dlfcn.h>
 
 #include <algorithm>
+#include <atomic>
 #include <chrono>
 #include <cmath>
 #include <cstdio>
@@ -19,6 +20,7 @@
 #include <memory>
 #include <string>
 #include <thread>
+#include <utility>
 #include <vector>
 
 #include "../../include/wfsa_dev.h"
@@ -63,25 +65,71 @@ struct NcclApi {
     }
 };
 NcclApi g_nccl;
+std::atomic<int64_t> g_held_bytes{0};         // wfsa_dev_held_bytes
 
-template <class T> struct DevBuf {
+// Owns one allocation of n elements: device memory, or with Pinned page-locked host memory (cudaHostAlloc `flags`).
+template <class T, bool Pinned> struct Buf {
     T* p = nullptr; size_t n = 0;
-    cudaError_t alloc(size_t count) { release(); n = count; return count ? cudaMalloc(&p, count * sizeof(T)) : cudaSuccess; }
+    Buf() = default;
+    Buf(const Buf&) = delete; Buf& operator=(const Buf&) = delete;
+    Buf(Buf&& o) noexcept : p(std::exchange(o.p, nullptr)), n(std::exchange(o.n, 0)) {}
+    Buf& operator=(Buf&& o) noexcept { if (this != &o) { release(); p = std::exchange(o.p, nullptr); n = std::exchange(o.n, 0); } return *this; }
+    ~Buf() { release(); }
+    cudaError_t alloc(size_t count, unsigned flags = 0)
+    {
+        release();
+        void* q = nullptr;
+        const cudaError_t e = !count ? cudaSuccess : Pinned ? cudaHostAlloc(&q, count * sizeof(T), flags) : cudaMalloc(&q, count * sizeof(T));
+        if (e == cudaSuccess && count) { p = static_cast<T*>(q); n = count; g_held_bytes += (int64_t)(n * sizeof(T)); }
+        return e;
+    }
     cudaError_t upload(const std::vector<T>& v, cudaStream_t s)
     {
         cudaError_t e = alloc(v.size());
         if (e != cudaSuccess || v.empty()) return e;
         return cudaMemcpyAsync(p, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice, s);
     }
-    void release() { if (p) cudaFree(p); p = nullptr; n = 0; }
+    void release() { if (p) { if (Pinned) cudaFreeHost(p); else cudaFree(p); g_held_bytes -= (int64_t)(n * sizeof(T)); } p = nullptr; n = 0; }
+};
+template <class T> using DevBuf = Buf<T, false>;
+template <class T> using PinnedBuf = Buf<T, true>;
+
+// Owns a stream, event, graph or graph exec; converts to the raw handle.
+template <class H, cudaError_t (*Destroy)(H)> struct Handle {
+    H raw = nullptr;
+    Handle() = default;
+    Handle(const Handle&) = delete; Handle& operator=(const Handle&) = delete;
+    Handle(Handle&& o) noexcept : raw(std::exchange(o.raw, nullptr)) {}
+    ~Handle() { reset(); }
+    void reset(H v = nullptr) { if (raw) Destroy(raw); raw = v; }
+    operator H() const { return raw; }
+};
+using Stream = Handle<cudaStream_t, cudaStreamDestroy>;
+using Event = Handle<cudaEvent_t, cudaEventDestroy>;
+using Graph = Handle<cudaGraph_t, cudaGraphDestroy>;
+using GraphExec = Handle<cudaGraphExec_t, cudaGraphExecDestroy>;
+
+// Events of the timers: one slot per timed evaluation, reused from every timer_begin on, at most 8192 per window.
+struct TimedSlot { Event begin, end, mid; };
+struct EventPool {
+    std::vector<TimedSlot> slots; size_t used = 0;
+    // the next slot (with `mid` also the event between the two stages of the general pipeline); nullptr when full
+    TimedSlot* next(bool mid)
+    {
+        if (used == slots.size() && used < 8192) { slots.emplace_back(); cudaEventCreate(&slots.back().begin.raw); cudaEventCreate(&slots.back().end.raw); }
+        if (used == slots.size()) return nullptr;
+        TimedSlot& s = slots[used++];
+        if (mid && !s.mid) cudaEventCreate(&s.mid.raw);
+        return &s;
+    }
 };
 }  // namespace
 
 struct wfsa_dev {
+    Stream stream;                             // first, so that it is destroyed after everything that uses it
     std::string err;
     int device = 0, sm_count = 0, kernel = 0, accum = 0;
     wfsa_dev_options opt{};
-    cudaStream_t stream = nullptr;
     HostFsa fsa;
     FastLayout fast;
     GenericLayout gen;
@@ -112,8 +160,8 @@ struct wfsa_dev {
     DevBuf<double> d_k3lat; DevBuf<int> d_k3exp;
     DevBuf<double> d_gscratch;
     long long g_batch = 0;
-    double* h_out = nullptr;                   // pinned [2 + n]
-    double* h_x = nullptr;                     // pinned and mapped [n + 1]
+    PinnedBuf<double> h_out;                   // [2 + n]
+    PinnedBuf<double> h_x;                     // mapped [n + 1]
     double* h_x_dev = nullptr;                 // device address of h_x (the host-buffer call lets the kernel fetch x itself)
     double fx_log2 = 0, ll_log2 = 44;
     int grid = 0, block = 0, stack_cap = 0, n_acc_smem = 0;      // warp-per-string (K2) launch
@@ -175,22 +223,20 @@ struct wfsa_dev {
     std::vector<uint32_t> hrw; std::vector<int64_t> hrgoff; std::vector<int32_t> hrgrows; std::vector<double> hrW;
     std::vector<int32_t> h_ttp, h_etp;
     bool hb_from_types = false, hb_user = false;
-    DevBuf<int32_t> d_hb_slot; DevBuf<double> d_type_lrmin, d_zero_logaw, d_rmin_part;
+    DevBuf<int32_t> d_hb_slot; DevBuf<double> d_type_lrmin, d_zero_logaw;
     int hb_fx_log2 = 40;
     // comm
     ncclComm_t comm = nullptr; int rank = 0, nranks = 1;
     // NVLink peer memory for the exchange inside k_eval6 (and the rank barrier of the benchmark); without it ncclAllReduce
     bool peer_ok = false; int peer_words = 0; size_t peer_ll_off = 0, peer_bar_off = 0; unsigned long long peer_bar_epoch = 0;
-    unsigned long long* peer_local = nullptr; unsigned long long* peer_ptrs[8] = {nullptr};
+    DevBuf<unsigned long long> peer_local; unsigned long long* peer_ptrs[8] = {nullptr};
     // timing
-    cudaEvent_t ev_begin = nullptr, ev_end = nullptr;
-    std::vector<std::pair<cudaEvent_t, cudaEvent_t>> kev;
-    size_t kev_used = 0; bool timing = false;
-    std::vector<cudaEvent_t> kev_mid;           // segmented path: behind kr_regions (what follows inside the bracket: overflow strings)
+    Event ev_begin, ev_end; bool timing = false;
+    EventPool kev;          // around the dominant kernel(s); mid, segmented path: behind kr_regions (what follows: overflow strings)
     cudaEvent_t mid_now = nullptr;
     DevBuf<unsigned char> d_flush; DevBuf<unsigned int> d_flush_sink; int flush_byte = 0;
     DevBuf<unsigned long long> d_bar;          // rank barrier without peer memory: a one-word ncclAllReduce
-    std::vector<std::pair<cudaEvent_t, cudaEvent_t>> sev; size_t sev_used = 0;      // per-evaluation event pairs (timer)
+    EventPool sev;                              // around each whole evaluation
     DevBuf<long long> d_llpart;             // bridge part of the log-likelihood: per-CTA partials of the weight kernel
     int llpart_n = 0;
     bool timing_detail = true;
@@ -219,13 +265,22 @@ struct wfsa_dev {
     DevBuf<Eval6Cls> d_e6cls;
     int e6_ncls = 0, e6_big_slots = 0, e6_big_rows = 0; size_t e6_smem = 0;
     bool e6_ok = false, any_overflow = false, e6_used = false, comm_failed = false;
-    cudaGraph_t e6_graph = nullptr; cudaGraphExec_t e6_exec = nullptr; bool e6_graph_tried = false;
+    Graph e6_graph; GraphExec e6_exec; bool e6_graph_tried = false;
     // host-buffer call: the graph's kernel writes [loglik, bad, grad, time-out epoch] and a completion word straight into mapped pinned memory
-    double* hm_out = nullptr; double* hm_out_dev = nullptr; unsigned int* hm_flag = nullptr; unsigned int* hm_flag_dev = nullptr; size_t hm_n = 0;
+    PinnedBuf<double> hm_out; double* hm_out_dev = nullptr; PinnedBuf<unsigned int> hm_flag; unsigned int* hm_flag_dev = nullptr; size_t hm_n = 0;
     bool out_on_host = false;               // the results of the last evaluation are in h_out only (graph path)
     unsigned int hm_runs = 0;               // host-buffer launches of k_eval6 since the control words were last reset
     double e2e_ns[4] = {0, 0, 0, 0}; long long e2e_calls = 0;   // WFSA_E2E_DEBUG: host time of the host-buffer call [stage x, graph launch, wait, copy out]
-    cudaEvent_t ev_x = nullptr; bool x_in_flight = false;
+    Event ev_x; bool x_in_flight = false;
+    // only the steps whose order matters: the members free themselves afterwards (the stream last)
+    ~wfsa_dev()
+    {
+        if (ks_thread.joinable()) ks_thread.join();
+        cudaSetDevice(device);
+        if (stream) cudaStreamSynchronize(stream);
+        for (int r = 0; r < 8; ++r) if (peer_ptrs[r] && r != rank) cudaIpcCloseMemHandle(peer_ptrs[r]);
+        if (comm && g_nccl.CommDestroy) g_nccl.CommDestroy(comm);
+    }
 };
 
 #define CK(call)                                                                              \
@@ -252,54 +307,9 @@ extern "C" const char* wfsa_dev_version(void) { return "wfsa_b200 0.1 (sm_100a)"
 
 extern "C" const char* wfsa_dev_last_error(const wfsa_dev* h) { return h ? h->err.c_str() : g_create_error.c_str(); }
 
-extern "C" void wfsa_dev_destroy(wfsa_dev* h)
-{
-    if (!h) return;
-    if (h->ks_thread.joinable()) h->ks_thread.join();
-    cudaSetDevice(h->device);
-    if (h->stream) cudaStreamSynchronize(h->stream);
-    for (int r = 0; r < 8; ++r) if (h->peer_ptrs[r] && r != h->rank) cudaIpcCloseMemHandle(h->peer_ptrs[r]);
-    if (h->peer_local) cudaFree(h->peer_local);
-    if (h->comm && g_nccl.CommDestroy) g_nccl.CommDestroy(h->comm);
-    DevBuf<int32_t>* i32[] = {&h->d_tokens, &h->d_order, &h->d_slot_emis, &h->d_slot_final, &h->d_arc_tid, &h->d_arc_eid,
-                              &h->d_emis_row, &h->d_emis_tok_off, &h->d_emis_tok, &h->d_trans_row, &h->d_trans_dst,
-                              &h->d_eps_order, &h->d_trans_tp, &h->d_emis_tp, &h->d_edge_tp, &h->d_edge_raw, &h->d_hb_cols};
-    for (auto* b : i32) b->release();
-    DevBuf<uint32_t>* u32[] = {&h->d_cand_off, &h->d_slot_state, &h->d_frow, &h->d_fent, &h->d_brow, &h->d_bent};
-    h->d_brow16.release(); h->d_sstate16.release(); h->d_bent8.release(); h->d_adst16.release();
-    h->d_order_w.release(); h->d_fws.release(); h->d_state_final.release(); h->d_ktlat.release();
-    h->d_ktcnt.release(); h->d_tokT.release(); h->d_goff.release();
-    h->d_klwords.release(); h->d_klcounter.release(); h->d_klgoff.release(); h->d_klgsid.release();
-    h->d_kl_arc_tid.release(); h->d_kl_arc_eid.release(); h->d_klaw.release(); h->d_klxs.release();
-    h->d_klacc.release(); h->d_klconst.release();
-    h->d_krwords.release(); h->d_kswords.release(); h->d_krgoff.release(); h->d_ksgoff.release(); h->d_krgrows.release();
-    h->d_ksgref.release(); h->d_kssid.release(); h->d_krW.release(); h->d_krlq.release(); h->d_ksp.release();
-    h->d_kslogq.release(); h->d_klogaw.release(); h->d_eoff.release(); h->d_earc.release();
-    for (auto* b : u32) b->release();
-    h->d_k7pef.release(); h->d_k7prf.release(); h->d_k7peb.release(); h->d_k7prb.release();
-    DevBuf<double>* f64[] = {&h->d_p, &h->d_x, &h->d_tw, &h->d_sw, &h->d_fw, &h->d_ltw, &h->d_lew, &h->d_logq, &h->d_pathcnt,
-                             &h->d_out, &h->d_k3lat, &h->d_gscratch, &h->d_aw, &h->d_hb_counts, &h->d_hb_p, &h->d_hb_r, &h->d_H, &h->d_rmin};
-    for (auto* b : f64) b->release();
-    DevBuf<int64_t>* i64[] = {&h->d_offs, &h->d_hb_path_off, &h->d_hb_col_off, &h->d_hb_val_off};
-    for (auto* b : i64) b->release();
-    h->d_acc.release(); h->d_red.release(); h->d_glstack.release(); h->d_Hfx.release(); h->d_used.release(); h->d_k3exp.release();
-    if (h->h_out) cudaFreeHost(h->h_out);
-    if (h->h_x) cudaFreeHost(h->h_x);
-    if (h->ev_begin) cudaEventDestroy(h->ev_begin);
-    if (h->ev_end) cudaEventDestroy(h->ev_end);
-    for (auto& e : h->kev) { cudaEventDestroy(e.first); cudaEventDestroy(e.second); }
-    for (auto& e : h->kev_mid) cudaEventDestroy(e);
-    h->d_llpart.release(); h->d_flush.release(); h->d_flush_sink.release(); h->d_bar.release();
-    for (auto& e : h->sev) { cudaEventDestroy(e.first); cudaEventDestroy(e.second); }
-    h->d_e6ctl.release(); h->d_e6acc.release(); h->d_e6red.release(); h->d_e6stamps.release(); h->d_arc_tp.release(); h->d_e6cls.release();
-    if (h->e6_exec) cudaGraphExecDestroy(h->e6_exec);
-    if (h->e6_graph) cudaGraphDestroy(h->e6_graph);
-    if (h->ev_x) cudaEventDestroy(h->ev_x);
-    if (h->hm_out) cudaFreeHost(h->hm_out);
-    if (h->hm_flag) cudaFreeHost(h->hm_flag);
-    if (h->stream) cudaStreamDestroy(h->stream);
-    delete h;
-}
+extern "C" void wfsa_dev_destroy(wfsa_dev* h) { if (h) delete h; }
+
+extern "C" int64_t wfsa_dev_held_bytes(void) { return g_held_bytes.load(); }
 
 // ---------------------------------------------------------------------------------------------
 static int setup_k2(wfsa_dev* h)
@@ -412,25 +422,24 @@ static int setup_k7_planes(wfsa_dev* h)
     size_t free_b = 0, total_b = 0;
     if (cudaMemGetInfo(&free_b, &total_b) != cudaSuccess) { cudaGetLastError(); return WFSA_OK; }
     if (2 * words * 4 > free_b / 8) return WFSA_OK;
-    DevBuf<int> d_kmax;
-    if (h->d_k7pef.alloc(n_keys * V * kK7Planes) != cudaSuccess || h->d_k7prf.alloc(n_keys * V) != cudaSuccess ||
-        h->d_k7peb.alloc(n_keys * V * kK7Planes) != cudaSuccess || h->d_k7prb.alloc(n_keys * V) != cudaSuccess ||
+    DevBuf<uint32_t> pef, prf, peb, prb; DevBuf<int> d_kmax;       // the planes go to the handle once they are built
+    if (pef.alloc(n_keys * V * kK7Planes) != cudaSuccess || prf.alloc(n_keys * V) != cudaSuccess ||
+        peb.alloc(n_keys * V * kK7Planes) != cudaSuccess || prb.alloc(n_keys * V) != cudaSuccess ||
         d_kmax.alloc(2 * n_keys) != cudaSuccess) {
         cudaGetLastError();
-        h->d_k7pef.release(); h->d_k7prf.release(); h->d_k7peb.release(); h->d_k7prb.release(); d_kmax.release();
         return WFSA_OK;
     }
     FastTablesD T{};
     T.cand_off = h->d_cand_off.p; T.slot_state = h->d_slot_state.p;
     T.frow = h->d_frow.p; T.fent = h->d_fent.p; T.brow = h->d_brow.p; T.bent = h->d_bent.p;
     T.n_sym = L.n_sym; T.n_states = h->fsa.n_states; T.n_arcs = L.n_arcs; T.n_slots = L.n_slots;
-    k7_build_planes<<<(unsigned)n_keys, (unsigned)V, 0, h->stream>>>(T, (int)V, 1, h->d_k7pef.p, h->d_k7prf.p, d_kmax.p);
-    k7_build_planes<<<(unsigned)n_keys, (unsigned)V, 0, h->stream>>>(T, (int)V, 0, h->d_k7peb.p, h->d_k7prb.p, d_kmax.p + n_keys);
+    k7_build_planes<<<(unsigned)n_keys, (unsigned)V, 0, h->stream>>>(T, (int)V, 1, pef.p, prf.p, d_kmax.p);
+    k7_build_planes<<<(unsigned)n_keys, (unsigned)V, 0, h->stream>>>(T, (int)V, 0, peb.p, prb.p, d_kmax.p + n_keys);
     h->k7_kf.assign(n_keys, 0); h->k7_kb.assign(n_keys, 0);
     CK(cudaMemcpyAsync(h->k7_kf.data(), d_kmax.p, n_keys * 4, cudaMemcpyDeviceToHost, h->stream));
     CK(cudaMemcpyAsync(h->k7_kb.data(), d_kmax.p + n_keys, n_keys * 4, cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
-    d_kmax.release();
+    h->d_k7pef = std::move(pef); h->d_k7prf = std::move(prf); h->d_k7peb = std::move(peb); h->d_k7prb = std::move(prb);
     h->k7_planes = true;
     return WFSA_OK;
 }
@@ -556,8 +565,9 @@ extern "C" int wfsa_dev_create(const wfsa_fsa_desc* fd, const wfsa_corpus_desc* 
     g_create_error.clear();
     if (!out) { g_create_error = "out is NULL"; return WFSA_ERR_INVALID; }
     *out = nullptr;
-    wfsa_dev* h = new wfsa_dev();
-    auto bail = [&](int code) { g_create_error = h->err; wfsa_dev_destroy(h); return code; };
+    std::unique_ptr<wfsa_dev> owner(new wfsa_dev());
+    wfsa_dev* const h = owner.get();
+    auto bail = [&](int code) { g_create_error = h->err; return code; };
     if (opt) h->opt = *opt;
     int status = WFSA_OK;
     std::string msg = copy_and_validate(fd, h->fsa, status);
@@ -582,8 +592,8 @@ extern "C" int wfsa_dev_create(const wfsa_fsa_desc* fd, const wfsa_corpus_desc* 
         return bail(WFSA_ERR_NO_DEVICE);
     }
     h->sm_count = prop.multiProcessorCount;
-    if (cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking) != cudaSuccess) { h->err = "cudaStreamCreate failed"; return bail(WFSA_ERR_CUDA); }
-    cudaEventCreate(&h->ev_begin); cudaEventCreate(&h->ev_end);
+    if (cudaStreamCreateWithFlags(&h->stream.raw, cudaStreamNonBlocking) != cudaSuccess) { h->err = "cudaStreamCreate failed"; return bail(WFSA_ERR_CUDA); }
+    cudaEventCreate(&h->ev_begin.raw); cudaEventCreate(&h->ev_end.raw);
 
     // ---- layout
     msg = build_fast_layout(h->fsa, h->fast, status);
@@ -676,7 +686,7 @@ extern "C" int wfsa_dev_create(const wfsa_fsa_desc* fd, const wfsa_corpus_desc* 
     if (choose_launch(h) != WFSA_OK) return bail(WFSA_ERR_CUDA);
     CKB(cudaStreamSynchronize(st));
 #undef CKB
-    *out = h;
+    *out = owner.release();
     return WFSA_OK;
 }
 
@@ -946,10 +956,8 @@ static int launch_pipeline(wfsa_dev* h, int mode, int kernel, const int32_t* d_o
     if (lean6 && h->e6_ok) {
         if (h->comm_failed) return set_err(h, WFSA_ERR_NCCL, "an earlier exchange over peer memory timed out: the ranks are out of step");
         cudaEvent_t e0 = nullptr, e1 = nullptr;
-        if (h->timing && h->timing_detail) {
-            if (h->kev_used == h->kev.size() && h->kev.size() < 8192) { cudaEvent_t a, b; cudaEventCreate(&a); cudaEventCreate(&b); h->kev.push_back({a, b}); }
-            if (h->kev_used < h->kev.size()) { e0 = h->kev[h->kev_used].first; e1 = h->kev[h->kev_used].second; h->kev_used++; }
-        }
+        if (h->timing && h->timing_detail)
+            if (const TimedSlot* s = h->kev.next(false)) { e0 = s->begin; e1 = s->end; }
         if (e0) cudaEventRecord(e0, st);
         {
             const cudaError_t le = launch_eval6(h, st);
@@ -1013,13 +1021,8 @@ static int launch_pipeline(wfsa_dev* h, int mode, int kernel, const int32_t* d_o
     O.fx_scale = (mode == MODE_STRUCT) ? 1.0 : std::ldexp(1.0, (int)h->fx_log2);
     O.ll_scale = std::ldexp(1.0, (int)h->ll_log2);
     cudaEvent_t e0 = nullptr, e1 = nullptr;
-    if (h->timing && h->timing_detail && mode == MODE_EVAL) {
-        if (h->kev_used == h->kev.size() && h->kev.size() < 8192) {
-            cudaEvent_t a, b; cudaEventCreate(&a); cudaEventCreate(&b); h->kev.push_back({a, b});
-        }
-        while (h->kev_mid.size() < h->kev.size()) { cudaEvent_t m; cudaEventCreate(&m); h->kev_mid.push_back(m); }
-        if (h->kev_used < h->kev.size()) { e0 = h->kev[h->kev_used].first; e1 = h->kev[h->kev_used].second; h->mid_now = h->kev_mid[h->kev_used]; h->kev_used++; }
-    }
+    if (h->timing && h->timing_detail && mode == MODE_EVAL)
+        if (const TimedSlot* s = h->kev.next(true)) { e0 = s->begin; e1 = s->end; h->mid_now = s->mid; }
     if (e0) cudaEventRecord(e0, st);
     h->lean_now = false;
     launch_main(h, kernel, mode, CorpusD{h->d_tokens.p, h->d_offs.p, h->d_p.p, d_order, n_order}, O);
@@ -1258,6 +1261,7 @@ extern "C" int wfsa_dev_set_param_map(wfsa_dev* h, const int32_t* trimmed, int32
         }
         h->n_active = (int64_t)good.size(); h->n_active_w = (int64_t)order_w.size();
         if (!order_w.empty()) CK(cudaMemcpyAsync(h->d_order_w.p, order_w.data(), order_w.size() * 4, cudaMemcpyHostToDevice, h->stream));
+        // the batches and the lattice of a previous map go first: the budget below counts their memory as free
         h->k7.clear();
         h->d_k7lat.release(); h->d_k7bt.release(); h->d_k7exp.release(); h->d_k7scale.release(); h->d_k7EQ.release(); h->d_k7F.release();
         size_t free_b = 0, total_b = 0;
@@ -1372,19 +1376,15 @@ extern "C" int wfsa_dev_set_param_map(wfsa_dev* h, const int32_t* trimmed, int32
         CK(cudaStreamSynchronize(h->stream));
     }
     if (h->n != n) {
-        if (h->h_out) cudaFreeHost(h->h_out);
-        if (h->h_x) cudaFreeHost(h->h_x);
-        h->h_out = nullptr; h->h_x = nullptr;
-        CK(cudaMallocHost(&h->h_out, ((size_t)n + 3) * 8));      // [loglik, non-finite terms, grad[n], epoch of a timed-out exchange]
-        CK(cudaHostAlloc(&h->h_x, ((size_t)n + 1) * 8, cudaHostAllocMapped));        // [x[n], log2 of the fixed-point scale of loglik]
+        CK(h->h_out.alloc((size_t)n + 3));                       // [loglik, non-finite terms, grad[n], epoch of a timed-out exchange]
+        CK(h->h_x.alloc((size_t)n + 1, cudaHostAllocMapped));    // [x[n], log2 of the fixed-point scale of loglik]
         h->h_x_dev = nullptr;
-        if (cudaHostGetDevicePointer(&h->h_x_dev, h->h_x, 0) != cudaSuccess) { cudaGetLastError(); h->h_x_dev = nullptr; }
+        if (cudaHostGetDevicePointer(&h->h_x_dev, h->h_x.p, 0) != cudaSuccess) { cudaGetLastError(); h->h_x_dev = nullptr; }
         CK(h->d_x.alloc((size_t)n + 1));
         CK(h->d_out.alloc((size_t)n + 3));
     }
     CK(cudaMemsetAsync(h->d_out.p, 0, h->d_out.n * 8, h->stream));
-    if (h->e6_exec) { cudaGraphExecDestroy(h->e6_exec); h->e6_exec = nullptr; }
-    if (h->e6_graph) { cudaGraphDestroy(h->e6_graph); h->e6_graph = nullptr; }
+    h->e6_exec.reset(); h->e6_graph.reset();
     h->e6_graph_tried = false;
     h->n = n;
     h->evaluated = false;
@@ -1421,7 +1421,7 @@ static int stage_x(wfsa_dev* h, const double* x)
     double mx = 0.0;
     {
         const int n = h->n;
-        double* __restrict__ dst = h->h_x;
+        double* __restrict__ dst = h->h_x.p;
         double m0 = 0.0, m1 = 0.0, m2 = 0.0, m3 = 0.0;
         int i = 0;
         for (; i + 4 <= n; i += 4) {
@@ -1443,7 +1443,7 @@ static int stage_x(wfsa_dev* h, const double* x)
     int bits = 1;
     while (std::ldexp(1.0, bits) <= B && bits < 40) ++bits;
     h->ll_log2 = finite ? 62 - bits : 22;
-    h->h_x[h->n] = h->ll_log2;
+    h->h_x.p[h->n] = h->ll_log2;
     return WFSA_OK;
 }
 
@@ -1452,8 +1452,8 @@ extern "C" int wfsa_dev_upload_x(wfsa_dev* h, const double* x)
     const int rc = stage_x(h, x);
     if (rc != WFSA_OK) return rc;
     CK(cudaSetDevice(h->device));
-    CK(cudaMemcpyAsync(h->d_x.p, h->h_x, ((size_t)h->n + 1) * 8, cudaMemcpyHostToDevice, h->stream));
-    if (!h->ev_x) CK(cudaEventCreateWithFlags(&h->ev_x, cudaEventDisableTiming));
+    CK(cudaMemcpyAsync(h->d_x.p, h->h_x.p, ((size_t)h->n + 1) * 8, cudaMemcpyHostToDevice, h->stream));
+    if (!h->ev_x) CK(cudaEventCreateWithFlags(&h->ev_x.raw, cudaEventDisableTiming));
     CK(cudaEventRecord(h->ev_x, h->stream));
     h->x_in_flight = true;
     return WFSA_OK;
@@ -1467,8 +1467,8 @@ static int setup_peer_allreduce(wfsa_dev* h)
     h->peer_ok = false;
     if (!h->comm || h->nranks > 8 || getenv("WFSA_NO_PEER")) return WFSA_OK;
     const int words = (int)h->d_red.n;
-    if (h->peer_local && h->peer_words == words) { h->peer_ok = true; return WFSA_OK; }
-    if (h->peer_local) return WFSA_OK;                       // sized for another parameter map: keep NCCL (rare)
+    if (h->peer_local.p && h->peer_words == words) { h->peer_ok = true; return WFSA_OK; }
+    if (h->peer_local.p) return WFSA_OK;                     // sized for another parameter map: keep NCCL (rare)
     // [packets of k_eval6: 2 parities x nranks senders x words x 2][words of k_peer_barrier: 2 x nranks]
     h->peer_ll_off = 0;
     h->peer_bar_off = h->peer_ll_off + (size_t)4 * h->nranks * words;       // then the words of k_peer_barrier: 2 x nranks
@@ -1476,9 +1476,9 @@ static int setup_peer_allreduce(wfsa_dev* h)
     unsigned long long ok = 1;
     cudaIpcMemHandle_t mine;
     std::memset(&mine, 0, sizeof(mine));
-    if (cudaMalloc(&h->peer_local, total * 8) != cudaSuccess) { h->peer_local = nullptr; ok = 0; }
-    if (ok && cudaMemset(h->peer_local, 0, total * 8) != cudaSuccess) ok = 0;
-    if (ok && cudaIpcGetMemHandle(&mine, h->peer_local) != cudaSuccess) ok = 0;
+    if (h->peer_local.alloc(total) != cudaSuccess) ok = 0;
+    if (ok && cudaMemset(h->peer_local.p, 0, total * 8) != cudaSuccess) ok = 0;
+    if (ok && cudaIpcGetMemHandle(&mine, h->peer_local.p) != cudaSuccess) ok = 0;
     cudaGetLastError();
     // table: per rank 8 words of handle + 1 word "ok"
     const int per = (int)(sizeof(cudaIpcMemHandle_t) / 8) + 1;
@@ -1488,16 +1488,15 @@ static int setup_peer_allreduce(wfsa_dev* h)
     DevBuf<unsigned long long> d_tab;
     CK(d_tab.upload(tab, h->stream));
     int rc = nccl_allreduce(h, d_tab.p, tab.size(), ncclUint64, ncclSum);
-    if (rc != WFSA_OK) { d_tab.release(); return rc; }
+    if (rc != WFSA_OK) return rc;
     CK(cudaMemcpyAsync(tab.data(), d_tab.p, tab.size() * 8, cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
-    d_tab.release();
     unsigned long long all_ok = 1;
     for (int r = 0; r < h->nranks; ++r) all_ok &= tab[(size_t)r * per + per - 1];
     unsigned long long mapped = all_ok;
     if (all_ok)
         for (int r = 0; r < h->nranks; ++r) {
-            if (r == h->rank) { h->peer_ptrs[r] = h->peer_local; continue; }
+            if (r == h->rank) { h->peer_ptrs[r] = h->peer_local.p; continue; }
             cudaIpcMemHandle_t hd;
             std::memcpy(&hd, &tab[(size_t)r * per], sizeof(hd));
             void* ptr = nullptr;
@@ -1526,12 +1525,8 @@ extern "C" int wfsa_dev_eval_launch(wfsa_dev* h)
     if (h->n < 0) return set_err(h, WFSA_ERR_STATE, "eval before set_param_map");
     CK(cudaSetDevice(h->device));
     cudaEvent_t s1 = nullptr;
-    if (h->timing) {                               // one event pair around the whole evaluation (weights, kernels, fold, collective)
-        if (h->sev_used == h->sev.size() && h->sev.size() < 8192) {
-            cudaEvent_t a, b; cudaEventCreate(&a); cudaEventCreate(&b); h->sev.push_back({a, b});
-        }
-        if (h->sev_used < h->sev.size()) { cudaEventRecord(h->sev[h->sev_used].first, h->stream); s1 = h->sev[h->sev_used].second; h->sev_used++; }
-    }
+    if (h->timing)                                 // one event pair around the whole evaluation (weights, kernels, fold, collective)
+        if (const TimedSlot* s = h->sev.next(false)) { cudaEventRecord(s->begin, h->stream); s1 = s->end; }
     h->out_on_host = false;
     const int rc = eval_launch_body(h);
     if (s1) cudaEventRecord(s1, h->stream);
@@ -1588,20 +1583,20 @@ static int ensure_ks(wfsa_dev* h)
 static int finish_fetch(wfsa_dev* h, double* loglik, double* grad, const double* src = nullptr)
 {
     if (src) {                                                 // results in mapped memory: one pass fills the caller's buffers and h_out
-        h->h_out[0] = src[0]; h->h_out[1] = src[1]; h->h_out[h->n + 2] = src[h->n + 2];
-        double* __restrict__ keep = h->h_out + 2;
+        h->h_out.p[0] = src[0]; h->h_out.p[1] = src[1]; h->h_out.p[h->n + 2] = src[h->n + 2];
+        double* __restrict__ keep = h->h_out.p + 2;
         const double* __restrict__ g = src + 2;
         if (grad) for (int i = 0; i < h->n; ++i) { const double v = g[i]; keep[i] = v; grad[i] = v; }
         else std::memcpy(keep, g, (size_t)h->n * 8);
         grad = nullptr;
     }
-    if (h->comm && (std::isnan(h->h_out[1]) || h->h_out[h->n + 2] != 0.0)) {
+    if (h->comm && (std::isnan(h->h_out.p[1]) || h->h_out.p[h->n + 2] != 0.0)) {
         // the ranks no longer agree on the epoch of the exchange: later evaluations of this handle fail as well
         h->comm_failed = true;
         return set_err(h, WFSA_ERR_NCCL, "all-reduce over peer memory: a rank did not deliver its share within the time limit");
     }
-    if (loglik) *loglik = h->h_out[0];
-    if (grad) std::memcpy(grad, h->h_out + 2, (size_t)h->n * 8);
+    if (loglik) *loglik = h->h_out.p[0];
+    if (grad) std::memcpy(grad, h->h_out.p + 2, (size_t)h->n * 8);
     return WFSA_OK;
 }
 
@@ -1610,7 +1605,7 @@ extern "C" int wfsa_dev_eval_fetch(wfsa_dev* h, double* loglik, double* logq, do
     if (!h) return WFSA_ERR_INVALID;
     if (h->n < 0) return set_err(h, WFSA_ERR_STATE, "fetch before set_param_map");
     if (!h->evaluated) return set_err(h, WFSA_ERR_STATE, "fetch before an evaluation was launched for this parameter map");
-    if (!h->out_on_host) CK(cudaMemcpyAsync(h->h_out, h->d_out.p, ((size_t)h->n + 3) * 8, cudaMemcpyDeviceToHost, h->stream));
+    if (!h->out_on_host) CK(cudaMemcpyAsync(h->h_out.p, h->d_out.p, ((size_t)h->n + 3) * 8, cudaMemcpyDeviceToHost, h->stream));
     if (logq && h->kernel == 6) { const int rc = ensure_ks(h); if (rc != WFSA_OK) return rc; }
     if (logq && h->kernel == 6 && h->ks_groups > 0) {
         if (!h->ks_done) {                       // per-string log q of the segmented path, from the lq of the last evaluation
@@ -1648,15 +1643,13 @@ static bool eval6_graph(wfsa_dev* h)
     if (cudaStreamSynchronize(h->stream) != cudaSuccess) return false;
     const size_t words = (size_t)h->n + 3;
     if (h->hm_n != words) {
-        if (h->hm_out) cudaFreeHost(h->hm_out);
-        if (h->hm_flag) cudaFreeHost(h->hm_flag);
-        h->hm_out = nullptr; h->hm_flag = nullptr; h->hm_n = 0;
-        if (cudaHostAlloc(&h->hm_out, words * 8, cudaHostAllocMapped) != cudaSuccess ||
-            cudaHostAlloc(&h->hm_flag, 64, cudaHostAllocMapped) != cudaSuccess ||
-            cudaHostGetDevicePointer(&h->hm_out_dev, h->hm_out, 0) != cudaSuccess ||
-            cudaHostGetDevicePointer(&h->hm_flag_dev, h->hm_flag, 0) != cudaSuccess) { cudaGetLastError(); return false; }
-        std::memset(h->hm_out, 0, words * 8);
-        *h->hm_flag = 0u;
+        h->hm_n = 0;
+        if (h->hm_out.alloc(words, cudaHostAllocMapped) != cudaSuccess ||
+            h->hm_flag.alloc(16, cudaHostAllocMapped) != cudaSuccess ||
+            cudaHostGetDevicePointer(&h->hm_out_dev, h->hm_out.p, 0) != cudaSuccess ||
+            cudaHostGetDevicePointer(&h->hm_flag_dev, h->hm_flag.p, 0) != cudaSuccess) { cudaGetLastError(); return false; }
+        std::memset(h->hm_out.p, 0, words * 8);
+        *h->hm_flag.p = 0u;
         h->hm_n = words;
     }
     if (cudaStreamBeginCapture(h->stream, cudaStreamCaptureModeThreadLocal) != cudaSuccess) { cudaGetLastError(); return false; }
@@ -1664,13 +1657,14 @@ static bool eval6_graph(wfsa_dev* h)
     // A copy node in front of the kernel cost 12.5 us per call (measured: the DMA set-up and the dependency between the two
     // nodes), the fetch inside the kernel ~3 us.  (WFSA_E2E_COPY_NODE=1 brings the copy node back.)
     const bool copy_node = !h->h_x_dev || getenv("WFSA_E2E_COPY_NODE");
-    if (copy_node) cudaMemcpyAsync(h->d_x.p, h->h_x, ((size_t)h->n + 1) * 8, cudaMemcpyHostToDevice, h->stream);
+    if (copy_node) cudaMemcpyAsync(h->d_x.p, h->h_x.p, ((size_t)h->n + 1) * 8, cudaMemcpyHostToDevice, h->stream);
     launch_eval6(h, h->stream, false, true, !copy_node);
     cudaGraph_t g = nullptr;
     if (cudaStreamEndCapture(h->stream, &g) != cudaSuccess || !g) { cudaGetLastError(); return false; }
+    h->e6_graph.reset(g);
     cudaGraphExec_t ex = nullptr;
-    if (cudaGraphInstantiate(&ex, g, 0) != cudaSuccess) { cudaGetLastError(); cudaGraphDestroy(g); return false; }
-    h->e6_graph = g; h->e6_exec = ex;
+    if (cudaGraphInstantiate(&ex, g, 0) != cudaSuccess) { cudaGetLastError(); h->e6_graph.reset(); return false; }
+    h->e6_exec.reset(ex);
     return true;
 }
 
@@ -1685,13 +1679,13 @@ extern "C" int wfsa_dev_eval(wfsa_dev* h, const double* x, double* loglik, doubl
             const int rc = stage_x(h, x);
             if (rc != WFSA_OK) return rc;
             const auto tp1 = std::chrono::steady_clock::now();
-            const unsigned int before = *reinterpret_cast<volatile unsigned int*>(h->hm_flag);   // the kernel writes a new count when it is through
+            const unsigned int before = *reinterpret_cast<volatile unsigned int*>(h->hm_flag.p);   // the kernel writes a new count when it is through
             ++h->hm_runs;
             CK(cudaGraphLaunch(h->e6_exec, h->stream));
             const auto tp2 = std::chrono::steady_clock::now();
             h->launches++; h->e6_used = true; h->evaluated = true; h->ks_done = false; h->lean_now = true; h->lean_finished = true;
             // wait for the completion word of this epoch; every now and then ask the stream whether it failed instead
-            volatile unsigned int* flag = h->hm_flag;
+            volatile unsigned int* flag = h->hm_flag.p;
             for (unsigned long long spin = 1; *flag == before; ++spin)
                 if ((spin & 0xfffffull) == 0) {
                     const cudaError_t q = cudaStreamQuery(h->stream);
@@ -1700,7 +1694,7 @@ extern "C" int wfsa_dev_eval(wfsa_dev* h, const double* x, double* loglik, doubl
             const auto tp3 = std::chrono::steady_clock::now();
             // (the same values are NOT in d_out: a later wfsa_dev_eval_fetch finds them in h_out)
             h->out_on_host = true;
-            const int frc = finish_fetch(h, loglik, grad, h->hm_out);
+            const int frc = finish_fetch(h, loglik, grad, h->hm_out.p);
             if (e2e_dbg) {
                 const auto tp4 = std::chrono::steady_clock::now();
                 auto ns = [](auto a, auto b) { return (double)std::chrono::duration_cast<std::chrono::nanoseconds>(b - a).count(); };
@@ -1995,10 +1989,9 @@ extern "C" int wfsa_dev_allreduce_f64(wfsa_dev* h, double* values, int n, int op
     CK(tmp.alloc(n));
     CK(cudaMemcpyAsync(tmp.p, values, (size_t)n * 8, cudaMemcpyHostToDevice, h->stream));
     const int rc = nccl_allreduce(h, tmp.p, n, 8 /* ncclFloat64 */, op == 1 ? ncclMax : ncclSum);
-    if (rc != WFSA_OK) { tmp.release(); return rc; }
+    if (rc != WFSA_OK) return rc;
     CK(cudaMemcpyAsync(values, tmp.p, (size_t)n * 8, cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
-    tmp.release();
     return WFSA_OK;
 }
 
@@ -2043,7 +2036,7 @@ extern "C" int wfsa_dev_eval6_phases(wfsa_dev* h, double* out4, int reset)
 extern "C" int wfsa_dev_timer_begin(wfsa_dev* h)
 {
     if (!h) return WFSA_ERR_INVALID;
-    h->timing = true; h->kev_used = 0; h->sev_used = 0; h->timing_detail = true;
+    h->timing = true; h->kev.used = 0; h->sev.used = 0; h->timing_detail = true;
     CK(cudaEventRecord(h->ev_begin, h->stream));
     return WFSA_OK;
 }
@@ -2071,14 +2064,15 @@ extern "C" int wfsa_dev_timer_kernel_ms(wfsa_dev* h, float* ms, int64_t* launche
 {
     if (!h) return WFSA_ERR_INVALID;
     float total = 0.f;
-    for (size_t i = 0; i < h->kev_used; ++i) {
+    for (size_t i = 0; i < h->kev.used; ++i) {
+        const TimedSlot& s = h->kev.slots[i];
         float t = 0.f;
-        CK(cudaEventSynchronize(h->kev[i].second));
-        CK(cudaEventElapsedTime(&t, h->kev[i].first, h->kev[i].second));
+        CK(cudaEventSynchronize(s.end));
+        CK(cudaEventElapsedTime(&t, s.begin, s.end));
         total += t;
     }
     if (ms) *ms = total;
-    if (launches) *launches = (int64_t)h->kev_used;
+    if (launches) *launches = (int64_t)h->kev.used;
     return WFSA_OK;
 }
 
@@ -2086,14 +2080,15 @@ extern "C" int wfsa_dev_timer_step_ms(wfsa_dev* h, float* ms, int64_t* steps)
 {
     if (!h) return WFSA_ERR_INVALID;
     float total = 0.f;
-    for (size_t i = 0; i < h->sev_used; ++i) {
+    for (size_t i = 0; i < h->sev.used; ++i) {
+        const TimedSlot& s = h->sev.slots[i];
         float t = 0.f;
-        CK(cudaEventSynchronize(h->sev[i].second));
-        CK(cudaEventElapsedTime(&t, h->sev[i].first, h->sev[i].second));
+        CK(cudaEventSynchronize(s.end));
+        CK(cudaEventElapsedTime(&t, s.begin, s.end));
         total += t;
     }
     if (ms) *ms = total;
-    if (steps) *steps = (int64_t)h->sev_used;
+    if (steps) *steps = (int64_t)h->sev.used;
     return WFSA_OK;
 }
 
@@ -2134,13 +2129,14 @@ extern "C" int wfsa_dev_timer_phase_ms(wfsa_dev* h, float* out3)
 {
     if (!h || !out3) return WFSA_ERR_INVALID;
     out3[0] = out3[1] = out3[2] = 0.f;
-    const size_t n = std::min(h->sev_used, h->kev_used);
+    const size_t n = std::min(h->sev.used, h->kev.used);
     for (size_t i = 0; i < n; ++i) {
+        const TimedSlot &s = h->sev.slots[i], &k = h->kev.slots[i];
         float t = 0.f;
-        CK(cudaEventSynchronize(h->sev[i].second));
-        if (cudaEventElapsedTime(&t, h->sev[i].first, h->kev[i].first) == cudaSuccess) out3[0] += t;
-        if (cudaEventElapsedTime(&t, h->kev[i].first, h->kev[i].second) == cudaSuccess) out3[1] += t;
-        if (cudaEventElapsedTime(&t, h->kev[i].second, h->sev[i].second) == cudaSuccess) out3[2] += t;
+        CK(cudaEventSynchronize(s.end));
+        if (cudaEventElapsedTime(&t, s.begin, k.begin) == cudaSuccess) out3[0] += t;
+        if (cudaEventElapsedTime(&t, k.begin, k.end) == cudaSuccess) out3[1] += t;
+        if (cudaEventElapsedTime(&t, k.end, s.end) == cudaSuccess) out3[2] += t;
     }
     cudaGetLastError();
     return WFSA_OK;
@@ -2170,11 +2166,13 @@ extern "C" int wfsa_dev_timer_split_ms(wfsa_dev* h, float* first_ms, float* seco
     if (!h) return WFSA_ERR_INVALID;
     float a = 0.f, b = 0.f;
     if (h->kernel == 6)
-        for (size_t i = 0; i < h->kev_used && i < h->kev_mid.size(); ++i) {
+        for (size_t i = 0; i < h->kev.used; ++i) {
+            const TimedSlot& k = h->kev.slots[i];
+            if (!k.mid) continue;
             float t = 0.f;
-            CK(cudaEventSynchronize(h->kev[i].second));
-            if (cudaEventElapsedTime(&t, h->kev[i].first, h->kev_mid[i]) == cudaSuccess) a += t;
-            if (cudaEventElapsedTime(&t, h->kev_mid[i], h->kev[i].second) == cudaSuccess) b += t;
+            CK(cudaEventSynchronize(k.end));
+            if (cudaEventElapsedTime(&t, k.begin, k.mid) == cudaSuccess) a += t;
+            if (cudaEventElapsedTime(&t, k.mid, k.end) == cudaSuccess) b += t;
         }
     cudaGetLastError();
     if (first_ms) *first_ms = a;

@@ -19,7 +19,7 @@ DEV_SYMBOLS = [
     "wfsa_dev_create", "wfsa_dev_structure", "wfsa_dev_set_param_map", "wfsa_dev_eval", "wfsa_dev_upload_x",
     "wfsa_dev_eval_launch", "wfsa_dev_eval_fetch", "wfsa_dev_sync", "wfsa_dev_set_path_blocks", "wfsa_dev_hessian",
     "wfsa_dev_comm_unique_id", "wfsa_dev_comm_init", "wfsa_dev_allreduce_f64", "wfsa_dev_timer_begin", "wfsa_dev_timer_begin_steps",
-    "wfsa_dev_timer_end", "wfsa_dev_timer_kernel_ms", "wfsa_dev_timer_split_ms", "wfsa_dev_timer_step_ms", "wfsa_dev_timer_phase_ms", "wfsa_dev_eval6_phases", "wfsa_dev_l2_flush", "wfsa_dev_rank_barrier", "wfsa_dev_get_info", "wfsa_dev_destroy", "wfsa_dev_last_error",
+    "wfsa_dev_timer_end", "wfsa_dev_timer_kernel_ms", "wfsa_dev_timer_split_ms", "wfsa_dev_timer_step_ms", "wfsa_dev_timer_phase_ms", "wfsa_dev_eval6_phases", "wfsa_dev_l2_flush", "wfsa_dev_rank_barrier", "wfsa_dev_get_info", "wfsa_dev_destroy", "wfsa_dev_held_bytes", "wfsa_dev_last_error",
     "wfsa_dev_version", "wfsa_lattice_compile", "wfsa_lattice_stats", "wfsa_segmented_compile", "wfsa_segmented_get",
     "wfsa_segmented_free",
 ]
@@ -109,6 +109,8 @@ def lib():
         L.wfsa_session_destroy.restype = None
         L.wfsa_dev_destroy.argtypes = [C.c_void_p]
         L.wfsa_dev_destroy.restype = None
+        L.wfsa_dev_held_bytes.argtypes = []
+        L.wfsa_dev_held_bytes.restype = C.c_int64
         L.wfsa_session_create.argtypes = [C.c_char_p, C.c_size_t, C.c_char_p, C.c_size_t, C.c_char_p,
                                           C.POINTER(SessionOptions), C.POINTER(C.c_void_p)]
         L.wfsa_host_parse.argtypes = [C.c_char_p, C.c_size_t, C.c_char_p, C.c_size_t, C.POINTER(C.c_char_p)]

@@ -68,7 +68,7 @@ typedef struct {
 typedef struct {
     int32_t device;              /* CUDA device ordinal                                       */
     int32_t force_kernel;        /* 0 auto, 1 warp-per-string, 2 CTA-per-string, 3 generic,
-                                    4 thread-per-string (table walk), 5 thread-per-string (compiled lattices),
+                                    4 thread-per-string (table walk),
                                     6 segmented compiled lattices (bridges folded into constants + region types),
                                     7 position-synchronous, pair-batched (dense automata: more than 32 states emit one symbol) */
     int32_t accum_mode;          /* 0 auto, 1 shared-memory accumulators, 2 global (L2) REDs  */
@@ -174,7 +174,7 @@ int wfsa_dev_l2_flush(wfsa_dev* h);
 /* Introspection */
 typedef struct {
     int32_t kernel;              /* 1 warp-per-string, 2 CTA-per-string, 3 generic, 4 thread-per-string
-                                    (table walk), 5 thread-per-string over compiled lattices,
+                                    (table walk),
                                     6 segmented compiled lattices (k_eval6 / kr_regions + ks_strings),
                                     7 position-synchronous pair-batched kernels (k7_fwd / k7_bwd)     */
     int32_t accum_mode;          /* 1 shared, 2 global                                          */
@@ -185,8 +185,8 @@ typedef struct {
     int64_t smem_bytes, table_bytes;
     int64_t kernels_launched;    /* total kernels this handle has launched                      */
     double  fixed_point_scale_log2;
-    /* compiled-lattice kernel (5): stream words incl. padding, lattice edges, edges whose posterior is
-       exactly 1 (folded into constant accumulators), strings handed to the secondary kernel, pool size */
+    /* segmented kernel (6): words of the region types and the per-string layout, lattice edges, edges whose posterior
+       is exactly 1 (bridges, folded into constant accumulators), strings handed to the secondary kernel, pool size */
     int64_t lattice_words, lattice_edges, lattice_bridge_edges, n_overflow_strings;
     int32_t pool_slots;
     int32_t eval_path;           /* bit 0: objective+gradient in ONE launch (k_eval6); bit 1: ranks combined through NVLink peer
@@ -205,20 +205,14 @@ typedef struct {
 } wfsa_dev_info;
 int wfsa_dev_get_info(wfsa_dev* h, wfsa_dev_info* info);
 
-/* Host-only introspection (no device needed): compiles the lattice stream of ONE string exactly as
- * wfsa_dev_set_param_map does for the compiled-lattice kernel (w-fsa_b200/csrc/lattice.hpp documents
- * the word format), so that tests can interpret the stream on the CPU.  trimmed may be NULL (no
- * parameter removed).  *n_words = words written, 0 = no accepting path, -1 = needs more than n_slots
+/* Host-only introspection (no device needed): compiles the lattice stream of ONE string in the word format
+ * that the DAG form of region types uses (w-fsa_b200/csrc/lattice.hpp documents it), so that tests can
+ * interpret the stream on the CPU.  trimmed may be NULL (no parameter removed).  *n_words = words written, 0 = no accepting path, -1 = needs more than n_slots
  * pool slots.  arc_tid / arc_eid (capacity arc_capacity, may be NULL) receive the combined-arc table:
  * arc -> (transition edge, emission edge or -1 for a final transition). */
 int wfsa_lattice_compile(const wfsa_fsa_desc* fsa, const int32_t* trimmed, const int32_t* tokens, int32_t len,
                          int32_t n_slots, uint32_t* words, int64_t capacity, int64_t* n_words,
                          int32_t* arc_tid, int32_t* arc_eid, int32_t arc_capacity, int32_t* n_arcs);
-
-/* Host-only: compiles a whole shard the way wfsa_dev_set_param_map does and reports
- * out[0..7] = lattice edges, bridge edges, stream words incl. padding, longest stream, strings
- * needing more than n_slots slots, strings without an accepting path, groups of 32, host milliseconds. */
-int wfsa_lattice_stats(const wfsa_fsa_desc* fsa, const wfsa_corpus_desc* corpus, int32_t n_slots, double* out8);
 
 /* Host-only introspection of the SEGMENTED compiled form (w-fsa_b200/csrc/lattice.hpp, kernels 6): compiles a
  * whole shard exactly as wfsa_dev_set_param_map does and exposes the arrays the device kernels read, so that

@@ -1,8 +1,8 @@
 """Host lattice compiler (w-fsa_b200/csrc/lattice.cpp) checked on the CPU: the compiled stream of every
-string is interpreted here word by word -- the same forward / backward recurrences the device kernel
-kl_fwdbwd runs (w-fsa_b200/csrc/kernels.cuh) -- and must reproduce the oracle's log q and expected
-edge counts.  This pins the stream format and the slot / flag / CHECK logic without a GPU; the
-device kernel itself is checked against the oracle in test_gpu_parity.py."""
+string is interpreted here word by word -- the same forward / backward recurrences the DAG form of region
+types runs on the device (big_fwd / big_bwd, w-fsa_b200/csrc/kernels_seg.cuh) -- and must reproduce the
+oracle's log q and expected edge counts.  This pins the stream format and the slot / flag / CHECK logic
+without a GPU; the device kernels themselves are checked against the oracle in test_gpu_parity.py."""
 import ctypes as C
 
 import numpy as np

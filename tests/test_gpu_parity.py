@@ -246,7 +246,7 @@ def medium():
     return model, low
 
 
-@pytest.mark.parametrize("kernel,accum,variant", [(6, 0, 0), (6, 0, 4 << 16), (5, 0, 0), (5, 0, 4 << 16), (5, 0, 4), (4, 0, 0), (4, 0, 4 << 16), (1, 1, 0), (1, 1, 1), (1, 2, 0), (2, 0, 0), (7, 0, 0), (3, 0, 0)])
+@pytest.mark.parametrize("kernel,accum,variant", [(6, 0, 0), (6, 0, 4 << 16), (4, 0, 0), (4, 0, 4 << 16), (1, 1, 0), (1, 1, 1), (1, 2, 0), (2, 0, 0), (7, 0, 0), (3, 0, 0)])
 def test_kernels_match_cpu_oracle(medium, kernel, accum, variant):
     model, low = medium
     count = 3000 if kernel != 3 else 300          # the generic kernel is the slow, dense one
@@ -269,13 +269,6 @@ def test_kernels_match_cpu_oracle(medium, kernel, accum, variant):
         # oracle gradient restricted to recognised strings == all strings (unrecognised contribute 0)
         ok, err = vec_tol_ok(grad, oracle_grad(low, trimmed, n, oee), 1e-9)
         assert ok, err
-    if kernel == 5:
-        # 16 pool slots hold every string of this corpus; with 4 slots the ambiguous stretches overflow onto the
-        # warp-per-string kernel; variant 4 disables the constant folding of bridge edges
-        i = dev.info()
-        assert i["n_active_strings"] == int(rec.sum()) and i["lattice_edges"] > 0
-        assert (i["n_overflow_strings"] > 0) == (variant == 4 << 16)
-        assert (i["lattice_bridge_edges"] > 0) == (variant != 4)
     if kernel == 6:
         # segmented form: bridges + merged region types; with 4 pool slots some regions do not fit and their
         # strings go to the warp-per-string kernel
@@ -355,7 +348,7 @@ def test_edge_cases():
     words = [("", 2.0), ("x", 1.0), ("xy", 1.0), ("zz", 1.0), ("xq", 3.0), ("yyyy", 1.0)]
     d = W.parse(fsa, "\nx 1\n")
     low = W.Lowered(d, corpus=words)
-    for kernel in (6, 5, 4, 1, 2, 3):
+    for kernel in (6, 4, 1, 2, 3):
         dev, rec, pc, trimmed, n = build_device(low, force_kernel=kernel)
         assert rec.tolist() == [1, 1, 1, 0, 0, 1] and pc.tolist() == [1, 1, 1, 0, 0, 1]
         x = np.array([-0.4, -1.1, -0.2, -0.6, -0.8, -1.3])[:n]
@@ -366,6 +359,10 @@ def test_edge_cases():
         ok, err = vec_tol_ok(grad, oracle_grad(low, trimmed, n, oee), 1e-9)
         assert ok, (kernel, err)
         dev.close()
+    # kernel 5 (thread per string over compiled lattices) was removed: forcing it is refused, not rerouted
+    with pytest.raises(W.WfsaError) as ei:
+        W.Device(low, force_kernel=5)
+    assert ei.value.code == 1                                          # WFSA_ERR_INVALID
     # an empty shard is legal (a rank may own no strings)
     low0 = W.Lowered(d, corpus=[])
     dev = W.Device(low0)
@@ -384,11 +381,9 @@ def test_long_strings_need_rescaling():
     low = model.lowered()
     offs, toks, w = model.corpus(40, 3500, 4000, seed=22)
     low.set_tokens(offs, toks, w / w.sum())
-    for kernel in (6, 5, 4, 1, 2):
+    for kernel in (6, 4, 1, 2):
         dev, rec, pc, trimmed, n = build_device(low, force_kernel=kernel)
         assert rec.all()
-        if kernel == 5:          # streams of up to 8192 words stay on the compiled-lattice kernel
-            assert dev.info()["n_overflow_strings"] < len(rec)
         rng = np.random.RandomState(4)
         for x in (rng.normal(-3.0, 1.0, size=n), rng.normal(+2.5, 1.0, size=n)):
             ll, logq, grad = dev.eval(x)

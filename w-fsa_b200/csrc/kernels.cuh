@@ -601,163 +601,6 @@ __global__ void __launch_bounds__(768, 1) kt_fwdbwd(const KTParams P)
 }
 
 // ------------------------------------------------------------------------------------------
-// KL: one THREAD per string over its *compiled lattice* (lattice.hpp).  The structure of a string's
-// trimmed lattice does not depend on the weights, so it is compiled once (like the reference's
-// P and M matrices, src/Learner.cpp:276-348) and every evaluation only streams it:
-//   forward : per EDGE word  x = pool[src] * w[arc]  (stored),  pool[dst] (+)= x
-//   backward: per EDGE word  post = x * pool[dst] * sc -> RED acc[arc];  pool[src] (+)= w[arc] * pool[dst]
-// No table walk, no search, no data-dependent trip counts: the 32 streams of a warp have the same
-// padded length, CHECK words sit at the same index in all of them, so the only divergence left is
-// the per-word flag handling.  pool = kLatMaxSlots doubles per thread in shared memory (slot-major:
-// bank = lane, conflict free), w = per-arc weights a(u,v)*b(v,e) staged once per CTA.
-// The x values (8 B per edge) go to a per-warp stack in global memory that the backward sweep
-// pops in reverse (most recently written first: served by L2 for a large part).
-// ------------------------------------------------------------------------------------------
-constexpr uint32_t kLEdge = 1u << 31, kLFin = 1u << 30, kLFirstIn = 1u << 29, kLLastOut = 1u << 28, kLBridge = 1u << 27;
-constexpr int kLBand = 200;
-
-struct KLParams {
-    const double* __restrict__ aw;        // [n_arcs] weights of the combined arcs (final transitions included)
-    const uint32_t* __restrict__ words;   // word i of lane l of group g at goff[g] + i*32 + l
-    const int64_t* __restrict__ goff;     // [n_groups+1]
-    const int32_t* __restrict__ gsid;     // [n_groups*32] string id or -1
-    const double* __restrict__ p;
-    long long n_groups;
-    double* xs;                           // per warp [xs_rows][32]
-    size_t xs_rows;
-    unsigned int* counter;                // dynamic group scheduler
-    EvalOutD O;                           // O.acc_global = [replicas][n_arcs]
-    int n_arcs, replicas;
-};
-
-__device__ __forceinline__ int pool_exp(const double* p) { return (reinterpret_cast<const int*>(p)[1] >> 20) & 0x7ff; }
-
-template <int ACC>
-__global__ void __launch_bounds__(1024, 1) kl_fwdbwd(const KLParams P)
-{
-    extern __shared__ unsigned long long smem[];
-    const int tid = threadIdx.x, NT = blockDim.x, lane = tid & 31;
-    double* aw = reinterpret_cast<double*>(smem);
-    double* pool = aw + P.n_arcs + tid;                       // slot s of this thread at pool[s*NT]
-    for (int i = tid; i < P.n_arcs; i += NT) aw[i] = P.aw[i];
-    __syncthreads();
-    const long long gwarp = ((long long)blockIdx.x * NT + tid) >> 5;
-    double* const xs = P.xs + (size_t)gwarp * P.xs_rows * 32 + lane;
-    unsigned long long* const acc_g = P.O.acc_global + (size_t)(blockIdx.x % P.replicas) * (size_t)P.n_arcs;
-    long long ll_fx = 0;
-    unsigned long long bad = 0;
-
-    for (;;) {
-        long long g = 0;
-        if (lane == 0) g = (long long)atomicAdd(P.counter, 1u);
-        g = __shfl_sync(FULL, g, 0);
-        if (g >= P.n_groups) break;
-        const long long o = P.goff[g];
-        const int nw = (int)((P.goff[g + 1] - o) >> 5);
-        const uint32_t* wp = P.words + o + lane;
-        const int sid = P.gsid[g * 32 + lane];
-        const double ps = sid >= 0 ? P.p[sid] : 0.0;
-        // ---------------- forward ----------------
-        pool[0] = 1.0;                                        // the start node owns slot 0
-        int E = 0, EQ = 0;
-        double qh = 0.0;
-        for (int i0 = 0; i0 < nw; i0 += 8) {
-            uint32_t w[8];
-#pragma unroll
-            for (int j = 0; j < 8; ++j) w[j] = __ldcs(wp + (size_t)(i0 + j) * 32);
-#pragma unroll
-            for (int j = 0; j < 8; ++j) {
-                const uint32_t wj = w[j];
-                if (j == 7 && (i0 & 8)) {                     // CHECK word (uniform across the warp)
-                    const uint32_t m0 = wj & 0xffffu;
-                    if (m0) {
-                        int emax = 0;
-                        for (uint32_t m = m0; m; m &= m - 1) emax = max(emax, pool_exp(pool + (__ffs(m) - 1) * NT));
-                        reinterpret_cast<long long*>(xs)[(size_t)(i0 + j) * 32] = E;
-                        if (emax != 0 && (emax < 1023 - kLBand || emax > 1023 + kLBand)) {
-                            const int shift = 1023 - emax;
-                            for (uint32_t m = m0; m; m &= m - 1) { double* q = pool + (__ffs(m) - 1) * NT; *q = scalbn(*q, shift); }
-                            E -= shift;
-                        }
-                    }
-                } else if (wj & kLEdge) {
-                    const int src = (wj >> 19) & 15, dst = (wj >> 23) & 15, arc = wj & 0xffff;
-                    const double xv = pool[src * NT] * aw[arc];
-                    if (!(wj & kLBridge)) xs[(size_t)(i0 + j) * 32] = xv;
-                    double* pd = pool + dst * NT;
-                    *pd = (wj & kLFirstIn) ? xv : *pd + xv;
-                } else if (wj & kLFin) {
-                    qh = pool[(wj & 15) * NT];
-                    EQ = E;
-                }
-            }
-        }
-        const bool ok = sid >= 0 && qh > 0.0 && isfinite(qh);
-        if (sid >= 0) {
-            if (ok) {
-                const double lq = log(qh) + (double)EQ * 0.69314718055994530942;
-                if (P.O.logq) P.O.logq[sid] = lq;
-                ll_fx += __double2ll_rn(ps * lq * P.O.ll_scale);
-            } else {
-                if (P.O.logq) P.O.logq[sid] = -INFINITY;
-                bad++;
-            }
-        }
-        // ---------------- backward ----------------
-        const double sc0 = ok ? (1.0 / qh) * ps * P.O.fx_scale : 0.0;
-        double sc = sc0;
-        int F = 0;
-        for (int i0 = nw - 8; i0 >= 0; i0 -= 8) {
-            uint32_t w[8];
-            double xv[8];
-#pragma unroll
-            for (int j = 0; j < 8; ++j) w[j] = __ldcs(wp + (size_t)(i0 + j) * 32);
-#pragma unroll
-            for (int j = 0; j < 8; ++j) {
-                const bool chk = (j == 7 && (i0 & 8));
-                const bool need = chk ? (w[j] & 0xffffu) != 0 : (w[j] & (kLEdge | kLBridge)) == kLEdge;
-                xv[j] = need ? xs[(size_t)(i0 + j) * 32] : 0.0;
-            }
-#pragma unroll
-            for (int j = 7; j >= 0; --j) {
-                const uint32_t wj = w[j];
-                if (j == 7 && (i0 & 8)) {
-                    const uint32_t m0 = wj & 0xffffu;
-                    if (m0) {
-                        const int Et = (int)__double_as_longlong(xv[j]);
-                        int emax = 0;
-                        for (uint32_t m = m0; m; m &= m - 1) emax = max(emax, pool_exp(pool + (__ffs(m) - 1) * NT));
-                        if (emax != 0 && (emax < 1023 - kLBand || emax > 1023 + kLBand)) {
-                            const int shift = 1023 - emax;
-                            for (uint32_t m = m0; m; m &= m - 1) { double* q = pool + (__ffs(m) - 1) * NT; *q = scalbn(*q, shift); }
-                            F -= shift;
-                        }
-                        sc = scalbn(sc0, Et + F - EQ);
-                    }
-                } else if (wj & kLEdge) {
-                    const int src = (wj >> 19) & 15, dst = (wj >> 23) & 15, arc = wj & 0xffff;
-                    const double bd = pool[dst * NT];
-                    const double c = aw[arc] * bd;
-                    double* psrc = pool + src * NT;
-                    *psrc = (wj & kLLastOut) ? c : *psrc + c;
-                    if (ACC != ACC_NONE && !(wj & kLBridge) && ok) {
-                        const long long v = __double2ll_rn(xv[j] * bd * sc);
-                        if (v) atomicAdd(acc_g + arc, (unsigned long long)v);
-                    }
-                } else if (wj & kLFin) {
-                    pool[(wj & 15) * NT] = 1.0;
-                }
-            }
-        }
-    }
-    for (int o = 16; o; o >>= 1) { ll_fx += __shfl_xor_sync(FULL, ll_fx, o); bad += __shfl_xor_sync(FULL, bad, o); }
-    if (lane == 0) {
-        if (ll_fx) atomicAdd(P.O.red, (unsigned long long)ll_fx);
-        if (bad) atomicAdd(P.O.red + 1, bad);
-    }
-}
-
-// ------------------------------------------------------------------------------------------
 // K3: one CTA per string for automata where more than 32 states emit one symbol.
 // Thread i <-> candidate slot i of the current symbol; alpha / beta~ vectors double-buffered in
 // shared memory; the lattice (dense over candidates) goes to a per-CTA slab in global memory

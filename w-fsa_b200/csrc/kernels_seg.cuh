@@ -137,7 +137,7 @@ __device__ __forceinline__ void kr_paths(const KRParams& P, const double* aw, in
     }
 }
 
-// ---- big DAG regions: the KL stream loop (CHECK words rescale, x values on a stack), one thread per region -------------
+// ---- big DAG regions: the stream format of lattice.hpp (CHECK words rescale, x values on a stack), one thread per region
 // A group is walked by three blocks: big_fwd (forward chain), big_bwd (backward chain) and big_red (the REDs).  One warp
 // runs all three (k_eval6 with one warp per group, kr_regions), or two warps split them (k_eval6, a CTA that owns one
 // staged group): warp 0 big_fwd, warp 1 big_bwd<false> on its own pool at the same time, then warp 0 big_red<true>.
@@ -155,6 +155,8 @@ __device__ __forceinline__ void kr_paths(const KRParams& P, const double* aw, in
 // (A generic store to the shared window sits in the same in-order LSU queue as the chain's LDS/STS and takes longer to
 // resolve.)  No memory clobbers: the pool and the staging area are touched by these volatile statements only, which keep
 // their order among themselves; a clobber would pin every other memory access around each of them.
+constexpr uint32_t kLEdge = 1u << 31, kLFin = 1u << 30, kLFirstIn = 1u << 29, kLLastOut = 1u << 28;   // = kLat* of lattice.hpp
+constexpr int kLBand = 200;
 struct BigPool { unsigned int p, ps, trash; };
 __device__ __forceinline__ double lds_f64(unsigned int a) { double v; asm volatile("ld.shared.f64 %0, [%1];" : "=d"(v) : "r"(a)); return v; }
 __device__ __forceinline__ void sts_f64(unsigned int a, double v) { asm volatile("st.shared.f64 [%0], %1;" :: "r"(a), "d"(v)); }

@@ -250,100 +250,6 @@ int compile_lattice(const HostFsa& f, const LatticeArcs& A, const uint8_t* alive
     return 1;
 }
 
-void compile_corpus(const HostFsa& f, const LatticeArcs& A, const uint8_t* alive, const int32_t* tokens,
-                    const int64_t* offs, const double* p, const std::vector<int32_t>& ids, int n_slots, double fx_scale,
-                    bool use_bridges, int max_stream_words, CompiledCorpus& out)
-{
-    out = CompiledCorpus();
-    const size_t n = ids.size();
-    out.const_acc.assign(A.n_arcs, 0);
-    unsigned hw = std::thread::hardware_concurrency();
-    const int T = (int)std::max<size_t>(1, std::min<size_t>({(size_t)(hw ? hw : 4), (size_t)64, n / 256 + 1}));
-    struct Local {
-        std::vector<uint32_t> words;
-        std::vector<int64_t> off;            // start of string (i*T + t) in words
-        std::vector<int32_t> cnt;            // words, 0 rejected, -1 overflow
-        std::vector<long long> cacc;
-        int64_t n_edges = 0, n_bridge = 0;
-    };
-    std::vector<Local> loc(T);
-    LatticeArcs Anb;                          // copy with bridges disabled when requested
-    const LatticeArcs* AP = &A;
-    if (!use_bridges && A.layered) { Anb = A; Anb.layered = false; AP = &Anb; }
-    auto work = [&](int t) {
-        Local& L = loc[t];
-        LatticeScratch S;
-        std::vector<int32_t> bridges;
-        L.cacc.assign(A.n_arcs, 0);
-        for (size_t i = t; i < n; i += T) {
-            const int32_t sid = ids[i];
-            const int len = (int)(offs[sid + 1] - offs[sid]);
-            bridges.clear();
-            L.off.push_back((int64_t)L.words.size());
-            const size_t before = L.words.size();
-            int rc = compile_lattice(f, *AP, alive, tokens + offs[sid], len, n_slots, S, L.words, bridges);
-            if (rc == 1 && L.words.size() - before > (size_t)max_stream_words) { rc = -1; L.words.resize(before); }
-            if (rc == 1) {
-                L.cnt.push_back((int32_t)(L.words.size() - before));
-                const long long c = llrint(p[sid] * fx_scale);
-                for (int32_t a : bridges) L.cacc[a] += c;
-                L.n_bridge += (int64_t)bridges.size();
-                for (size_t k = before; k < L.words.size(); ++k) L.n_edges += (L.words[k] >> 31);
-            } else L.cnt.push_back(rc);
-        }
-    };
-    {
-        std::vector<std::thread> th;
-        for (int t = 1; t < T; ++t) th.emplace_back(work, t);
-        work(0);
-        for (auto& x : th) x.join();
-    }
-    for (int t = 0; t < T; ++t) {
-        for (int a = 0; a < A.n_arcs; ++a) out.const_acc[a] += loc[t].cacc[a];
-        out.n_edges += loc[t].n_edges; out.n_bridge += loc[t].n_bridge;
-    }
-    // strings with a stream, longest stream first (ties in input order => deterministic)
-    std::vector<int64_t> ok;                 // indices into ids
-    for (size_t i = 0; i < n; ++i) {
-        const int c = loc[i % T].cnt[i / T];
-        if (c > 0) ok.push_back((int64_t)i);
-        else if (c < 0) out.overflow.push_back(ids[i]);
-        else out.rejected.push_back(ids[i]);
-    }
-    std::stable_sort(ok.begin(), ok.end(), [&](int64_t a, int64_t b) { return loc[a % T].cnt[a / T] > loc[b % T].cnt[b / T]; });
-    const int64_t groups = ((int64_t)ok.size() + 31) / 32;
-    out.goff.assign(groups + 1, 0);
-    out.gsid.assign((size_t)groups * 32, -1);
-    for (int64_t g = 0; g < groups; ++g) {
-        const int64_t a = ok[g * 32];
-        int64_t mx = loc[a % T].cnt[a / T];                       // sorted: the first of the group is the longest
-        mx = (mx + kCheckEvery - 1) / kCheckEvery * kCheckEvery;
-        out.goff[g + 1] = out.goff[g] + mx * 32;
-        out.max_words = std::max(out.max_words, mx);
-    }
-    out.n_words = out.goff[groups];
-    out.words.assign((size_t)out.n_words + 32, 0u);
-    auto fill = [&](int t) {
-        for (int64_t g = t; g < groups; g += T) {
-            uint32_t* dst = out.words.data() + out.goff[g];
-            for (int l = 0; l < 32 && g * 32 + l < (int64_t)ok.size(); ++l) {
-                const int64_t i = ok[g * 32 + l];
-                const Local& L = loc[i % T];
-                const uint32_t* src = L.words.data() + L.off[i / T];
-                const int c = L.cnt[i / T];
-                for (int k = 0; k < c; ++k) dst[(size_t)k * 32 + l] = src[k];
-                out.gsid[(size_t)g * 32 + l] = ids[i];
-            }
-        }
-    };
-    {
-        std::vector<std::thread> th;
-        for (int t = 1; t < T; ++t) th.emplace_back(fill, t);
-        fill(0);
-        for (auto& x : th) x.join();
-    }
-}
-
 // ---------------------------------------------------------------------------------------------
 // Segmented form
 // ---------------------------------------------------------------------------------------------

@@ -1,4 +1,4 @@
-// w-fsa_b200/csrc/lattice.hpp -- compiled per-string lattices of the thread-per-string kernel KL.
+// w-fsa_b200/csrc/lattice.hpp -- compiled per-string lattices: the word stream and the segmented form.
 //
 // The reference freezes the structure of every corpus string once, as the path matrices P and M
 // (/root/reference/src/Learner.cpp:276-348), and every later evaluation is arithmetic on that
@@ -10,7 +10,9 @@
 // string and the trim map, never on the weights x, so it is compiled once per
 // wfsa_dev_set_param_map and streamed by every evaluation.
 //
-// Stream of one string = 32-bit words in a topological order of the edges (grouped by source node):
+// Stream = 32-bit words in a topological order of the edges (grouped by source node).  The DAG form of a region type
+// (big_fwd / big_bwd in kernels_seg.cuh) is the stream of one region with region-local slots; compile_lattice writes
+// the stream of a whole string, which the tests interpret on the CPU:
 //
 //   EDGE  bit31=1 | first_in<<29 | last_out<<28 | bridge<<27 | dst_slot<<23 | src_slot<<19 | arc
 //         forward :  x = pool[src] * w[arc];  pool[dst] = first_in ? x : pool[dst] + x
@@ -68,21 +70,6 @@ struct LatticeScratch {
 // another kernel).  bridge_arcs receives the arcs of bridge edges (for the constant accumulators).
 int compile_lattice(const HostFsa& f, const LatticeArcs& A, const uint8_t* arc_alive, const int32_t* tok, int len,
                     int n_slots, LatticeScratch& S, std::vector<uint32_t>& words, std::vector<int32_t>& bridge_arcs);
-
-// Whole shard: compiled streams of the strings in `ids`, grouped 32 to a warp (longest streams first),
-// transposed so that word i of lane l of group g is at goff[g] + i*32 + l.
-struct CompiledCorpus {
-    std::vector<uint32_t> words;
-    std::vector<int64_t> goff;                 // [n_groups+1]
-    std::vector<int32_t> gsid;                 // [n_groups*32] string id or -1
-    std::vector<int32_t> overflow;             // strings that need more than n_slots slots
-    std::vector<int32_t> rejected;             // strings without an accepting path
-    std::vector<long long> const_acc;          // [n_arcs] fixed-point constant gradient part (bridge edges)
-    int64_t n_edges = 0, n_bridge = 0, n_words = 0, max_words = 0;
-};
-void compile_corpus(const HostFsa& f, const LatticeArcs& A, const uint8_t* arc_alive, const int32_t* tokens,
-                    const int64_t* offs, const double* p, const std::vector<int32_t>& ids, int n_slots, double fx_scale,
-                    bool use_bridges, int max_stream_words, CompiledCorpus& out);
 
 
 // ---------------------------------------------------------------------------------------------

@@ -169,20 +169,17 @@ struct wfsa_dev {
     int k3_grid = 0, k3_block = 0; size_t k3_smem = 0;
             // CTA-per-string (K3) launch
     int kt_grid = 0, kt_block = 0, kt_K = 0; size_t kt_smem = 0, kt_lat_words = 0;   // thread-per-string (KT)
-    int secondary = 0;                                            // kernel that takes KT's / KL's overflow strings
+    int secondary = 0;                                            // kernel that takes KT's / the segmented path's overflow strings
     int skernel = 0;                                              // kernel of the structural pass
-    // compiled-lattice thread-per-string kernel (KL)
+    // segmented compiled lattices (KR + KS, kernel 6): launch of k_eval6 / kr_regions, per-arc weights and accumulators
     LatticeArcs larcs;
-    int kl_grid = 0, kl_block = 0, kl_K = 0; size_t kl_smem = 0;
+    int seg_grid = 0, seg_block = 0, seg_slots = 0; size_t seg_smem = 0;
     bool awg = false;                         // segmented path with the arc weights in HBM/L2 (they do not fit shared memory)
-    bool kl_bridges = true;
-    int64_t kl_groups = 0, kl_words = 0, kl_edges = 0, kl_bridge_edges = 0, kl_max_words = 0;
-    DevBuf<uint32_t> d_klwords, d_klcounter;
-    DevBuf<int64_t> d_klgoff;
-    DevBuf<int32_t> d_klgsid, d_kl_arc_tid, d_kl_arc_eid;
-    DevBuf<double> d_klaw, d_klxs;
-    DevBuf<unsigned long long> d_klacc, d_klconst;
-    // segmented compiled lattices (KR + KS, kernel 6)
+    int64_t seg_max_big_rows = 0;
+    DevBuf<uint32_t> d_seg_counter;
+    DevBuf<int32_t> d_seg_arc_tid, d_seg_arc_eid;
+    DevBuf<double> d_seg_aw, d_seg_xs;
+    DevBuf<unsigned long long> d_seg_acc, d_seg_const;
     size_t ks_smem = 0; int ks_grid = 0, ks_block = 512, ks_ctas = 2;
     int64_t kr_big_groups = 0;                  // DAG-form groups (they sort first)
     int64_t kr_groups = 0, ks_groups = 0, seg_types = 0, seg_instances = 0, seg_region_edges = 0, seg_type_edges = 0,
@@ -197,7 +194,7 @@ struct wfsa_dev {
     DevBuf<uint32_t> d_krwords, d_kswords;
     DevBuf<int64_t> d_krgoff, d_ksgoff;
     DevBuf<int32_t> d_krgrows, d_ksgref, d_kssid, d_eoff, d_earc;
-    DevBuf<double> d_krW, d_krlq, d_ksp, d_kslogq, d_klogaw;
+    DevBuf<double> d_krW, d_krlq, d_ksp, d_kslogq, d_seg_logaw;
     std::vector<double> h_p;
     int64_t n_overflow = 0, n_active_w = 0;
     DevBuf<int32_t> d_order_w;                                    // overflow strings (secondary kernel)
@@ -389,10 +386,10 @@ static int setup_kt(wfsa_dev* h)
     return WFSA_OK;
 }
 
-// compiled-lattice kernel: per-arc weights + kLatMaxSlots pool doubles per thread must fit 227 KB
+// segmented kernels: per-arc weights + K pool doubles per thread must fit 227 KB
 // `awg` (may be null = not allowed): set when the table does not fit but the pool alone does -- the segmented kernels then read
-// the weights from HBM/L2 (their AWG instances); the thread-per-string kernel 5 has no such form
-static bool kl_possible(const wfsa_dev* h, int K, int want_nt, int& nt, size_t& smem, bool* awg = nullptr)
+// the weights from HBM/L2 (their AWG instances)
+static bool seg_possible(const wfsa_dev* h, int K, int want_nt, int& nt, size_t& smem, bool* awg = nullptr)
 {
     const LatticeArcs& A = h->larcs;
     if (awg) *awg = false;
@@ -444,65 +441,60 @@ static int setup_k7_planes(wfsa_dev* h)
     return WFSA_OK;
 }
 
-static int setup_kl(wfsa_dev* h)
+static int setup_seg(wfsa_dev* h)
 {
     int K = (h->opt.reserved >> 16) & 0xff;
     if (K == 0 || K > kLatMaxSlots) K = kLatMaxSlots;
     int nt = 0; size_t smem = 0;
     int want_nt = ((h->opt.reserved >> 24) & 0x7f) * 32;
-    if (want_nt == 0 && h->kernel == 6) want_nt = 512;       // measured: 16 warps leave the L1 to the register spills
+    if (want_nt == 0) want_nt = 512;       // measured: 16 warps leave the L1 to the register spills
     bool awg = false;
-    if (!kl_possible(h, K, want_nt, nt, smem, h->kernel == 6 ? &awg : nullptr))
-        return set_err(h, WFSA_ERR_LIMIT, "compiled-lattice kernel: the arc weights do not fit shared memory");
+    if (!seg_possible(h, K, want_nt, nt, smem, &awg))
+        return set_err(h, WFSA_ERR_LIMIT, "segmented kernel: the arc weights do not fit shared memory");
     h->awg = awg;
-    if (h->kernel == 6 && (want_nt == 512 || nt > 512 || awg)) {   // k_eval6 is compiled for 512, 256 and 128 threads (AWG: 512), kr_regions for up to 512
+    if (want_nt == 512 || nt > 512 || awg) {   // k_eval6 is compiled for 512, 256 and 128 threads (AWG: 512), kr_regions for up to 512
         nt = awg ? 512 : (nt >= 512 ? 512 : (nt >= 256 ? 256 : 128));
         smem = (awg ? 0 : ((size_t)h->larcs.n_arcs + 1) * 8) + (size_t)nt * K * 8;
     }
-    h->kl_K = K; h->kl_block = nt; h->kl_grid = h->sm_count; h->kl_smem = smem;
+    h->seg_slots = K; h->seg_block = nt; h->seg_grid = h->sm_count; h->seg_smem = smem;
     // experiment / test knob: a smaller persistent grid, so that a small shard reaches the schedules of a large one (more big DAG
-    // groups than CTAs, several per warp).  Read here, before the per-warp x stacks are sized from kl_grid.
-    if (const char* g = getenv("WFSA_E6_GRID")) h->kl_grid = std::min(h->sm_count, std::max(1, atoi(g)));
-    h->kl_bridges = !(h->opt.reserved & 4);
+    // groups than CTAs, several per warp).  Read here, before the per-warp x stacks are sized from seg_grid.
+    if (const char* g = getenv("WFSA_E6_GRID")) h->seg_grid = std::min(h->sm_count, std::max(1, atoi(g)));
     const LatticeArcs& A = h->larcs;
-    CK(h->d_kl_arc_tid.upload(A.arc_tid, h->stream)); CK(h->d_kl_arc_eid.upload(A.arc_eid, h->stream));
-    CK(h->d_klaw.alloc((size_t)A.n_arcs + 1)); CK(cudaMemsetAsync(h->d_klaw.p, 0, ((size_t)A.n_arcs + 1) * 8, h->stream)); CK(h->d_klacc.alloc((size_t)A.n_arcs * h->replicas)); CK(h->d_klconst.alloc(A.n_arcs));
-    CK(h->d_klcounter.alloc(2));
+    CK(h->d_seg_arc_tid.upload(A.arc_tid, h->stream)); CK(h->d_seg_arc_eid.upload(A.arc_eid, h->stream));
+    CK(h->d_seg_aw.alloc((size_t)A.n_arcs + 1)); CK(cudaMemsetAsync(h->d_seg_aw.p, 0, ((size_t)A.n_arcs + 1) * 8, h->stream)); CK(h->d_seg_acc.alloc((size_t)A.n_arcs * h->replicas)); CK(h->d_seg_const.alloc(A.n_arcs));
+    CK(h->d_seg_counter.alloc(2));
     CK(h->d_llpart.alloc(2 * (size_t)((std::max(h->larcs.n_arcs, 1) + 255) / 256)));
-    if (h->kernel == 6) {
-        CK(h->d_klogaw.alloc((size_t)A.n_arcs + 16)); CK(cudaMemsetAsync(h->d_klogaw.p, 0, ((size_t)A.n_arcs + 16) * 8, h->stream));   // (+ the zero entries of the padding ids)
-        {   // arcs of every edge (transition edges, then emission edges) for the gather in k_fold_finish6
-            const int nt = h->fsa.n_trans(), ne = nt + h->fsa.n_emis();
-            std::vector<int32_t> off((size_t)ne + 1, 0), arc;
-            for (int a = 0; a < A.n_arcs; ++a) { off[A.arc_tid[a] + 1]++; if (A.arc_eid[a] >= 0) off[nt + A.arc_eid[a] + 1]++; }
-            for (int e = 0; e < ne; ++e) off[e + 1] += off[e];
-            arc.resize((size_t)off[ne]);
-            std::vector<int32_t> fill(off.begin(), off.end() - 1);
-            for (int a = 0; a < A.n_arcs; ++a) { arc[fill[A.arc_tid[a]]++] = a; if (A.arc_eid[a] >= 0) arc[fill[nt + A.arc_eid[a]]++] = a; }
-            CK(h->d_eoff.upload(off, h->stream)); CK(h->d_earc.upload(arc, h->stream));
-        }
-        {   // single-launch evaluation: control words (tickets, barrier arrivals, epoch = 1), reduction cells, phase stamps
-            const std::vector<unsigned int> ctl = {0u, 0u, 0u, 1u, 0u, 0u, 0u, 0u};
-            CK(h->d_e6ctl.upload(ctl, h->stream));
-            CK(h->d_e6red.alloc(2)); CK(cudaMemsetAsync(h->d_e6red.p, 0, 16, h->stream));
-            CK(h->d_e6stamps.alloc(8 + 8 * 1024)); CK(cudaMemsetAsync(h->d_e6stamps.p, 0, (8 + 8 * 1024) * 8, h->stream));
-            cudaFuncSetAttribute(k_eval6<512>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024 - 8192);
-            cudaFuncSetAttribute(k_eval6<384>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024 - 8192);
-            cudaFuncSetAttribute(k_eval6<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024 - 8192);
-            cudaFuncSetAttribute(k_eval6<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024 - 8192);
-        }
-        h->ks_smem = h->awg ? 0 : ((size_t)A.n_arcs + 16) * 8;
-        h->ks_block = kKsWarps * 32;
-        h->ks_ctas = h->ks_smem * 2 + 2048 <= 227 * 1024 ? 2 : 1;
-        h->ks_grid = h->sm_count * h->ks_ctas;
-        cudaFuncSetAttribute(k_eval6<512, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024 - 8192);
-        cudaFuncSetAttribute(kr_regions<ACC_GLOBAL, 512>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024 - 8192 - 1024);
-        cudaFuncSetAttribute(kr_regions<ACC_NONE, 512>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024 - 8192 - 1024);
-        cudaFuncSetAttribute(kr_regions<ACC_GLOBAL, 512, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024 - 8192 - 1024);
-        cudaFuncSetAttribute(ks_strings<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->ks_smem);   // it also has static shared memory
+    CK(h->d_seg_logaw.alloc((size_t)A.n_arcs + 16)); CK(cudaMemsetAsync(h->d_seg_logaw.p, 0, ((size_t)A.n_arcs + 16) * 8, h->stream));   // (+ the zero entries of the padding ids)
+    {   // arcs of every edge (transition edges, then emission edges) for the gather in k_fold_finish6
+        const int nt = h->fsa.n_trans(), ne = nt + h->fsa.n_emis();
+        std::vector<int32_t> off((size_t)ne + 1, 0), arc;
+        for (int a = 0; a < A.n_arcs; ++a) { off[A.arc_tid[a] + 1]++; if (A.arc_eid[a] >= 0) off[nt + A.arc_eid[a] + 1]++; }
+        for (int e = 0; e < ne; ++e) off[e + 1] += off[e];
+        arc.resize((size_t)off[ne]);
+        std::vector<int32_t> fill(off.begin(), off.end() - 1);
+        for (int a = 0; a < A.n_arcs; ++a) { arc[fill[A.arc_tid[a]]++] = a; if (A.arc_eid[a] >= 0) arc[fill[nt + A.arc_eid[a]]++] = a; }
+        CK(h->d_eoff.upload(off, h->stream)); CK(h->d_earc.upload(arc, h->stream));
     }
-    cudaFuncSetAttribute(kl_fwdbwd<ACC_GLOBAL>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-    cudaFuncSetAttribute(kl_fwdbwd<ACC_NONE>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+    {   // single-launch evaluation: control words (tickets, barrier arrivals, epoch = 1), reduction cells, phase stamps
+        const std::vector<unsigned int> ctl = {0u, 0u, 0u, 1u, 0u, 0u, 0u, 0u};
+        CK(h->d_e6ctl.upload(ctl, h->stream));
+        CK(h->d_e6red.alloc(2)); CK(cudaMemsetAsync(h->d_e6red.p, 0, 16, h->stream));
+        CK(h->d_e6stamps.alloc(8 + 8 * 1024)); CK(cudaMemsetAsync(h->d_e6stamps.p, 0, (8 + 8 * 1024) * 8, h->stream));
+        cudaFuncSetAttribute(k_eval6<512>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024 - 8192);
+        cudaFuncSetAttribute(k_eval6<384>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024 - 8192);
+        cudaFuncSetAttribute(k_eval6<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024 - 8192);
+        cudaFuncSetAttribute(k_eval6<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024 - 8192);
+    }
+    h->ks_smem = h->awg ? 0 : ((size_t)A.n_arcs + 16) * 8;
+    h->ks_block = kKsWarps * 32;
+    h->ks_ctas = h->ks_smem * 2 + 2048 <= 227 * 1024 ? 2 : 1;
+    h->ks_grid = h->sm_count * h->ks_ctas;
+    cudaFuncSetAttribute(k_eval6<512, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024 - 8192);
+    cudaFuncSetAttribute(kr_regions<ACC_GLOBAL, 512>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024 - 8192 - 1024);
+    cudaFuncSetAttribute(kr_regions<ACC_NONE, 512>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024 - 8192 - 1024);
+    cudaFuncSetAttribute(kr_regions<ACC_GLOBAL, 512, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024 - 8192 - 1024);
+    cudaFuncSetAttribute(ks_strings<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->ks_smem);   // it also has static shared memory
     return WFSA_OK;
 }
 
@@ -528,11 +520,11 @@ static int choose_launch(wfsa_dev* h)
     }
     int rc = WFSA_OK;
     h->skernel = h->kernel;
-    if (h->kernel == 5 || h->kernel == 6) {
+    if (h->kernel == 6) {
         h->secondary = h->fast.warp_ok ? 1 : (h->fast.ok ? 2 : 3);
         int nt = 0; size_t sm = 0; int K = (h->opt.reserved >> 16) & 0xff; if (K == 0) K = 8;
         h->skernel = (h->fast.ok && kt_possible(h, K, nt, sm)) ? 4 : h->secondary;
-        rc = setup_kl(h);
+        rc = setup_seg(h);
         if (rc == WFSA_OK && h->skernel == 4) rc = setup_kt(h);
         if (rc == WFSA_OK) rc = h->secondary == 1 ? setup_k2(h) : (h->secondary == 2 ? setup_k3(h) : setup_generic(h));
     } else if (h->kernel == 4) {
@@ -605,15 +597,15 @@ extern "C" int wfsa_dev_create(const wfsa_fsa_desc* fd, const wfsa_corpus_desc* 
     if (kernel == 0) {
         int nt = 0; size_t sm = 0; int K = (h->opt.reserved >> 16) & 0xff; if (K == 0) K = 8;
         bool awg = false;
-        if (kl_possible(h, kLatMaxSlots, 0, nt, sm)) kernel = h->larcs.n_arcs < 65520 ? 6 : 5;
-        else if (h->larcs.n_arcs < 65520 && kl_possible(h, kLatMaxSlots, 0, nt, sm, &awg)) kernel = 6;      // weights in HBM/L2 (16-bit arc ids still fit)
+        if (h->larcs.n_arcs < 65520 && seg_possible(h, kLatMaxSlots, 0, nt, sm, &awg)) kernel = 6;      // weights in shared memory or in HBM/L2 (16-bit arc ids still fit)
         else kernel = !h->fast.ok ? 3 : (kt_possible(h, K, nt, sm) ? 4 : (h->fast.warp_ok ? 1 : (((h->fast.max_cand + 31) / 32 * 32 <= 512 && cd && cd->n_strings >= 200000) ? 7 : 2)));     // K7 pays off once ~3 strings share a symbol pair per position
     }
     if (kernel == 6 && h->larcs.n_arcs >= 65520) { h->err = "forced segmented kernel but the automaton has 65520 or more combined arcs"; return bail(WFSA_ERR_INVALID); }
-    if (kernel == 5 || kernel == 6) { int nt = 0; size_t sm = 0; bool awg = false; if (!kl_possible(h, kLatMaxSlots, 0, nt, sm, kernel == 6 ? &awg : nullptr)) { h->err = "forced compiled-lattice kernel but the arc weights do not fit shared memory"; return bail(WFSA_ERR_INVALID); } }
+    if (kernel == 6) { int nt = 0; size_t sm = 0; bool awg = false; if (!seg_possible(h, kLatMaxSlots, 0, nt, sm, &awg)) { h->err = "forced segmented kernel but the arc weights do not fit shared memory"; return bail(WFSA_ERR_INVALID); } }
     if (kernel == 7 && h->fast.ok && (h->fast.max_cand + 31) / 32 * 32 > 512) { h->err = "forced batched kernel but more than 512 states emit one symbol"; return bail(WFSA_ERR_INVALID); }
     if ((kernel == 1 || kernel == 2 || kernel == 4 || kernel == 7) && !h->fast.ok) { h->err = "forced fast kernel but emissions are not all one token long"; return bail(WFSA_ERR_INVALID); }
     if (kernel == 1 && !h->fast.warp_ok) { h->err = "forced warp-per-string kernel but more than 32 states emit one symbol"; return bail(WFSA_ERR_INVALID); }
+    if (kernel == 5) { h->err = "force_kernel 5 (thread-per-string over compiled lattices) was removed: the segmented kernel 6 takes every input it took"; return bail(WFSA_ERR_INVALID); }
     if (kernel < 1 || kernel > 7) { h->err = "force_kernel out of range"; return bail(WFSA_ERR_INVALID); }
     h->kernel = kernel;
 
@@ -724,16 +716,16 @@ static void launch_main(wfsa_dev* h, int kernel, int mode, const CorpusD& C, con
     if (C.n_order <= 0) return;
     if (kernel == 6) {
         // (the general path: evaluations with overflow strings, or without the single-launch kernel)
-        cudaMemsetAsync(h->d_klcounter.p, 0, 8, st);
+        cudaMemsetAsync(h->d_seg_counter.p, 0, 8, st);
         if (h->kr_groups > 0) {
             KRParams P{};
-            P.aw = h->d_klaw.p; P.words = h->d_krwords.p; P.goff = h->d_krgoff.p; P.grows = h->d_krgrows.p; P.typeW = h->d_krW.p;
-            P.lq = h->d_krlq.p; P.n_groups = h->kr_groups; P.xs = h->d_klxs.p; P.xs_rows = (size_t)std::max<int64_t>(h->kl_max_words, 1);
-            P.counter = h->d_klcounter.p; P.acc = h->d_klacc.p; P.fx_scale = O.fx_scale; P.n_arcs = h->larcs.n_arcs; P.replicas = h->replicas;
+            P.aw = h->d_seg_aw.p; P.words = h->d_krwords.p; P.goff = h->d_krgoff.p; P.grows = h->d_krgrows.p; P.typeW = h->d_krW.p;
+            P.lq = h->d_krlq.p; P.n_groups = h->kr_groups; P.xs = h->d_seg_xs.p; P.xs_rows = (size_t)std::max<int64_t>(h->seg_max_big_rows, 1);
+            P.counter = h->d_seg_counter.p; P.acc = h->d_seg_acc.p; P.fx_scale = O.fx_scale; P.n_arcs = h->larcs.n_arcs; P.replicas = h->replicas;
             P.ll_scale = O.ll_scale; P.red = O.red; P.llpart = h->d_llpart.p; P.n_llpart = h->llpart_n;
-            if (h->awg) kr_regions<ACC_GLOBAL, 512, true><<<h->kl_grid, h->kl_block, h->kl_smem, st>>>(P);       // weights read from HBM/L2
-            else if (h->opt.reserved & 2) kr_regions<ACC_NONE, 512><<<h->kl_grid, h->kl_block, h->kl_smem, st>>>(P);   // timing experiment
-            else kr_regions<ACC_GLOBAL, 512><<<h->kl_grid, h->kl_block, h->kl_smem, st>>>(P);
+            if (h->awg) kr_regions<ACC_GLOBAL, 512, true><<<h->seg_grid, h->seg_block, h->seg_smem, st>>>(P);       // weights read from HBM/L2
+            else if (h->opt.reserved & 2) kr_regions<ACC_NONE, 512><<<h->seg_grid, h->seg_block, h->seg_smem, st>>>(P);   // timing experiment
+            else kr_regions<ACC_GLOBAL, 512><<<h->seg_grid, h->seg_block, h->seg_smem, st>>>(P);
             h->launches++;
         }
         if (h->mid_now) cudaEventRecord(h->mid_now, st);
@@ -745,16 +737,6 @@ static void launch_main(wfsa_dev* h, int kernel, int mode, const CorpusD& C, con
             k_add_llpart<<<1, 32, 0, st>>>(h->d_llpart.p, h->llpart_n, O.red);
             h->launches++;
         }
-    } else if (kernel == 5) {
-        KLParams P{};
-        P.aw = h->d_klaw.p; P.words = h->d_klwords.p; P.goff = h->d_klgoff.p; P.gsid = h->d_klgsid.p; P.p = h->d_p.p;
-        P.n_groups = h->kl_groups; P.xs = h->d_klxs.p; P.xs_rows = (size_t)std::max<int64_t>(h->kl_max_words, 1);
-        P.counter = h->d_klcounter.p; P.O = O; P.O.acc_global = h->d_klacc.p;
-        P.n_arcs = h->larcs.n_arcs; P.replicas = h->replicas;
-        cudaMemsetAsync(h->d_klcounter.p, 0, 4, st);
-        if (h->opt.reserved & 2) kl_fwdbwd<ACC_NONE><<<h->kl_grid, h->kl_block, h->kl_smem, st>>>(P);   // timing experiment
-        else kl_fwdbwd<ACC_GLOBAL><<<h->kl_grid, h->kl_block, h->kl_smem, st>>>(P);
-        h->launches++;
     } else if (kernel == 4) {
         KTParams P{};
         P.T = ThreadTablesD{h->d_brow16.p, h->d_adst16.p, h->d_aw.p, h->d_fws.p, F.n_sym, F.n_states, L.n_arcs, F.start, L.start_final_tid};
@@ -889,7 +871,7 @@ static void launch_main(wfsa_dev* h, int kernel, int mode, const CorpusD& C, con
 static int eval6_big_dedicate(const wfsa_dev* h)
 {
     const int ded_div = getenv("WFSA_E6_DED_DIV") ? std::max(1, atoi(getenv("WFSA_E6_DED_DIV"))) : 4;
-    return (h->kr_big_groups > 0 && h->kr_big_groups * ded_div <= h->kl_grid && !getenv("WFSA_E6_NO_DEDICATE")) ? 1 : 0;
+    return (h->kr_big_groups > 0 && h->kr_big_groups * ded_div <= h->seg_grid && !getenv("WFSA_E6_NO_DEDICATE")) ? 1 : 0;
 }
 
 // The whole evaluation of the segmented path in one launch (kernels_eval6.cuh).  All launch parameters are constant per
@@ -902,11 +884,11 @@ static void fill_eval6_params(wfsa_dev* h, Eval6Params& P)
     // static share of the regular groups: 70 % measured best for the full corpus; none when CTAs are dedicated to their big
     // groups first (a CTA that starts late cannot give its static share away)
     P.static_pct = getenv("WFSA_E6_STATIC") ? std::min(100, std::max(0, atoi(getenv("WFSA_E6_STATIC")))) : 70;
-    P.xs = h->d_klxs.p; P.xs_rows = (size_t)std::max<int64_t>(h->kl_max_words, 1);
+    P.xs = h->d_seg_xs.p; P.xs_rows = (size_t)std::max<int64_t>(h->seg_max_big_rows, 1);
     P.arc_tp = h->d_arc_tp.p; P.x = h->d_x.p; P.n = h->n; P.n_arcs = h->larcs.n_arcs;
-    P.direct_exp = (size_t)h->n > (size_t)h->kl_block * h->kl_K ? 1 : 0;
-    P.aw_g = h->d_klaw.p;
-    P.const_acc = h->d_klconst.p; P.acc = h->d_e6acc.p; P.replicas = h->replicas;
+    P.direct_exp = (size_t)h->n > (size_t)h->seg_block * h->seg_slots ? 1 : 0;
+    P.aw_g = h->d_seg_aw.p;
+    P.const_acc = h->d_seg_const.p; P.acc = h->d_e6acc.p; P.replicas = h->replicas;
     P.fx_scale = std::ldexp(1.0, (int)h->fx_log2); P.inv_fx = std::ldexp(1.0, -(int)h->fx_log2);
     P.red = h->d_e6red.p; P.ctl = h->d_e6ctl.p;
     P.n_edges = h->n_edges; P.e_off = h->d_eoff.p; P.e_arc = h->d_earc.p; P.edge_tp = h->d_edge_tp.p; P.out = h->d_out.p;
@@ -914,7 +896,7 @@ static void fill_eval6_params(wfsa_dev* h, Eval6Params& P)
     for (int r = 0; r < 8; ++r) P.peers[r] = (h->comm && r < h->nranks) ? h->peer_ptrs[r] : nullptr;
     P.stamps = h->d_e6stamps.p;
     P.debug = getenv("WFSA_E6_DEBUG") ? atoi(getenv("WFSA_E6_DEBUG")) : 0;
-    P.pool_slots = h->kl_K; P.big_slots = h->e6_big_slots; P.big_rows = h->e6_big_rows;
+    P.pool_slots = h->seg_slots; P.big_slots = h->e6_big_slots; P.big_rows = h->e6_big_rows;
     P.big_dedicate = eval6_big_dedicate(h);
     // dedicated CTAs: the shard is small (a few regular groups per warp): everything static among the free CTAs; one global
     // ticket counter for ~3.5 k groups costs ~3 ns per ticket in the L2, i.e. ~10 us of a ~14 us phase
@@ -928,16 +910,16 @@ static cudaError_t launch_eval6(wfsa_dev* h, cudaStream_t st, bool count = true,
     if (to_host) { P.out = h->hm_out_dev; P.done_flag = h->hm_flag_dev; }
     if (x_from_host) { P.x_host = h->h_x_dev; P.x_w = h->d_x.p; }
     cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3(h->kl_grid); cfg.blockDim = dim3(h->kl_block); cfg.dynamicSmemBytes = h->e6_smem; cfg.stream = st;
+    cfg.gridDim = dim3(h->seg_grid); cfg.blockDim = dim3(h->seg_block); cfg.dynamicSmemBytes = h->e6_smem; cfg.stream = st;
     cudaLaunchAttribute at[1];
     at[0].id = cudaLaunchAttributeCooperative;             // all CTAs resident: the grid barrier and the exchange rely on it
     at[0].val.cooperative = 1;
     cfg.attrs = at; cfg.numAttrs = getenv("WFSA_E6_PLAIN_LAUNCH") ? 0 : 1;
     cudaError_t e;
     if (h->awg) e = cudaLaunchKernelEx(&cfg, k_eval6<512, true>, P);
-    else if (h->kl_block == 512) e = cudaLaunchKernelEx(&cfg, k_eval6<512>, P);
-    else if (h->kl_block == 384) e = cudaLaunchKernelEx(&cfg, k_eval6<384>, P);
-    else if (h->kl_block == 256) e = cudaLaunchKernelEx(&cfg, k_eval6<256>, P);
+    else if (h->seg_block == 512) e = cudaLaunchKernelEx(&cfg, k_eval6<512>, P);
+    else if (h->seg_block == 384) e = cudaLaunchKernelEx(&cfg, k_eval6<384>, P);
+    else if (h->seg_block == 256) e = cudaLaunchKernelEx(&cfg, k_eval6<256>, P);
     else e = cudaLaunchKernelEx(&cfg, k_eval6<128>, P);
     if (e == cudaSuccess && count) { h->launches++; h->e6_used = true; }
     return e;
@@ -963,11 +945,11 @@ static int launch_pipeline(wfsa_dev* h, int mode, int kernel, const int32_t* d_o
             const cudaError_t le = launch_eval6(h, st);
             if (le != cudaSuccess) {
                 int nb = -1;
-                if (h->kl_block == 512) cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_eval6<512>, h->kl_block, h->kl_smem);
+                if (h->seg_block == 512) cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_eval6<512>, h->seg_block, h->seg_smem);
                 cudaFuncAttributes fa{};
                 cudaFuncGetAttributes(&fa, k_eval6<512>);
-                h->err = std::string("k_eval6 launch: ") + cudaGetErrorString(le) + " (grid " + std::to_string(h->kl_grid) + ", block " + std::to_string(h->kl_block) +
-                         ", dynamic smem " + std::to_string(h->kl_smem) + ", static smem " + std::to_string(fa.sharedSizeBytes) + ", regs " + std::to_string(fa.numRegs) +
+                h->err = std::string("k_eval6 launch: ") + cudaGetErrorString(le) + " (grid " + std::to_string(h->seg_grid) + ", block " + std::to_string(h->seg_block) +
+                         ", dynamic smem " + std::to_string(h->seg_smem) + ", static smem " + std::to_string(fa.sharedSizeBytes) + ", regs " + std::to_string(fa.numRegs) +
                          ", local " + std::to_string(fa.localSizeBytes) + ", max dyn smem " + std::to_string(fa.maxDynamicSharedSizeBytes) + ", occupancy " + std::to_string(nb) + " CTAs/SM)";
                 cudaGetLastError();
                 return WFSA_ERR_CUDA;
@@ -998,22 +980,17 @@ static int launch_pipeline(wfsa_dev* h, int mode, int kernel, const int32_t* d_o
             k_state_final_weights<<<(F.n_states + 255) / 256, 256, 0, st>>>(F.n_states, h->d_state_final.p, h->d_tw.p, h->d_fws.p);
             h->launches++;
         }
-        if (kernel == 5 || kernel == 6) {
+        if (kernel == 6) {
             const int na = h->larcs.n_arcs;
-            if (kernel == 6) {
-                k_arc_weights_log<<<(na + 255) / 256, 256, 0, st>>>(na, h->d_kl_arc_tid.p, h->d_kl_arc_eid.p, h->d_trans_tp.p,
-                                                                  h->d_emis_tp.p, h->d_x.p, h->d_klaw.p, h->d_klogaw.p, h->d_klconst.p,
-                                                                  std::ldexp(1.0, -(int)h->fx_log2), std::ldexp(1.0, (int)h->ll_log2),
-                                                                  h->d_llpart.p);
-                h->llpart_n = (na + 255) / 256;
-            } else {
-                k_arc_weights<<<(na + 255) / 256, 256, 0, st>>>(na, h->d_kl_arc_tid.p, h->d_kl_arc_eid.p, h->d_emis_tp.p, h->d_tw.p,
-                                                              h->d_x.p, unit, h->d_klaw.p);
-            }
+            k_arc_weights_log<<<(na + 255) / 256, 256, 0, st>>>(na, h->d_seg_arc_tid.p, h->d_seg_arc_eid.p, h->d_trans_tp.p,
+                                                              h->d_emis_tp.p, h->d_x.p, h->d_seg_aw.p, h->d_seg_logaw.p, h->d_seg_const.p,
+                                                              std::ldexp(1.0, -(int)h->fx_log2), std::ldexp(1.0, (int)h->ll_log2),
+                                                              h->d_llpart.p);
+            h->llpart_n = (na + 255) / 256;
             h->launches++;
             // replica 0 starts from the constant part (bridge edges: posterior exactly 1), the others from 0
-            CK(cudaMemcpyAsync(h->d_klacc.p, h->d_klconst.p, (size_t)na * 8, cudaMemcpyDeviceToDevice, st));
-            if (h->replicas > 1) CK(cudaMemsetAsync(h->d_klacc.p + na, 0, (size_t)na * (h->replicas - 1) * 8, st));
+            CK(cudaMemcpyAsync(h->d_seg_acc.p, h->d_seg_const.p, (size_t)na * 8, cudaMemcpyDeviceToDevice, st));
+            if (h->replicas > 1) CK(cudaMemsetAsync(h->d_seg_acc.p + na, 0, (size_t)na * (h->replicas - 1) * 8, st));
         }
     }
     EvalOutD O{};
@@ -1031,14 +1008,14 @@ static int launch_pipeline(wfsa_dev* h, int mode, int kernel, const int32_t* d_o
     h->mid_now = nullptr;
     CK(cudaGetLastError());
     h->lean_finished = false;
-    if (fold && (kernel == 5 || kernel == 6)) {
+    if (fold && kernel == 6) {
         const int na = h->larcs.n_arcs;
-        k_arcs_to_edges<<<(na + 255) / 256, 256, 0, st>>>(na, 0, F.n_trans(), h->d_klacc.p, h->replicas, h->d_kl_arc_tid.p,
-                                                         h->d_kl_arc_eid.p, nullptr, h->d_red.p + 2);
+        k_arcs_to_edges<<<(na + 255) / 256, 256, 0, st>>>(na, 0, F.n_trans(), h->d_seg_acc.p, h->replicas, h->d_seg_arc_tid.p,
+                                                         h->d_seg_arc_eid.p, nullptr, h->d_red.p + 2);
         h->launches++;
         CK(cudaGetLastError());
     }
-    const bool fast_used = (kernel == 5 || kernel == 6) ? (kernel2 == 1 || kernel2 == 2) && n_order2 > 0 : (kernel != 3);
+    const bool fast_used = kernel == 6 ? (kernel2 == 1 || kernel2 == 2) && n_order2 > 0 : (kernel != 3);
     if (fold && h->fast.ok && fast_used) {
         const int total = h->fast.n_arcs + F.n_states;
         k_arcs_to_edges<<<(total + 255) / 256, 256, 0, st>>>(h->fast.n_arcs, F.n_states, F.n_trans(), h->d_acc.p, h->replicas,
@@ -1140,7 +1117,7 @@ extern "C" int wfsa_dev_set_param_map(wfsa_dev* h, const int32_t* trimmed, int32
             tokens += len; max_len = std::max<int>(max_len, (int)len);
         }
     h->n_active = (int64_t)order.size(); h->n_active_w = (int64_t)order_w.size(); h->n_active_tokens = tokens;
-    if (h->kernel != 5 && h->kernel != 6) {
+    if (h->kernel != 6) {
         if (!order.empty()) CK(cudaMemcpyAsync(h->d_order.p, order.data(), order.size() * 4, cudaMemcpyHostToDevice, h->stream));
         if (!order_w.empty()) CK(cudaMemcpyAsync(h->d_order_w.p, order_w.data(), order_w.size() * 4, cudaMemcpyHostToDevice, h->stream));
     }
@@ -1174,7 +1151,7 @@ extern "C" int wfsa_dev_set_param_map(wfsa_dev* h, const int32_t* trimmed, int32
         if (h->ks_thread.joinable()) h->ks_thread.join();       // the layout job of a previous parameter map
         h->ks_job.reset(); h->ks_sc.reset(); h->ks_failed = false;
         SegmentedCorpus sc;
-        h->ks_job = compile_corpus_regions(h->fsa, A, alive.data(), h->h_tokens.data(), h->h_offs.data(), h->h_p.data(), order, h->kl_K,
+        h->ks_job = compile_corpus_regions(h->fsa, A, alive.data(), h->h_tokens.data(), h->h_offs.data(), h->h_p.data(), order, h->seg_slots,
                                            std::ldexp(1.0, (int)h->fx_log2), sc);
         h->ks_sc.reset(new SegmentedCorpus());
         {
@@ -1194,13 +1171,13 @@ extern "C" int wfsa_dev_set_param_map(wfsa_dev* h, const int32_t* trimmed, int32
         h->seg_types = sc.n_types; h->seg_instances = sc.n_region_instances; h->seg_region_edges = sc.n_region_edges;
         h->seg_type_edges = sc.n_type_edges; h->seg_bridges = sc.n_bridge; h->seg_host_ms = sc.host_ms;
         h->seg_words = (int64_t)sc.rwords.size();               // + the per-string words once they are built
-        h->kl_max_words = sc.max_big_rows;
+        h->seg_max_big_rows = sc.max_big_rows;
         CK(h->d_krwords.upload(sc.rwords, h->stream)); CK(h->d_krgoff.upload(sc.rgoff, h->stream));
         CK(h->d_krgrows.upload(sc.rgrows, h->stream)); CK(h->d_krW.upload(sc.typeW, h->stream));
         CK(h->d_krlq.alloc((size_t)h->kr_groups * 32 + 1));
         CK(cudaMemsetAsync(h->d_krlq.p, 0, h->d_krlq.n * 8, h->stream));
         std::vector<unsigned long long> cacc(sc.const_acc.begin(), sc.const_acc.end());
-        CK(cudaMemcpyAsync(h->d_klconst.p, cacc.data(), cacc.size() * 8, cudaMemcpyHostToDevice, h->stream));
+        CK(cudaMemcpyAsync(h->d_seg_const.p, cacc.data(), cacc.size() * 8, cudaMemcpyHostToDevice, h->stream));
         if (!order_w.empty()) CK(cudaMemcpyAsync(h->d_order_w.p, order_w.data(), order_w.size() * 4, cudaMemcpyHostToDevice, h->stream));
         {   // single-launch evaluation (k_eval6): trimmed parameters per arc, class table of the regular groups, two accumulator buffers
             std::vector<int2> atp((size_t)A.n_arcs);
@@ -1215,16 +1192,16 @@ extern "C" int wfsa_dev_set_param_map(wfsa_dev* h, const int32_t* trimmed, int32
                 if (cls.empty() || cls.back().code != code) cls.push_back(Eval6Cls{(int)g, code, (long long)sc.rgoff[g]});
             }
             h->e6_ncls = (int)cls.size();
-            h->e6_ok = regular && cls.size() <= (size_t)kE6MaxCls && (h->kl_block == 512 || h->kl_block == 384 || h->kl_block == 256 || h->kl_block == 128) && h->kr_groups < (int64_t)0x7fffffff && !getenv("WFSA_EVAL6_OFF");
+            h->e6_ok = regular && cls.size() <= (size_t)kE6MaxCls && (h->seg_block == 512 || h->seg_block == 384 || h->seg_block == 256 || h->seg_block == 128) && h->kr_groups < (int64_t)0x7fffffff && !getenv("WFSA_EVAL6_OFF");
             if (cls.empty()) cls.push_back(Eval6Cls{0, 4, 0});
             {   // staging areas for the big DAG groups in the shared memory the tables and the pool leave free
-                const size_t room = (size_t)(227 * 1024 - 8192) - h->kl_smem;
+                const size_t room = (size_t)(227 * 1024 - 8192) - h->seg_smem;
                 int rows = (int)std::max<int64_t>(sc.max_big_rows, 0);
                 if (rows > 0 && (size_t)rows * 384 > room) rows = (int)(room / 384 / 16) * 16;      // larger groups stay in HBM
                 h->e6_big_rows = rows;
                 h->e6_big_slots = rows > 0 ? (int)std::min<size_t>(4, room / ((size_t)rows * 384)) : 0;
                 if (getenv("WFSA_E6_NO_STAGING")) h->e6_big_slots = 0;
-                h->e6_smem = h->kl_smem + (size_t)h->e6_big_slots * h->e6_big_rows * 384;
+                h->e6_smem = h->seg_smem + (size_t)h->e6_big_slots * h->e6_big_rows * 384;
             }
             CK(h->d_e6cls.upload(cls, h->stream));
             const size_t cells = (size_t)A.n_arcs * h->replicas;
@@ -1234,10 +1211,10 @@ extern "C" int wfsa_dev_set_param_map(wfsa_dev* h, const int32_t* trimmed, int32
             CK(cudaMemsetAsync(h->d_e6red.p, 0, 16, h->stream));
             CK(cudaStreamSynchronize(h->stream));
         }
-        const size_t warps = (size_t)h->kl_grid * h->kl_block / 32;
+        const size_t warps = (size_t)h->seg_grid * h->seg_block / 32;
         const size_t need = warps * (size_t)std::max<int64_t>(sc.max_big_rows, 1) * 32;
-        if (h->d_klxs.n < need) {
-            const cudaError_t e = h->d_klxs.alloc(need);
+        if (h->d_seg_xs.n < need) {
+            const cudaError_t e = h->d_seg_xs.alloc(need);
             if (e != cudaSuccess) return set_err(h, WFSA_ERR_NOMEM, "segmented kernel: cannot allocate the per-warp x stacks");
         }
         CK(cudaStreamSynchronize(h->stream));
@@ -1345,35 +1322,6 @@ extern "C" int wfsa_dev_set_param_map(wfsa_dev* h, const int32_t* trimmed, int32
             }
         }
         h->k7_host_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_begin).count();
-    }
-    if (h->kernel == 5) {
-        // compile the trimmed lattice of every participating string (structure is independent of x)
-        const LatticeArcs& A = h->larcs;
-        std::vector<uint8_t> alive((size_t)A.n_arcs);
-        for (int a = 0; a < A.n_arcs; ++a)
-            alive[a] = ttp[A.arc_tid[a]] != -2 && (A.arc_eid[a] < 0 || etp[A.arc_eid[a]] != -2);
-        CompiledCorpus cc;
-        compile_corpus(h->fsa, A, alive.data(), h->h_tokens.data(), h->h_offs.data(), h->h_p.data(), order, h->kl_K,
-                       std::ldexp(1.0, (int)h->fx_log2), h->kl_bridges, 8192, cc);
-        // strings that need more pool slots, and strings without a path under this trim map (their q is 0:
-        // the numeric kernels report them as non-finite), go to the secondary kernel
-        order_w = cc.overflow;
-        order_w.insert(order_w.end(), cc.rejected.begin(), cc.rejected.end());
-        h->n_active = (int64_t)order.size() - (int64_t)order_w.size(); h->n_active_w = (int64_t)order_w.size();
-        h->kl_groups = (int64_t)cc.goff.size() - 1; h->kl_words = cc.n_words; h->kl_edges = cc.n_edges;
-        h->kl_bridge_edges = cc.n_bridge; h->kl_max_words = cc.max_words;
-        CK(h->d_klwords.upload(cc.words, h->stream)); CK(h->d_klgoff.upload(cc.goff, h->stream));
-        CK(h->d_klgsid.upload(cc.gsid, h->stream));
-        std::vector<unsigned long long> cacc(cc.const_acc.begin(), cc.const_acc.end());
-        CK(cudaMemcpyAsync(h->d_klconst.p, cacc.data(), cacc.size() * 8, cudaMemcpyHostToDevice, h->stream));
-        if (!order_w.empty()) CK(cudaMemcpyAsync(h->d_order_w.p, order_w.data(), order_w.size() * 4, cudaMemcpyHostToDevice, h->stream));
-        const size_t warps = (size_t)h->kl_grid * h->kl_block / 32;
-        const size_t need = warps * (size_t)std::max<int64_t>(cc.max_words, 1) * 32;
-        if (h->d_klxs.n < need) {
-            const cudaError_t e = h->d_klxs.alloc(need);
-            if (e != cudaSuccess) return set_err(h, WFSA_ERR_NOMEM, "compiled-lattice kernel: cannot allocate the per-warp x stacks");
-        }
-        CK(cudaStreamSynchronize(h->stream));
     }
     if (h->n != n) {
         CK(h->h_out.alloc((size_t)n + 3));                       // [loglik, non-finite terms, grad[n], epoch of a timed-out exchange]
@@ -1610,12 +1558,12 @@ extern "C" int wfsa_dev_eval_fetch(wfsa_dev* h, double* loglik, double* logq, do
     if (logq && h->kernel == 6 && h->ks_groups > 0) {
         if (!h->ks_done) {                       // per-string log q of the segmented path, from the lq of the last evaluation
             KSParams S{};
-            S.logaw = h->d_klogaw.p; S.words = h->d_kswords.p; S.sgoff = h->d_ksgoff.p; S.gref = h->d_ksgref.p; S.lq = h->d_krlq.p;
-            S.p = h->d_ksp.p; S.logq = h->d_kslogq.p; S.n_sgroups = h->ks_groups; S.counter = h->d_klcounter.p + 1;
+            S.logaw = h->d_seg_logaw.p; S.words = h->d_kswords.p; S.sgoff = h->d_ksgoff.p; S.gref = h->d_ksgref.p; S.lq = h->d_krlq.p;
+            S.p = h->d_ksp.p; S.logq = h->d_kslogq.p; S.n_sgroups = h->ks_groups; S.counter = h->d_seg_counter.p + 1;
             S.n_arcs = h->larcs.n_arcs;
-            CK(cudaMemsetAsync(h->d_klcounter.p + 1, 0, 4, h->stream));
+            CK(cudaMemsetAsync(h->d_seg_counter.p + 1, 0, 4, h->stream));
             if (h->e6_used && h->lean_now) {     // the single-launch evaluation keeps the arc weights on chip: log weights from x now
-                k_arc_logw<<<(h->larcs.n_arcs + 255) / 256, 256, 0, h->stream>>>(h->larcs.n_arcs, h->d_arc_tp.p, h->d_x.p, h->d_klogaw.p);
+                k_arc_logw<<<(h->larcs.n_arcs + 255) / 256, 256, 0, h->stream>>>(h->larcs.n_arcs, h->d_arc_tp.p, h->d_x.p, h->d_seg_logaw.p);
                 h->launches++;
             }
             if (h->awg) ks_strings<true><<<h->ks_grid, h->ks_block, 0, h->stream>>>(S); else ks_strings<false><<<h->ks_grid, h->ks_block, h->ks_smem, h->stream>>>(S);
@@ -1933,8 +1881,8 @@ extern "C" int wfsa_dev_hessian(wfsa_dev* h, const double* x, double* Hf, double
             if (h->d_zero_logaw.n < (size_t)h->larcs.n_arcs + 16) { CK(h->d_zero_logaw.alloc((size_t)h->larcs.n_arcs + 16)); CK(cudaMemsetAsync(h->d_zero_logaw.p, 0, h->d_zero_logaw.n * 8, h->stream)); }
             KSParams S{};
             S.logaw = h->d_zero_logaw.p; S.words = h->d_kswords.p; S.sgoff = h->d_ksgoff.p; S.gref = h->d_ksgref.p; S.lq = h->d_type_lrmin.p;
-            S.p = h->d_ksp.p; S.logq = h->d_kslogq.p; S.n_sgroups = h->ks_groups; S.counter = h->d_klcounter.p + 1; S.n_arcs = h->larcs.n_arcs;
-            CK(cudaMemsetAsync(h->d_klcounter.p + 1, 0, 4, h->stream));
+            S.p = h->d_ksp.p; S.logq = h->d_kslogq.p; S.n_sgroups = h->ks_groups; S.counter = h->d_seg_counter.p + 1; S.n_arcs = h->larcs.n_arcs;
+            CK(cudaMemsetAsync(h->d_seg_counter.p + 1, 0, 4, h->stream));
             CK(cudaMemsetAsync(h->d_kslogq.p, 0, h->d_kslogq.n * 8, h->stream));
             if (h->awg) ks_strings<true><<<h->ks_grid, h->ks_block, 0, h->stream>>>(S); else ks_strings<false><<<h->ks_grid, h->ks_block, h->ks_smem, h->stream>>>(S);
             k_min_exp<<<1, 1024, 0, h->stream>>>((long long)h->d_kslogq.n, h->d_kslogq.p, h->d_rmin.p);
@@ -2010,22 +1958,22 @@ extern "C" int wfsa_dev_eval6_phases(wfsa_dev* h, double* out4, int reset)
     if (getenv("WFSA_E6_DEBUG"))
         fprintf(stderr, "[k_eval6 debug] longest group %.2f us (rows code 0x%x), latest end of the region phase %.2f us after the start of CTA 0, longest wait for staged words %.2f us\n",
                 (double)(v[4] >> 32) * 1e-3, (unsigned)(v[4] & 0xffffffffu), (double)v[5] * 1e-3, (double)v[7] * 1e-3);
-    if (getenv("WFSA_E6_DEBUG") && (atoi(getenv("WFSA_E6_DEBUG")) & 16) && h->kl_grid <= 1024) {
+    if (getenv("WFSA_E6_DEBUG") && (atoi(getenv("WFSA_E6_DEBUG")) & 16) && h->seg_grid <= 1024) {
         // per-CTA timeline of the last launch: when each phase ended, relative to the earliest CTA start
-        std::vector<unsigned long long> tl((size_t)h->kl_grid * 8);
+        std::vector<unsigned long long> tl((size_t)h->seg_grid * 8);
         CK(cudaMemcpy(tl.data(), h->d_e6stamps.p + 8, tl.size() * 8, cudaMemcpyDeviceToHost));
         unsigned long long t0 = ~0ull;
-        for (int b = 0; b < h->kl_grid; ++b) t0 = std::min(t0, tl[(size_t)b * 8]);
+        for (int b = 0; b < h->seg_grid; ++b) t0 = std::min(t0, tl[(size_t)b * 8]);
         const char* nm[5] = {"start", "weights done", "regions done", "barrier passed", "end"};
         for (int k = 0; k < 5; ++k) {
             double mn = 1e30, mx = 0, sum = 0; int amx = 0;
-            for (int b = 0; b < h->kl_grid; ++b) { const double d = (double)(tl[(size_t)b * 8 + k] - t0) * 1e-3; if (d < mn) mn = d; if (d > mx) { mx = d; amx = b; } sum += d; }
-            fprintf(stderr, "[k_eval6 timeline] %-14s min %7.2f  mean %7.2f  max %7.2f us (CTA %d)\n", nm[k], mn, sum / h->kl_grid, mx, amx);
+            for (int b = 0; b < h->seg_grid; ++b) { const double d = (double)(tl[(size_t)b * 8 + k] - t0) * 1e-3; if (d < mn) mn = d; if (d > mx) { mx = d; amx = b; } sum += d; }
+            fprintf(stderr, "[k_eval6 timeline] %-14s min %7.2f  mean %7.2f  max %7.2f us (CTA %d)\n", nm[k], mn, sum / h->seg_grid, mx, amx);
         }
         if (atoi(getenv("WFSA_E6_DEBUG")) & 32) {             // every CTA: time from the grid barrier to its end (fold + exchange)
             std::string line = "[k_eval6 timeline] rank " + std::to_string(h->rank) + " fold+exchange us per CTA:";
             char buf[32];
-            for (int b = 0; b < h->kl_grid; ++b) { snprintf(buf, sizeof buf, " %.1f", (double)(tl[(size_t)b * 8 + 4] - tl[(size_t)b * 8 + 3]) * 1e-3); line += buf; }
+            for (int b = 0; b < h->seg_grid; ++b) { snprintf(buf, sizeof buf, " %.1f", (double)(tl[(size_t)b * 8 + 4] - tl[(size_t)b * 8 + 3]) * 1e-3); line += buf; }
             fprintf(stderr, "%s\n", line.c_str());
         }
     }
@@ -2216,30 +2164,6 @@ extern "C" int wfsa_lattice_compile(const wfsa_fsa_desc* fd, const int32_t* trim
     return WFSA_OK;
 }
 
-extern "C" int wfsa_lattice_stats(const wfsa_fsa_desc* fd, const wfsa_corpus_desc* cd, int32_t n_slots, double* out8)
-{
-    g_create_error.clear();
-    if (!fd || !cd || !out8 || n_slots < 1 || n_slots > kLatMaxSlots || cd->n_strings < 0) { g_create_error = "lattice_stats: bad arguments"; return WFSA_ERR_INVALID; }
-    HostFsa f; GenericLayout g; LatticeArcs A;
-    int status = WFSA_OK;
-    std::string msg = copy_and_validate(fd, f, status);
-    if (status == WFSA_OK) msg = build_generic_layout(f, g, status);
-    if (status != WFSA_OK) { g_create_error = msg; return status; }
-    build_lattice_arcs(f, g, A);
-    std::vector<int32_t> ids((size_t)cd->n_strings);
-    std::iota(ids.begin(), ids.end(), 0);
-    std::stable_sort(ids.begin(), ids.end(), [&](int32_t a, int32_t b) {
-        return (cd->offsets[a + 1] - cd->offsets[a]) > (cd->offsets[b + 1] - cd->offsets[b]);
-    });
-    CompiledCorpus cc;
-    const auto t0 = std::chrono::steady_clock::now();
-    compile_corpus(f, A, nullptr, cd->tokens, cd->offsets, cd->p, ids, n_slots, 1.0, true, 8192, cc);
-    const double ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
-    out8[0] = (double)cc.n_edges; out8[1] = (double)cc.n_bridge; out8[2] = (double)cc.n_words; out8[3] = (double)cc.max_words;
-    out8[4] = (double)cc.overflow.size(); out8[5] = (double)cc.rejected.size(); out8[6] = (double)cc.goff.size() - 1; out8[7] = ms;
-    return WFSA_OK;
-}
-
 struct wfsa_segmented {
     SegmentedCorpus sc;
     LatticeArcs arcs;
@@ -2315,30 +2239,25 @@ extern "C" int wfsa_dev_get_info(wfsa_dev* h, wfsa_dev_info* info)
     info->n_arcs = h->fast.ok ? h->fast.n_arcs : 0; info->n_slots = h->fast.ok ? h->fast.n_slots : 0;
     info->max_candidates = h->fast.ok ? h->fast.max_cand : 0;
     info->sm_count = h->sm_count;
-    info->grid = h->kernel >= 5 ? h->kl_grid : (h->kernel == 4 ? h->kt_grid : (h->kernel == 2 ? h->k3_grid : h->grid));
-    info->block = h->kernel >= 5 ? h->kl_block : (h->kernel == 4 ? h->kt_block : (h->kernel == 2 ? h->k3_block : (h->kernel == 3 ? 128 : h->block)));
+    info->grid = h->kernel == 6 ? h->seg_grid : (h->kernel == 4 ? h->kt_grid : (h->kernel == 2 ? h->k3_grid : h->grid));
+    info->block = h->kernel == 6 ? h->seg_block : (h->kernel == 4 ? h->kt_block : (h->kernel == 2 ? h->k3_block : (h->kernel == 3 ? 128 : h->block)));
     if (h->kernel == 7) { info->grid = 0; info->block = h->k7_V; }
     info->n_strings = h->n_strings; info->n_tokens = h->n_tokens;
     info->n_active_tokens = h->n_active_tokens;
-    info->smem_bytes = (int64_t)(h->kernel >= 5 ? h->kl_smem : (h->kernel == 4 ? h->kt_smem : (h->kernel == 2 ? h->k3_smem : h->smem_bytes)));
+    info->smem_bytes = (int64_t)(h->kernel == 6 ? h->seg_smem : (h->kernel == 4 ? h->kt_smem : (h->kernel == 2 ? h->k3_smem : h->smem_bytes)));
     if (h->kernel == 7) { info->smem_bytes = (int64_t)kK7Chunk * h->k7_V * 8; info->seg_host_ms = h->k7_host_ms; info->lattice_words = (int64_t)h->k7_rows * h->k7_V * 2; info->pool_slots = (int32_t)h->k7.size(); }
-    if (h->kernel == 5) {
-        info->n_arcs = h->larcs.n_arcs;
-        info->lattice_words = h->kl_words; info->lattice_edges = h->kl_edges; info->lattice_bridge_edges = h->kl_bridge_edges;
-        info->n_overflow_strings = h->n_active_w; info->pool_slots = h->kl_K;
-    }
     if (h->kernel == 6) {
         { const int rc = ensure_ks(h); if (rc != WFSA_OK) return rc; }     // word counts and compile time include the per-string layout
         info->n_arcs = h->larcs.n_arcs;
         info->lattice_words = h->seg_words; info->lattice_edges = h->seg_bridges + h->seg_region_edges;
-        info->lattice_bridge_edges = h->seg_bridges; info->n_overflow_strings = h->n_active_w; info->pool_slots = h->kl_K;
+        info->lattice_bridge_edges = h->seg_bridges; info->n_overflow_strings = h->n_active_w; info->pool_slots = h->seg_slots;
         info->seg_types = h->seg_types; info->seg_region_instances = h->seg_instances; info->seg_region_edges = h->seg_region_edges;
         info->seg_type_edges = h->seg_type_edges; info->seg_host_ms = h->seg_host_ms;
         if (h->n >= 0) {                                           // the conditions of k_eval6's P1 (kernels_eval6.cuh)
             info->e6_big_groups = h->kr_big_groups; info->e6_big_dedicate = eval6_big_dedicate(h);
-            info->e6_big_slots = h->e6_big_slots; info->e6_big_rows = h->e6_big_rows; info->e6_max_big_rows = (int32_t)h->kl_max_words;
+            info->e6_big_slots = h->e6_big_slots; info->e6_big_rows = h->e6_big_rows; info->e6_max_big_rows = (int32_t)h->seg_max_big_rows;
             int two = 0;
-            if (h->kr_big_groups <= h->kl_grid && h->e6_big_slots >= 2)
+            if (h->kr_big_groups <= h->seg_grid && h->e6_big_slots >= 2)
                 for (int64_t b = 0; b < h->kr_big_groups; ++b)
                     two += (h->hrgoff[b + 1] - h->hrgoff[b]) >> 5 <= h->e6_big_rows && !(h->hrgrows[b] & 0x10000);
             info->e6_two_warp_eligible = two;

@@ -20,7 +20,7 @@ DEV_SYMBOLS = [
     "wfsa_dev_eval_launch", "wfsa_dev_eval_fetch", "wfsa_dev_sync", "wfsa_dev_set_path_blocks", "wfsa_dev_hessian",
     "wfsa_dev_comm_unique_id", "wfsa_dev_comm_init", "wfsa_dev_allreduce_f64", "wfsa_dev_timer_begin", "wfsa_dev_timer_begin_steps",
     "wfsa_dev_timer_end", "wfsa_dev_timer_kernel_ms", "wfsa_dev_timer_split_ms", "wfsa_dev_timer_step_ms", "wfsa_dev_timer_phase_ms", "wfsa_dev_eval6_phases", "wfsa_dev_l2_flush", "wfsa_dev_rank_barrier", "wfsa_dev_get_info", "wfsa_dev_destroy", "wfsa_dev_held_bytes", "wfsa_dev_last_error",
-    "wfsa_dev_version", "wfsa_lattice_compile", "wfsa_lattice_stats", "wfsa_segmented_compile", "wfsa_segmented_get",
+    "wfsa_dev_version", "wfsa_lattice_compile", "wfsa_segmented_compile", "wfsa_segmented_get",
     "wfsa_segmented_free",
 ]
 HOST_SYMBOLS = [
@@ -145,7 +145,6 @@ def lib():
         L.wfsa_dev_timer_phase_ms.argtypes = [C.c_void_p, C.POINTER(C.c_float)]
         L.wfsa_dev_eval6_phases.argtypes = [C.c_void_p, F64P, C.c_int]
         L.wfsa_dev_get_info.argtypes = [C.c_void_p, C.POINTER(DevInfo)]
-        L.wfsa_lattice_stats.argtypes = [C.POINTER(FsaDesc), C.POINTER(CorpusDesc), C.c_int32, F64P]
         L.wfsa_lattice_compile.argtypes = [C.POINTER(FsaDesc), I32P, I32P, C.c_int32, C.c_int32, C.POINTER(C.c_uint32), C.c_int64,
                                            I64P, I32P, I32P, C.c_int32, I32P]
         L.wfsa_segmented_compile.argtypes = [C.POINTER(FsaDesc), C.POINTER(CorpusDesc), I32P, C.c_int32, C.c_double,

@@ -225,7 +225,8 @@ int wfsa_lattice_compile(const wfsa_fsa_desc* fsa, const int32_t* trimmed, const
  *        13 path_off(i64) 14 col_off(i64) 15 val_off(i64) 16 cols(i32) 17 counts(f64) 18 p(f64) 19 type slot(i32): the path blocks
  *           wfsa_dev_hessian derives from the region types (layout of wfsa_path_blocks, p = weight of the type).  The
  *           evaluation does not need them: a shard whose blocks cannot be built still compiles (wfsa_dev_hessian of such
- *           a shard returns WFSA_ERR_LIMIT). */
+ *           a shard returns WFSA_ERR_LIMIT).
+ *        20 pwords(u32) 21 pgoff(i64): the reduction plan of the path-form groups (lattice.hpp, SegmentedCorpus::pwords) */
 typedef struct wfsa_segmented wfsa_segmented;
 int wfsa_segmented_compile(const wfsa_fsa_desc* fsa, const wfsa_corpus_desc* corpus, const int32_t* trimmed,
                            int32_t n_slots, double fx_scale, wfsa_segmented** out);

@@ -7,8 +7,8 @@
 //       (exp(x) once per parameter, then one product per combined arc), adds its share of the bridge part of the
 //       log-likelihood (sum_arc c[arc] * log w[arc], kernels_seg.cuh) and re-arms the accumulator buffer and the
 //       ticket counter of the NEXT evaluation (two of each, used alternately);
-//   P1  region types, 32 to a warp, handed out by a ticket counter (kr_regions' loop).  Path-form types of the common
-//       shapes are fully unrolled: all rows of a group are loaded in one round trip and stay in registers for the REDs;
+//   P1  region types, 32 to a warp, handed out by a ticket counter (kr_regions' loop).  Path-form types: the rows of a group
+//       in batches of one round trip each, one RED per distinct arc of the group from its reduction plan (kr_paths);
 //       group descriptors of the regular classes come from a class table in shared memory, not from HBM; big DAG groups are
 //       staged in shared memory and, when a CTA owns one, walked by two warps (forward chain on warp 0, backward chain on
 //       warp 1, REDs on warp 0: kernels_seg.cuh big_fwd / big_bwd<false> / big_red<true>), else by one (big_one);
@@ -34,6 +34,8 @@ struct Eval6Params {
     const int64_t* __restrict__ goff;
     const int32_t* __restrict__ grows;
     const double* __restrict__ typeW;
+    const uint32_t* __restrict__ pwords;        // reduction plan of the path-form groups
+    const int64_t* __restrict__ pgoff;
     double* lq;
     long long n_groups, n_big;                  // groups [0, n_big): big DAG regions (descriptor from goff/grows)
     int static_pct;                             // share of the regular groups dealt out statically per CTA (the rest: ticket counter)
@@ -265,7 +267,7 @@ __global__ void __launch_bounds__(NT, 1) k_eval6(const Eval6Params P)
     if (tline) tl1 = e6_timer();
     // ---- P1: region types -------------------------------------------------------------------------------------
     KRParams R{};
-    R.words = P.words; R.goff = P.goff; R.typeW = P.typeW; R.lq = P.lq; R.xs = P.xs; R.xs_rows = P.xs_rows;
+    R.words = P.words; R.goff = P.goff; R.typeW = P.typeW; R.pwords = P.pwords; R.pgoff = P.pgoff; R.lq = P.lq; R.xs = P.xs; R.xs_rows = P.xs_rows;
     R.fx_scale = P.fx_scale; R.ll_scale = ll_scale; R.red = P.red; R.n_arcs = P.n_arcs;
     const bool path_reds = !(P.debug & 8);                     // timing experiment (debug bit 3): no REDs from path-form types
     const BigPool pl{(unsigned int)__cvta_generic_to_shared(pool), (unsigned int)NT * 8u, (unsigned int)__cvta_generic_to_shared(&s_trash[tid])};
@@ -340,11 +342,11 @@ __global__ void __launch_bounds__(NT, 1) k_eval6(const Eval6Params P)
         if (rows & 0x10000) {                                  // path form: paths << 8 | length
             const int L = rows & 0xff;
             switch ((rows >> 8) & 0xff) {
-                case 2: kr_paths<2>(R, aw, L, g, off, lane, acc_g, ll, path_reds); break;
-                case 3: kr_paths<3>(R, aw, L, g, off, lane, acc_g, ll, path_reds); break;
-                case 4: kr_paths<4>(R, aw, L, g, off, lane, acc_g, ll, path_reds); break;
-                case 6: kr_paths<6>(R, aw, L, g, off, lane, acc_g, ll, path_reds); break;
-                default: kr_paths<8>(R, aw, L, g, off, lane, acc_g, ll, path_reds); break;
+                case 2: kr_paths<2>(R, aw, pl, L, g, off, lane, acc_g, ll, path_reds); break;
+                case 3: kr_paths<3>(R, aw, pl, L, g, off, lane, acc_g, ll, path_reds); break;
+                case 4: kr_paths<4>(R, aw, pl, L, g, off, lane, acc_g, ll, path_reds); break;
+                case 6: kr_paths<6>(R, aw, pl, L, g, off, lane, acc_g, ll, path_reds); break;
+                default: kr_paths<8>(R, aw, pl, L, g, off, lane, acc_g, ll, path_reds); break;
             }
         } else {
             {

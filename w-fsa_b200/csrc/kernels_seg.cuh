@@ -26,6 +26,8 @@ struct KRParams {
     const int64_t* __restrict__ goff;     // [n_groups+1]
     const int32_t* __restrict__ grows;    // [n_groups] 0x10000|paths<<8|length = path form; 4/8/12/16 = small DAG; else big DAG (multiple of 16)
     const double* __restrict__ typeW;     // [n_groups*32]
+    const uint32_t* __restrict__ pwords;  // reduction plan of the path-form groups: word r of lane l of group g at pgoff[g] + r*32 + l
+    const int64_t* __restrict__ pgoff;    // [n_groups+1] (lattice.hpp, SegmentedCorpus::pwords)
     double* lq;                           // [n_groups*32 + 1] log q per type (last = dummy, stays 0)
     long long n_groups;
     double* xs;                           // big regions: per warp [xs_rows][32]
@@ -60,34 +62,35 @@ __device__ __forceinline__ void kr_loglik(const KRParams& P, double W, bool ok, 
     }
 }
 
-// Adds one fixed-point value per lane into acc[key].  Region types are sorted by their arcs, so at the first
-// edge positions a whole warp usually holds ONE arc: then the 32 values are summed with shuffles (integers:
-// exact, order independent) and a single RED is issued; otherwise every lane issues its own.
-// Must be called by all 32 lanes; key < 0 = nothing to add.
-__device__ __forceinline__ void red_uniform(unsigned long long* acc_g, int key, long long v, int lane)
-{
-    const int k0 = __shfl_sync(FULL, key, 0);
-    if (__all_sync(FULL, key == k0)) {
-#pragma unroll
-        for (int o = 16; o; o >>= 1) v += __shfl_xor_sync(FULL, v, o);
-        if (lane == 0 && key >= 0 && v) red_add64(acc_g + key, (unsigned long long)v);
-    } else if (key >= 0 && v) red_add64(acc_g + key, (unsigned long long)v);
-}
+// The pool of a thread: node value of slot s of the thread at shared byte address p + s * ps; trash: where a lane without an
+// edge stores (big_fwd, big_bwd).  kr_paths borrows slots 0 .. kPathSlots-1 of the warp's own columns (the pool area has
+// at least kPathSlots slots per thread).
+struct BigPool { unsigned int p, ps, trash; };
+constexpr int kPathSlots = 8;                                  // = kSegMaxPaths of lattice.hpp
+constexpr uint32_t kPLast = 1u << 31;                          // = kPlanLast of lattice.hpp
+__device__ __forceinline__ double lds_f64(unsigned int a) { double v; asm volatile("ld.shared.f64 %0, [%1];" : "=d"(v) : "r"(a)); return v; }
+__device__ __forceinline__ void sts_f64(unsigned int a, double v) { asm volatile("st.shared.f64 [%0], %1;" :: "r"(a), "d"(v)); }
+__device__ __forceinline__ long long lds_s64(unsigned int a) { long long v; asm volatile("ld.shared.s64 %0, [%1];" : "=l"(v) : "r"(a)); return v; }
+__device__ __forceinline__ void sts_s64(unsigned int a, long long v) { asm volatile("st.shared.s64 [%0], %1;" :: "r"(a), "l"(v)); }
 
 // One region in PATH FORM per thread: PP paths (padded with zero-weight paths) of L edges each, arc of edge l of path p at
 // row l*PP + p.  q = sum_p prod_l w[arc]; every edge of path p gets the posterior r_p / q.  Registers only: PP independent
 // multiply chains, no pool, no flags (the reference's P.x / exp / M algebra, src/Learner.cpp:530-545, for one small segment).
-// Levels go in batches of LB = 24 / PP: every batch is ONE round trip (LB*PP loads in flight), for the products and again for
-// the REDs (the arc ids of a long type do not fit the registers; the second pass finds them in the L1/L2); a rolled loop pays
-// a round trip per level.  One instance per PP serves every length: fully unrolled instances per (PP, L) made k_eval6 26 k
+// Levels go in batches of LB = 24 / PP: every batch is ONE round trip (LB*PP loads in flight); a rolled loop pays a round
+// trip per level.  One instance per PP serves every length: fully unrolled instances per (PP, L) made k_eval6 26 k
 // instructions, and a warp that runs a rarely used instance waits for instruction fetches from the L2 (cold after the flush)
-// far longer than for data -- measured 15-40 us for ONE group.  reds = false: no REDs (timing experiments).
+// far longer than for data -- measured 15-40 us for ONE group.
+// The REDs follow the group's reduction plan (lattice.cpp, build_path_plans): every lane parks its rounded posteriors v[p]
+// in its pool column, and walks its plan entries, each the cells (lane', p) of one arc of the group, summing v[p] of lane'
+// (64-bit integers: exact and order independent, so the accumulators get the same bits as with one RED per cell) into ONE
+// RED per entry.  reds = false: no REDs (timing experiments).
 template <int PP>
-__device__ __forceinline__ void kr_paths(const KRParams& P, const double* aw, int L, long long g, long long off, int lane,
-                                         unsigned long long* acc_g, long long& ll, bool reds)
+__device__ __forceinline__ void kr_paths(const KRParams& P, const double* aw, const BigPool& pl, int L, long long g, long long off,
+                                         int lane, unsigned long long* acc_g, long long& ll, bool reds)
 {
     constexpr int LB = 24 / PP;
     const uint32_t* wp = P.words + off + lane;
+    const long long poff = P.pgoff[g], pend = P.pgoff[g + 1];
     // more than one batch: ask for all rows of the group now (one 128-byte row per lane and round), so that the later
     // batches find them in the L2 instead of paying a DRAM round trip each (an 8 x 16 group took 26 us: twelve batches)
     if (L > LB)
@@ -100,6 +103,9 @@ __device__ __forceinline__ void kr_paths(const KRParams& P, const double* aw, in
         uint32_t a[LB * PP];
 #pragma unroll
         for (int i = 0; i < LB * PP; ++i) a[i] = l0 * PP + i < L * PP ? __ldg(wp + (size_t)(l0 * PP + i) * 32) : (uint32_t)P.n_arcs;
+        // the plan rows are on their way to the L2 while the products are formed
+        if (l0 == 0 && reds)
+            for (long long i = poff + lane * 32; i < pend; i += 32 * 32) asm volatile("prefetch.global.L2 [%0];" :: "l"(P.pwords + i));
 #pragma unroll
         for (int l = 0; l < LB; ++l)
             if (l0 + l < L) {
@@ -116,25 +122,31 @@ __device__ __forceinline__ void kr_paths(const KRParams& P, const double* aw, in
         P.lq[g * 32 + lane] = lq;
         kr_loglik(P, W, ok, lq, ll);
     }
-    const double sc = ok ? W * P.fx_scale / q : 0.0;
-    long long v[PP];
-#pragma unroll
-    for (int p = 0; p < PP; ++p) v[p] = __double2ll_rn(r[p] * sc);
     if (!reds) return;
-    for (int l0 = 0; l0 < L; l0 += LB) {
-        uint32_t a[LB * PP];
+    const double sc = ok ? W * P.fx_scale / q : 0.0;
 #pragma unroll
-        for (int i = 0; i < LB * PP; ++i) a[i] = l0 * PP + i < L * PP ? __ldg(wp + (size_t)(l0 * PP + i) * 32) : (uint32_t)P.n_arcs;
+    for (int p = 0; p < PP; ++p) sts_s64(pl.p + (unsigned int)p * pl.ps, __double2ll_rn(r[p] * sc));
+    __syncwarp();
+    const unsigned int col0 = pl.p - (unsigned int)lane * 8u;          // the warp's lane 0
+    const uint32_t* pp = P.pwords + poff + lane;
+    const int prow = (int)((pend - poff) >> 5);
+    long long s = 0;
+    for (int r0 = 0; r0 < prow; r0 += 8) {
+        uint32_t w[8];
 #pragma unroll
-        for (int l = 0; l < LB; ++l)
-            if (l0 + l < L) {
+        for (int j = 0; j < 8; ++j) w[j] = r0 + j < prow ? __ldcs(pp + (size_t)(r0 + j) * 32) : 0u;
 #pragma unroll
-                for (int p = 0; p < PP; ++p) {
-                    if (l0 + l == 0 && p < 2) red_uniform(acc_g, v[p] ? (int)a[p] : -1, v[p], lane);
-                    else if (v[p]) red_add64(acc_g + a[l * PP + p], (unsigned long long)v[p]);
+        for (int j = 0; j < 8; ++j)
+            if (r0 + j < prow) {
+                const uint32_t c = (w[j] >> 16) & 0xffu;
+                s += lds_s64(col0 + (c >> 3) * 8u + (c & 7u) * pl.ps);
+                if (w[j] & kPLast) {
+                    if (s) red_add64(acc_g + (w[j] & 0xffffu), (unsigned long long)s);
+                    s = 0;
                 }
             }
     }
+    __syncwarp();                                              // the other lanes are done with this lane's column
 }
 
 // ---- big DAG regions: the stream format of lattice.hpp (CHECK words rescale, x values on a stack), one thread per region
@@ -157,9 +169,6 @@ __device__ __forceinline__ void kr_paths(const KRParams& P, const double* aw, in
 // their order among themselves; a clobber would pin every other memory access around each of them.
 constexpr uint32_t kLEdge = 1u << 31, kLFin = 1u << 30, kLFirstIn = 1u << 29, kLLastOut = 1u << 28;   // = kLat* of lattice.hpp
 constexpr int kLBand = 200;
-struct BigPool { unsigned int p, ps, trash; };
-__device__ __forceinline__ double lds_f64(unsigned int a) { double v; asm volatile("ld.shared.f64 %0, [%1];" : "=d"(v) : "r"(a)); return v; }
-__device__ __forceinline__ void sts_f64(unsigned int a, double v) { asm volatile("st.shared.f64 [%0], %1;" :: "r"(a), "d"(v)); }
 __device__ __forceinline__ int lds_exp(unsigned int a) { int hi; asm volatile("ld.shared.u32 %0, [%1];" : "=r"(hi) : "r"(a + 4u)); return (hi >> 20) & 0x7ff; }
 
 // Where the words (row i: word of the lane) and the x stack (row i: 64 bits of the lane) of a group live.  BigSmem: the
@@ -379,11 +388,11 @@ __global__ void __launch_bounds__(MAXNT, 1) kr_regions(const KRParams P)
         if (rows & 0x10000) {                                  // path form: paths << 8 | length
             const int L = rows & 0xff;
             switch ((rows >> 8) & 0xff) {
-                case 2: kr_paths<2>(P, aw, L, g, off, lane, acc_g, ll, reds); break;
-                case 3: kr_paths<3>(P, aw, L, g, off, lane, acc_g, ll, reds); break;
-                case 4: kr_paths<4>(P, aw, L, g, off, lane, acc_g, ll, reds); break;
-                case 6: kr_paths<6>(P, aw, L, g, off, lane, acc_g, ll, reds); break;
-                default: kr_paths<8>(P, aw, L, g, off, lane, acc_g, ll, reds); break;
+                case 2: kr_paths<2>(P, aw, pl, L, g, off, lane, acc_g, ll, reds); break;
+                case 3: kr_paths<3>(P, aw, pl, L, g, off, lane, acc_g, ll, reds); break;
+                case 4: kr_paths<4>(P, aw, pl, L, g, off, lane, acc_g, ll, reds); break;
+                case 6: kr_paths<6>(P, aw, pl, L, g, off, lane, acc_g, ll, reds); break;
+                default: kr_paths<8>(P, aw, pl, L, g, off, lane, acc_g, ll, reds); break;
             }
         } else big_one(P, aw, pl, BigGmem{P.words + off + lane, xs}, (int)((P.goff[g + 1] - off) >> 5), g, lane, acc_g, ll, reds);
         g = __shfl_sync(FULL, gn, 0);

@@ -511,6 +511,75 @@ struct SegmentedStringsJob::State {
     std::vector<int32_t> ids;
     const double* p = nullptr;
 };
+// Reduction plan of every path-form group (layout: SegmentedCorpus::pwords).  Types are sorted by their arcs, so the 32
+// types of a group share most of them: summing the contributions of a group per distinct arc before the RED leaves
+// 0.6 of the REDs at 100 k config-4 strings (the sums are integers: the same bits in any order).  An entry lists the
+// cells (lane, p) of one arc in (level, path, lane) order, an arc on several levels of a path once per level; an entry
+// longer than the group's ideal stream (cells / 32 rows) is cut, so that no lane walks much more than its share.  Entries
+// are dealt out largest first (ties: lower arc), each to the lane with the shortest stream (ties: lower lane).  Groups
+// are planned on T threads in contiguous ranges: the result does not depend on T.
+static void build_path_plans(SegmentedCorpus& out, int n_arcs, int T)
+{
+    const int64_t n_rg = (int64_t)out.rgrows.size();
+    std::vector<int64_t> rows_of((size_t)n_rg, 0);
+    std::vector<std::vector<uint32_t>> part(T);
+    auto plan = [&](int t) {
+        const int64_t g0 = n_rg * t / T, g1 = n_rg * (t + 1) / T;
+        std::vector<uint64_t> cells;                                      // arc << 32 | cell index (level, path, lane) << 8 | code
+        std::vector<std::pair<int, int>> ent;                             // [begin, end) in cells
+        std::vector<uint32_t> lanes[32];
+        for (int64_t g = g0; g < g1; ++g) {
+            const int32_t code = out.rgrows[g];
+            if (!(code & 0x10000)) continue;
+            const int PP = (code >> 8) & 0xff, L = code & 0xff;
+            const uint32_t* w = out.rwords.data() + out.rgoff[g];
+            cells.clear();
+            for (int k = 0; k < PP * L; ++k)
+                for (int ln = 0; ln < 32; ++ln)
+                    if (w[(size_t)k * 32 + ln] != (uint32_t)n_arcs)
+                        cells.push_back((uint64_t)w[(size_t)k * 32 + ln] << 32 | (uint64_t)(k * 32 + ln) << 8 | (uint64_t)(ln << 3 | k % PP));
+            if (cells.empty()) continue;
+            std::sort(cells.begin(), cells.end());
+            const int cap = (int)((cells.size() + 31) / 32);
+            ent.clear();
+            for (size_t b = 0; b < cells.size();) {
+                size_t e = b;
+                while (e < cells.size() && (cells[e] >> 32) == (cells[b] >> 32)) ++e;
+                for (size_t c = b; c < e; c += (size_t)cap) ent.emplace_back((int)c, (int)std::min(e, c + (size_t)cap));
+                b = e;
+            }
+            std::stable_sort(ent.begin(), ent.end(), [](const std::pair<int, int>& x, const std::pair<int, int>& y) {
+                return x.second - x.first > y.second - y.first;
+            });
+            for (auto& v : lanes) v.clear();
+            for (const auto& [b, e] : ent) {
+                int best = 0;
+                for (int ln = 1; ln < 32; ++ln) if (lanes[ln].size() < lanes[best].size()) best = ln;
+                for (int c = b; c < e; ++c)
+                    lanes[best].push_back((uint32_t)(cells[c] >> 32) | (uint32_t)(cells[c] & 0xff) << 16 | (c + 1 == e ? kPlanLast : 0u));
+            }
+            size_t rows = 0;
+            for (const auto& v : lanes) rows = std::max(rows, v.size());
+            rows_of[g] = (int64_t)rows;
+            std::vector<uint32_t>& dst = part[t];
+            for (size_t r = 0; r < rows; ++r)
+                for (int ln = 0; ln < 32; ++ln) dst.push_back(r < lanes[ln].size() ? lanes[ln][r] : 0u);
+        }
+    };
+    {
+        std::vector<std::thread> th;
+        for (int t = 1; t < T; ++t) th.emplace_back(plan, t);
+        plan(0);
+        for (auto& x : th) x.join();
+    }
+    out.pgoff.assign((size_t)n_rg + 1, 0);
+    for (int64_t g = 0; g < n_rg; ++g) out.pgoff[g + 1] = out.pgoff[g] + rows_of[g] * 32;
+    out.pwords.clear();
+    out.pwords.reserve((size_t)out.pgoff[n_rg] + 32);
+    for (int t = 0; t < T; ++t) { out.pwords.insert(out.pwords.end(), part[t].begin(), part[t].end()); std::vector<uint32_t>().swap(part[t]); }
+    out.pwords.resize((size_t)out.pgoff[n_rg] + 32, 0u);
+}
+
 SegmentedStringsJob::SegmentedStringsJob() : st(new State) {}
 SegmentedStringsJob::~SegmentedStringsJob() { delete st; }
 
@@ -781,6 +850,8 @@ std::shared_ptr<SegmentedStringsJob> compile_corpus_regions(const HostFsa& f, co
         for (int t = 0; t < T; ++t) out.n_type_edges += edges_of[t];
     }
     lap("region layout");
+    build_path_plans(out, A.n_arcs, T);
+    lap("reduction plans");
     out.host_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_begin).count();
     auto job = std::make_shared<SegmentedStringsJob>();
     SegmentedStringsJob::State& S = *job->st;

@@ -99,6 +99,7 @@ constexpr int kSegMaxPathLen = 16;        // ... all of one length, at most this
 constexpr int kKsSuper = 16;              // groups (warps) per super-group of the KS layout
 constexpr int kKsChunkRows = 8;           // rows per interleaving chunk of the KS layout
 constexpr int kSegSmallStep = 4;          // small regions are padded to 4, 8, 12 or 16 word rows
+constexpr uint32_t kPlanLast = 1u << 31;  // reduction plan: last contributor of an entry (SegmentedCorpus::pwords)
 
 struct SegString {                         // one string, compiled
     int status = 0;                        // 1 ok, 0 no accepting path, -1 needs another kernel
@@ -116,6 +117,12 @@ struct SegmentedCorpus {
     std::vector<int64_t> rgoff;                // [n_rgroups+1]
     std::vector<int32_t> rgrows;               // [n_rgroups]
     std::vector<double> typeW;                 // [n_rgroups*32] sum of p_s over the instances (0 = padding lane)
+    // reduction plan of the path-form groups (kr_paths): word r of lane l of group g at pgoff[g] + r*32 + l; a lane's
+    // stream is a list of entries, one word per contributing cell:  arc | (lane' << 3 | p) << 16 | kPlanLast on the
+    // entry's last word.  The kernel sums v[p] of lane' over an entry and issues one RED to `arc`.  Entries cover every
+    // non-padding cell of the group once; a stream ends in 0 words.  DAG groups have no plan (pgoff[g+1] == pgoff[g]).
+    std::vector<uint32_t> pwords;
+    std::vector<int64_t> pgoff;                // [n_rgroups+1]
     int64_t n_types = 0, n_region_instances = 0, n_region_edges = 0, n_type_edges = 0, max_big_rows = 0;
     // KS: strings in groups of 32 (one warp), longest first; string position kpos = g*32 + l.  kKsSuper groups
     // form a super-group (one CTA); its words are chunk-interleaved:

@@ -191,8 +191,8 @@ struct wfsa_dev {
     std::shared_ptr<SegmentedStringsJob> ks_job;
     std::unique_ptr<SegmentedCorpus> ks_sc;
     bool ks_failed = false;
-    DevBuf<uint32_t> d_krwords, d_kswords;
-    DevBuf<int64_t> d_krgoff, d_ksgoff;
+    DevBuf<uint32_t> d_krwords, d_krpwords, d_kswords;
+    DevBuf<int64_t> d_krgoff, d_krpgoff, d_ksgoff;
     DevBuf<int32_t> d_krgrows, d_ksgref, d_kssid, d_eoff, d_earc;
     DevBuf<double> d_krW, d_krlq, d_ksp, d_kslogq, d_seg_logaw;
     std::vector<double> h_p;
@@ -396,14 +396,15 @@ static bool seg_possible(const wfsa_dev* h, int K, int want_nt, int& nt, size_t&
     if (A.n_arcs <= 0 || A.n_arcs >= (1 << kLatArcBits)) return false;
     size_t tab = ((size_t)A.n_arcs + 1) * 8;
     const size_t max_smem = 227 * 1024 - 9216;     // + the zero weight of padding (kr_regions); k_eval6 has 7 KB of static shared memory, kr_regions up to 8
-    if (tab + (size_t)128 * K * 8 > max_smem) {
+    const int S = std::max(K, kPathSlots);          // pool slots per thread: K for the DAG form, at least kPathSlots (kr_paths)
+    if (tab + (size_t)128 * S * 8 > max_smem) {
         if (!awg) return false;
         *awg = true; tab = 0;
     }
-    nt = (int)((max_smem - tab) / ((size_t)K * 8) / 32) * 32;
+    nt = (int)((max_smem - tab) / ((size_t)S * 8) / 32) * 32;
     nt = std::min(nt, 1024);
     if (want_nt > 0) nt = std::min(nt, want_nt);
-    smem = tab + (size_t)nt * K * 8;
+    smem = tab + (size_t)nt * S * 8;
     return nt >= 128;
 }
 
@@ -454,7 +455,7 @@ static int setup_seg(wfsa_dev* h)
     h->awg = awg;
     if (want_nt == 512 || nt > 512 || awg) {   // k_eval6 is compiled for 512, 256 and 128 threads (AWG: 512), kr_regions for up to 512
         nt = awg ? 512 : (nt >= 512 ? 512 : (nt >= 256 ? 256 : 128));
-        smem = (awg ? 0 : ((size_t)h->larcs.n_arcs + 1) * 8) + (size_t)nt * K * 8;
+        smem = (awg ? 0 : ((size_t)h->larcs.n_arcs + 1) * 8) + (size_t)nt * std::max(K, kPathSlots) * 8;
     }
     h->seg_slots = K; h->seg_block = nt; h->seg_grid = h->sm_count; h->seg_smem = smem;
     // experiment / test knob: a smaller persistent grid, so that a small shard reaches the schedules of a large one (more big DAG
@@ -720,6 +721,7 @@ static void launch_main(wfsa_dev* h, int kernel, int mode, const CorpusD& C, con
         if (h->kr_groups > 0) {
             KRParams P{};
             P.aw = h->d_seg_aw.p; P.words = h->d_krwords.p; P.goff = h->d_krgoff.p; P.grows = h->d_krgrows.p; P.typeW = h->d_krW.p;
+            P.pwords = h->d_krpwords.p; P.pgoff = h->d_krpgoff.p;
             P.lq = h->d_krlq.p; P.n_groups = h->kr_groups; P.xs = h->d_seg_xs.p; P.xs_rows = (size_t)std::max<int64_t>(h->seg_max_big_rows, 1);
             P.counter = h->d_seg_counter.p; P.acc = h->d_seg_acc.p; P.fx_scale = O.fx_scale; P.n_arcs = h->larcs.n_arcs; P.replicas = h->replicas;
             P.ll_scale = O.ll_scale; P.red = O.red; P.llpart = h->d_llpart.p; P.n_llpart = h->llpart_n;
@@ -880,6 +882,7 @@ static void fill_eval6_params(wfsa_dev* h, Eval6Params& P)
 {
     P = Eval6Params{};
     P.words = h->d_krwords.p; P.goff = h->d_krgoff.p; P.grows = h->d_krgrows.p; P.typeW = h->d_krW.p; P.lq = h->d_krlq.p;
+    P.pwords = h->d_krpwords.p; P.pgoff = h->d_krpgoff.p;
     P.n_groups = h->kr_groups; P.n_big = h->kr_big_groups; P.cls = h->d_e6cls.p; P.n_cls = h->e6_ncls;
     // static share of the regular groups: 70 % measured best for the full corpus; none when CTAs are dedicated to their big
     // groups first (a CTA that starts late cannot give its static share away)
@@ -896,7 +899,7 @@ static void fill_eval6_params(wfsa_dev* h, Eval6Params& P)
     for (int r = 0; r < 8; ++r) P.peers[r] = (h->comm && r < h->nranks) ? h->peer_ptrs[r] : nullptr;
     P.stamps = h->d_e6stamps.p;
     P.debug = getenv("WFSA_E6_DEBUG") ? atoi(getenv("WFSA_E6_DEBUG")) : 0;
-    P.pool_slots = h->seg_slots; P.big_slots = h->e6_big_slots; P.big_rows = h->e6_big_rows;
+    P.pool_slots = std::max(h->seg_slots, kPathSlots); P.big_slots = h->e6_big_slots; P.big_rows = h->e6_big_rows;
     P.big_dedicate = eval6_big_dedicate(h);
     // dedicated CTAs: the shard is small (a few regular groups per warp): everything static among the free CTAs; one global
     // ticket counter for ~3.5 k groups costs ~3 ns per ticket in the L2, i.e. ~10 us of a ~14 us phase
@@ -1174,6 +1177,7 @@ extern "C" int wfsa_dev_set_param_map(wfsa_dev* h, const int32_t* trimmed, int32
         h->seg_max_big_rows = sc.max_big_rows;
         CK(h->d_krwords.upload(sc.rwords, h->stream)); CK(h->d_krgoff.upload(sc.rgoff, h->stream));
         CK(h->d_krgrows.upload(sc.rgrows, h->stream)); CK(h->d_krW.upload(sc.typeW, h->stream));
+        CK(h->d_krpwords.upload(sc.pwords, h->stream)); CK(h->d_krpgoff.upload(sc.pgoff, h->stream));
         CK(h->d_krlq.alloc((size_t)h->kr_groups * 32 + 1));
         CK(cudaMemsetAsync(h->d_krlq.p, 0, h->d_krlq.n * 8, h->stream));
         std::vector<unsigned long long> cacc(sc.const_acc.begin(), sc.const_acc.end());
@@ -2222,7 +2226,7 @@ extern "C" int wfsa_segmented_get(const wfsa_segmented* s, int which, const void
         SEG_ARR(0, c.rwords) SEG_ARR(1, c.rgoff) SEG_ARR(2, c.rgrows) SEG_ARR(3, c.typeW) SEG_ARR(4, c.swords) SEG_ARR(5, c.sgoff)
         SEG_ARR(6, c.sgref) SEG_ARR(7, c.ksid) SEG_ARR(8, c.kp) SEG_ARR(9, c.overflow) SEG_ARR(10, c.rejected) SEG_ARR(11, c.const_acc)
         SEG_ARR(12, s->stats) SEG_ARR(13, s->blocks.po) SEG_ARR(14, s->blocks.co) SEG_ARR(15, s->blocks.vo) SEG_ARR(16, s->blocks.cols)
-        SEG_ARR(17, s->blocks.counts) SEG_ARR(18, s->blocks.bp) SEG_ARR(19, s->blocks.slots)
+        SEG_ARR(17, s->blocks.counts) SEG_ARR(18, s->blocks.bp) SEG_ARR(19, s->blocks.slots) SEG_ARR(20, c.pwords) SEG_ARR(21, c.pgoff)
         default: return WFSA_ERR_INVALID;
     }
 #undef SEG_ARR

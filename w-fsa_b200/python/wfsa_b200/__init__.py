@@ -159,7 +159,8 @@ def lib():
 _SEG_ARRAYS = [("rwords", np.uint32), ("rgoff", np.int64), ("rgrows", np.int32), ("typeW", np.float64), ("swords", np.uint32),
                ("sgoff", np.int64), ("sgref", np.int32), ("ksid", np.int32), ("kp", np.float64), ("overflow", np.int32),
                ("rejected", np.int32), ("const_acc", np.int64), ("stats", np.int64), ("hb_path_off", np.int64), ("hb_col_off", np.int64), ("hb_val_off", np.int64),
-               ("hb_cols", np.int32), ("hb_counts", np.float64), ("hb_p", np.float64), ("hb_slot", np.int32)]
+               ("hb_cols", np.int32), ("hb_counts", np.float64), ("hb_p", np.float64), ("hb_slot", np.int32), ("pwords", np.uint32),
+               ("pgoff", np.int64)]
 
 
 def segmented_compile(lowered, trimmed=None, n_slots=16, fx_scale=1.0):

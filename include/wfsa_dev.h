@@ -130,6 +130,15 @@ typedef struct {
     const double*  p;            /* [n_blocks] p_s of the block's string                         */
 } wfsa_path_blocks;
 int wfsa_dev_set_path_blocks(wfsa_dev* h, const wfsa_path_blocks* blocks);
+/* rmin = the smallest path posterior over all strings of all ranks, min_s min_pi w(pi) / q_s (at most 1; 1 when no string
+ * has a choice).  Where it comes from:
+ *   - blocks set by wfsa_dev_set_path_blocks: from the blocks (Hf needs them on every kernel but the segmented one);
+ *   - no blocks, Hf == NULL, any kernel: no enumeration -- a forward sweep in the (min, +) semiring over the lattice of the
+ *     evaluation gives m_s = min_pi log w(pi), and r_s = exp(m_s - log q_s);
+ *   - segmented kernel (6) without blocks: blocks and per-string minima from the compiled region types, the overflow
+ *     strings by the sweep; when a region type has more than 2^20 paths an rmin-only call sweeps every string, a call
+ *     with Hf returns WFSA_ERR_LIMIT.
+ * Without blocks a call with Hf != NULL returns WFSA_ERR_STATE on the other kernels.  Collective with a communicator. */
 int wfsa_dev_hessian(wfsa_dev* h, const double* x, double* Hf /* n*n, or NULL: only rmin is computed */, double* rmin /* or NULL */);
 
 /* Multi-GPU: one handle per process/GPU; results of eval/structure/hessian are all-reduced as exact integer

@@ -23,7 +23,7 @@ constexpr int kRowCntBitsD = 8;
 constexpr int kRescaleEvery = 4;       // positions between exponent checks
 constexpr int kRescaleBand = 300;      // rescale when the largest entry leaves 2^(+-300)
 
-enum { MODE_EVAL = 0, MODE_STRUCT = 1 };
+enum { MODE_EVAL = 0, MODE_STRUCT = 1, MODE_MINPATH = 2 /* generic kernel: forward only, in (min, +) */ };
 enum { ACC_SMEM_CAS = 0, ACC_SMEM_SPLIT = 1, ACC_GLOBAL = 2, ACC_NONE = 3 /* timing experiments only */ };
 
 struct FastTablesD {
@@ -829,7 +829,7 @@ struct GenericTablesD {
 };
 struct GenericParams {
     GenericTablesD G;
-    const double* __restrict__ ltw;    // log transition weights
+    const double* __restrict__ ltw;    // log transition weights (MODE_MINPATH: +inf where absent)
     const double* __restrict__ lew;    // log emission weights
     CorpusD C;
     EvalOutD O;
@@ -847,9 +847,10 @@ __device__ __forceinline__ double logaddexp_d(double a, double b)
 }
 
 // semiring: MODE_EVAL = (logaddexp, +) on log-weights; MODE_STRUCT = (+, *) on path counts
-// (linear domain so that counts stay exact integers; every weight is 1)
-template <int MODE> __device__ __forceinline__ double sr_zero() { return MODE == MODE_STRUCT ? 0.0 : -INFINITY; }
-template <int MODE> __device__ __forceinline__ double sr_plus(double a, double b) { return MODE == MODE_STRUCT ? a + b : logaddexp_d(a, b); }
+// (linear domain so that counts stay exact integers; every weight is 1); MODE_MINPATH = (min, +) on log-weights whose
+// absent edges are +inf (k_minplus_weights), never -inf: the minimum would pick them
+template <int MODE> __device__ __forceinline__ double sr_zero() { return MODE == MODE_STRUCT ? 0.0 : (MODE == MODE_MINPATH ? INFINITY : -INFINITY); }
+template <int MODE> __device__ __forceinline__ double sr_plus(double a, double b) { return MODE == MODE_STRUCT ? a + b : (MODE == MODE_MINPATH ? fmin(a, b) : logaddexp_d(a, b)); }
 template <int MODE> __device__ __forceinline__ double sr_times(double a, double b) { return MODE == MODE_STRUCT ? a * b : a + b; }
 
 template <int MODE>
@@ -896,6 +897,10 @@ __global__ void __launch_bounds__(128) kg_fwdbwd(const GenericParams P)
                 }
             }
         }
+    }
+    if (MODE == MODE_MINPATH) {                  // lq = m_s, the smallest log weight of a path (+inf: none); no backward
+        P.O.logq[sid] = lq;
+        return;
     }
     if (MODE == MODE_STRUCT) {
         P.O.path_count[sid] = lq;
@@ -1174,7 +1179,7 @@ __global__ void __launch_bounds__(256) k5_hessian(const HessParams P)
     }
 }
 
-// rmin = exp(min over the strings of the summed log rmin of their regions); one CTA
+// rmin = exp(min over the strings of the summed log rmin of their regions, or of m_s - log q_s); one CTA
 __global__ void k_min_exp(long long n, const double* __restrict__ v, double* out)
 {
     __shared__ double s_m[32];

@@ -28,6 +28,7 @@
 #include "kernels_seg.cuh"
 #include "kernels_eval6.cuh"
 #include "kernels_k7.cuh"
+#include "kernels_rmin.cuh"
 #include "layout.hpp"
 #include "lattice.hpp"
 
@@ -220,8 +221,11 @@ struct wfsa_dev {
     std::vector<uint32_t> hrw; std::vector<int64_t> hrgoff; std::vector<int32_t> hrgrows; std::vector<double> hrW;
     std::vector<int32_t> h_ttp, h_etp;
     bool hb_from_types = false, hb_user = false;
+    bool hb_types_failed = false;              // the region types of this parameter map have too many paths for blocks
     DevBuf<int32_t> d_hb_slot; DevBuf<double> d_type_lrmin, d_zero_logaw;
     int hb_fx_log2 = 40;
+    // rmin without path blocks (rmin_sweep): per string m_s - log q_s, log q and (generic kernel) m_s, (min, +) weights, rmin
+    DevBuf<double> d_rterm, d_mlq, d_mpath, d_mtw, d_mew, d_msw, d_mfw, d_rsweep;
     // comm
     ncclComm_t comm = nullptr; int rank = 0, nranks = 1;
     // NVLink peer memory for the exchange inside k_eval6 (and the rank barrier of the benchmark); without it ncclAllReduce
@@ -543,6 +547,7 @@ static int choose_launch(wfsa_dev* h)
                 cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
             };
             prep(k7_fwd2<320, 4>); prep(k7_fwd2<512, 2>); prep(k7_bwd2<320, 3>); prep(k7_bwd2<512, 2>);
+            prep(k7_minfwd2<320, 4>); prep(k7_minfwd2<512, 2>);
         }
         rc = setup_k3(h);
         if (rc == WFSA_OK) rc = setup_k7_planes(h);
@@ -1120,10 +1125,9 @@ extern "C" int wfsa_dev_set_param_map(wfsa_dev* h, const int32_t* trimmed, int32
             tokens += len; max_len = std::max<int>(max_len, (int)len);
         }
     h->n_active = (int64_t)order.size(); h->n_active_w = (int64_t)order_w.size(); h->n_active_tokens = tokens;
-    if (h->kernel != 6) {
-        if (!order.empty()) CK(cudaMemcpyAsync(h->d_order.p, order.data(), order.size() * 4, cudaMemcpyHostToDevice, h->stream));
-        if (!order_w.empty()) CK(cudaMemcpyAsync(h->d_order_w.p, order_w.data(), order_w.size() * 4, cudaMemcpyHostToDevice, h->stream));
-    }
+    // (the segmented path reads the list of all its strings only in an rmin sweep without region-type blocks)
+    if (!order.empty()) CK(cudaMemcpyAsync(h->d_order.p, order.data(), order.size() * 4, cudaMemcpyHostToDevice, h->stream));
+    if (h->kernel != 6 && !order_w.empty()) CK(cudaMemcpyAsync(h->d_order_w.p, order_w.data(), order_w.size() * 4, cudaMemcpyHostToDevice, h->stream));
     if (h->kernel == 4) { const int rc = upload_transposed_tokens(h, order); if (rc != WFSA_OK) return rc; }
     // every logq defaults to -inf (unrecognised strings are never touched by an evaluation)
     {
@@ -1226,7 +1230,7 @@ extern "C" int wfsa_dev_set_param_map(wfsa_dev* h, const int32_t* trimmed, int32
         h->hrw = std::move(sc.rwords); h->hrgoff = std::move(sc.rgoff); h->hrgrows = std::move(sc.rgrows); h->hrW = std::move(sc.typeW);
         h->h_ttp = ttp; h->h_etp = etp;
         if (!h->hb_user) h->hb_blocks = -1;
-        h->hb_from_types = false;
+        h->hb_from_types = false; h->hb_types_failed = false;
     }
     if (h->kernel == 7) {
         // K7: batches of strings (longest first) whose alpha lattices fit the device memory; per batch and position the
@@ -1840,18 +1844,173 @@ static int build_type_blocks(wfsa_dev* h)
 
 static int ensure_ks(wfsa_dev* h);
 
+// rterm[s] = m_s - log q_s of the strings of one order list with fast tables (k3_minpath) or without (generic kernel:
+// a (min, +) forward, an evaluation for log q, k_rmin_terms)
+static void rmin_sweep_list(wfsa_dev* h, const int32_t* d_ord, int64_t n_ord)
+{
+    const HostFsa& F = h->fsa;
+    const FastLayout& L = h->fast;
+    cudaStream_t st = h->stream;
+    if (n_ord <= 0) return;
+    const CorpusD C{h->d_tokens.p, h->d_offs.p, h->d_p.p, d_ord, n_ord};
+    if (L.ok) {
+        K3MinParams P{};
+        P.T = FastTablesD{h->d_cand_off.p, h->d_slot_state.p, h->d_frow.p, h->d_fent.p, h->d_brow.p, h->d_bent.p,
+                          F.n_sym, F.n_states, L.n_arcs, L.n_slots, F.start, L.start_final_tid};
+        P.W = EvalWeightsD{h->d_tw.p, h->d_sw.p, h->d_fw.p};
+        P.mtw = h->d_mtw.p; P.msw = h->d_msw.p; P.mfw = h->d_mfw.p; P.C = C; P.rterm = h->d_rterm.p;
+        const int nt = std::max(64, (L.max_cand + 31) / 32 * 32);
+        const int grid = h->sm_count * std::max(1, std::min(4, 1024 / nt));
+        k3_minpath<<<grid, nt, (size_t)(4 * nt + 64) * 8 + 32 * 4, st>>>(P);
+        h->launches++;
+        return;
+    }
+    GenericParams P{};
+    P.G = GenericTablesD{h->d_emis_row.p, h->d_emis_tok_off.p, h->d_emis_tok.p, h->d_trans_row.p, h->d_trans_dst.p,
+                         h->d_eps_order.p, F.n_states, F.n_trans(), F.start, F.end};
+    P.C = C; P.scratch = h->d_gscratch.p; P.max_len = h->max_len;
+    P.O.red = h->d_red.p; P.O.fx_scale = std::ldexp(1.0, (int)h->fx_log2); P.O.ll_scale = std::ldexp(1.0, (int)h->ll_log2);
+    for (long long first = 0; first < n_ord; first += h->g_batch) {
+        P.first = first; P.count = std::min<long long>(h->g_batch, n_ord - first);
+        const int grid = (int)((P.count + 127) / 128);
+        P.ltw = h->d_mtw.p; P.lew = h->d_mew.p; P.O.logq = h->d_mpath.p;             // m_s
+        kg_fwdbwd<MODE_MINPATH><<<grid, 128, 0, st>>>(P);
+        P.ltw = h->d_ltw.p; P.lew = h->d_lew.p; P.O.logq = h->d_mlq.p;               // log q (its posteriors go to the scratch d_red)
+        kg_fwdbwd<MODE_EVAL><<<grid, 128, 0, st>>>(P);
+        h->launches += 2;
+    }
+    k_rmin_terms<<<(unsigned)((n_ord + 255) / 256), 256, 0, st>>>(n_ord, d_ord, h->d_mpath.p, h->d_mlq.p, h->d_rterm.p);
+    h->launches++;
+}
+
+// The smallest path posterior without enumerating paths: r_s = exp(m_s - log q_s), m_s the smallest log weight of a path
+// of s, by a forward sweep in (min, +) over the lattice of the evaluation; rmin = min_s r_s (1 when no string has a choice).
+// `all`: every active string (else, on the segmented path, its overflow strings only).  x is on the device; d_rsweep
+// receives rmin.
+static int rmin_sweep(wfsa_dev* h, bool all)
+{
+    const HostFsa& F = h->fsa;
+    const FastLayout& L = h->fast;
+    cudaStream_t st = h->stream;
+    const size_t ns = (size_t)std::max<int64_t>(h->n_strings, 1);
+    if (h->d_rterm.n < ns) {
+        CK(h->d_rterm.alloc(ns)); CK(h->d_mlq.alloc(ns)); CK(h->d_rsweep.alloc(1));
+        if (!L.ok) CK(h->d_mpath.alloc(ns));
+        CK(h->d_mtw.alloc(std::max(F.n_trans(), 1))); CK(h->d_mew.alloc(std::max(F.n_emis(), 1)));
+        CK(h->d_msw.alloc(std::max(L.ok ? L.n_slots : 0, 1))); CK(h->d_mfw.alloc(std::max(L.ok ? L.n_slots : 0, 1)));
+    }
+    CK(cudaMemsetAsync(h->d_rterm.p, 0, ns * 8, st));
+    const int n_slots = L.ok ? L.n_slots : 0;
+    const int total = F.n_trans() + F.n_emis() + n_slots;
+    if (total > 0) {
+        k_weights<<<(total + 255) / 256, 256, 0, st>>>(F.n_trans(), F.n_emis(), n_slots, h->d_trans_tp.p, h->d_emis_tp.p,
+                                                      h->d_slot_emis.p, h->d_slot_final.p, h->d_x.p, 0, h->d_tw.p,
+                                                      h->d_sw.p, h->d_fw.p, h->d_ltw.p, h->d_lew.p);
+        k_minplus_weights<<<(total + 255) / 256, 256, 0, st>>>(F.n_trans(), F.n_emis(), n_slots, h->d_trans_tp.p, h->d_emis_tp.p,
+                                                              h->d_slot_emis.p, h->d_slot_final.p, h->d_x.p, h->d_mtw.p,
+                                                              h->d_mew.p, h->d_msw.p, h->d_mfw.p);
+        h->launches += 2;
+    }
+    if (h->kernel == 6) {
+        if (all) rmin_sweep_list(h, h->d_order.p, h->n_active + h->n_active_w);
+        else rmin_sweep_list(h, h->d_order_w.p, h->n_active_w);
+    } else if (h->kernel == 7 && h->k7_planes) {
+        // K7's batches: the forward sweep of the evaluation (k7_fwd2, k7_finish_q) for log q, beside it the (min, +)
+        // sweep (k7_minfwd2) in the two rows of the backward sweep, k7_finish_min where strings end; strings with unknown
+        // symbols on the CTA-per-string kernel, as in the evaluation
+        FastTablesD T{};
+        T.cand_off = h->d_cand_off.p; T.slot_state = h->d_slot_state.p;
+        T.frow = h->d_frow.p; T.fent = h->d_fent.p; T.brow = h->d_brow.p; T.bent = h->d_bent.p;
+        T.n_sym = F.n_sym; T.n_states = F.n_states; T.n_arcs = L.n_arcs; T.n_slots = L.n_slots;
+        T.start_state = F.start; T.start_final_tid = L.start_final_tid;
+        const EvalWeightsD Wt{h->d_tw.p, h->d_sw.p, h->d_fw.p};
+        EvalOutD O{};
+        O.logq = h->d_mlq.p; O.red = h->d_red.p; O.ll_scale = std::ldexp(1.0, (int)h->ll_log2);   // (loglik goes to the scratch d_red)
+        const int V = h->k7_V;
+        const size_t smem = (size_t)kK7Chunk * V * 8;
+        double* const lat = h->d_k7lat.p;
+        double* const mu[2] = {h->d_k7bt.p, h->d_k7bt.p + h->k7_nb * (size_t)V};
+        for (auto& B : h->k7) {
+            K7FinParams Fn{};
+            Fn.T = T; Fn.W = Wt; Fn.O = O; Fn.sid = B.d_sid.p; Fn.last_tok = B.d_last.p; Fn.p = h->d_p.p;
+            Fn.scale = h->d_k7scale.p; Fn.EQ = h->d_k7EQ.p; Fn.F = h->d_k7F.p; Fn.V = V;
+            K7Params P{};
+            P.T = T; P.W = Wt; P.O = O; P.V = V; P.pe = h->d_k7pef.p; P.pr = h->d_k7prf.p;
+            K7MinParams M{};
+            M.T = T; M.mtw = h->d_mtw.p; M.msw = h->d_msw.p; M.pe = h->d_k7pef.p; M.pr = h->d_k7prf.p; M.V = V;
+            K7MinFinParams Mf{};
+            Mf.T = T; Mf.sid = B.d_sid.p; Mf.last_tok = B.d_last.p; Mf.mfw = h->d_mfw.p; Mf.logq = h->d_mlq.p; Mf.rterm = h->d_rterm.p; Mf.V = V;
+            for (int t = 0; t < B.Tmax; ++t) {
+                P.desc = M.desc = B.d_desc.p + B.desc_off[t]; P.perm = M.perm = B.d_perm.p + B.row_off[t];
+                P.src = t ? lat + B.row_off[t - 1] * V : nullptr; P.dst = lat + B.row_off[t] * V;
+                P.exp_src = t ? h->d_k7exp.p + B.row_off[t - 1] : nullptr; P.exp_dst = h->d_k7exp.p + B.row_off[t];
+                P.rescale = (t & (kRescaleEvery - 1)) == kRescaleEvery - 1;
+                M.src = t ? mu[(t - 1) & 1] : nullptr; M.dst = mu[t & 1];
+                const unsigned nd = (unsigned)(B.desc_off[t + 1] - B.desc_off[t]);
+                if (nd) {
+                    if (V <= 320) { k7_fwd2<320, 4><<<nd, V, smem, st>>>(P); k7_minfwd2<320, 4><<<nd, V, smem, st>>>(M); }
+                    else { k7_fwd2<512, 2><<<nd, V, smem, st>>>(P); k7_minfwd2<512, 2><<<nd, V, smem, st>>>(M); }
+                    h->launches += 2;
+                }
+                if (B.n_t[t + 1] < B.n_t[t]) {
+                    Fn.r0 = Mf.r0 = B.n_t[t + 1]; Fn.r1 = Mf.r1 = B.n_t[t];
+                    Fn.lat = lat + B.row_off[t] * V; Fn.exp_t = h->d_k7exp.p + B.row_off[t]; Mf.mu = mu[t & 1];
+                    k7_finish_q<<<(Fn.r1 - Fn.r0 + 7) / 8, 256, 0, st>>>(Fn);
+                    k7_finish_min<<<(Mf.r1 - Mf.r0 + 7) / 8, 256, 0, st>>>(Mf);
+                    h->launches += 2;
+                }
+            }
+        }
+        rmin_sweep_list(h, h->d_order_w.p, h->n_active_w);
+    } else if (h->kernel == 7) {
+        rmin_sweep_list(h, h->d_order.p, h->n_active + h->n_active_w);    // without pair planes: every string on k3_minpath
+    } else {
+        rmin_sweep_list(h, h->d_order.p, h->n_active);
+        rmin_sweep_list(h, h->d_order_w.p, h->n_active_w);                  // (kernel 4: strings beyond its active sets)
+    }
+    if (h->n_strings) {
+        k_min_exp<<<1, 1024, 0, st>>>((long long)h->n_strings, h->d_rterm.p, h->d_rsweep.p);
+        h->launches++;
+    } else {
+        const double one = 1.0;
+        CK(cudaMemcpyAsync(h->d_rsweep.p, &one, 8, cudaMemcpyHostToDevice, st));
+    }
+    CK(cudaGetLastError());
+    return WFSA_OK;
+}
+
 extern "C" int wfsa_dev_hessian(wfsa_dev* h, const double* x, double* Hf, double* rmin)
 {
     if (!h || (!Hf && !rmin)) return set_err(h, WFSA_ERR_INVALID, "hessian: bad arguments");
     if (h->n < 0) return set_err(h, WFSA_ERR_STATE, "hessian before set_param_map");
+    // rmin only, without path blocks: the (min, +) sweep over every active string, on every kernel (the segmented path
+    // when its region types have too many paths for blocks)
+    bool sweep_all = false;
     if (h->hb_blocks < 0) {
-        if (h->kernel != 6) return set_err(h, WFSA_ERR_STATE, "hessian before set_path_blocks");
-        CK(cudaSetDevice(h->device));
-        const int rc = build_type_blocks(h);              // the segmented path derives the blocks from its region types
-        if (rc != WFSA_OK) return rc;
+        if (h->kernel != 6) {
+            if (Hf) return set_err(h, WFSA_ERR_STATE, "hessian before set_path_blocks");
+            sweep_all = true;
+        } else if (Hf || !h->hb_types_failed) {
+            CK(cudaSetDevice(h->device));
+            const int rc = build_type_blocks(h);          // the segmented path derives the blocks from its region types
+            if (rc == WFSA_ERR_LIMIT) h->hb_types_failed = true;
+            if (rc == WFSA_ERR_LIMIT && !Hf) sweep_all = true;
+            else if (rc != WFSA_OK) return rc;
+        } else sweep_all = true;
     }
     int rc = wfsa_dev_upload_x(h, x);
     if (rc != WFSA_OK) return rc;
+    if (sweep_all) {
+        rc = rmin_sweep(h, true);
+        if (rc != WFSA_OK) return rc;
+        double rm = 1.0;
+        CK(cudaMemcpyAsync(&rm, h->d_rsweep.p, 8, cudaMemcpyDeviceToHost, h->stream));
+        CK(cudaStreamSynchronize(h->stream));
+        CK(cudaGetLastError());
+        if (h->comm) { rm = -rm; const int r2 = wfsa_dev_allreduce_f64(h, &rm, 1, 1); if (r2 != WFSA_OK) return r2; rm = -rm; }
+        *rmin = rm;
+        return WFSA_OK;
+    }
     const size_t nn = Hf ? (size_t)h->n * h->n : 0;          // Hf == NULL: only rmin is wanted, nothing of H is touched
     if (Hf) CK(cudaMemsetAsync(h->d_Hfx.p, 0, std::max<size_t>(nn, 1) * 8, h->stream));
     const double inf = INFINITY;
@@ -1894,9 +2053,15 @@ extern "C" int wfsa_dev_hessian(wfsa_dev* h, const double* x, double* Hf, double
             h->ks_done = false;                           // the per-string buffer no longer holds log q
         }
     }
+    // the overflow strings of the segmented path are not in the per-string layout: the (min, +) sweep of the secondary kernel
+    const bool overflow_sweep = rmin && h->hb_from_types && h->n_active_w > 0;
+    if (overflow_sweep) { rc = rmin_sweep(h, false); if (rc != WFSA_OK) return rc; }
     CK(cudaMemcpyAsync(&rm, h->d_rmin.p, 8, cudaMemcpyDeviceToHost, h->stream));
+    double rm_w = INFINITY;
+    if (overflow_sweep) CK(cudaMemcpyAsync(&rm_w, h->d_rsweep.p, 8, cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     CK(cudaGetLastError());
+    rm = std::min(rm, rm_w);
     if (rmin) {
         if (h->comm) { rm = -rm; const int r2 = wfsa_dev_allreduce_f64(h, &rm, 1, 1); if (r2 != WFSA_OK) return r2; rm = -rm; }
         *rmin = rm;

@@ -430,17 +430,12 @@ bool QuasiNewtonLearner::HaltCondition(double tol)
 }
 
 // smallest path posterior over all strings at the current x (the rmin column of both optimisers): the H_f entry point of the
-// backend without its matrix
+// backend without its matrix, which needs no path enumeration on any kernel
 double Learner::ComputeRmin()
 {
     if (HasUniquePaths()) return 0.0;
     double rm = 0.0;
-    int rc = wfsa_dev_hessian(dev, _x.data(), nullptr, &rm);
-    if (rc == WFSA_ERR_STATE && !have_blocks) {
-        BuildPathBlocks();
-        rc = wfsa_dev_hessian(dev, _x.data(), nullptr, &rm);
-    }
-    check(rc, "wfsa_dev_hessian");
+    check(wfsa_dev_hessian(dev, _x.data(), nullptr, &rm), "wfsa_dev_hessian");
     return std::isfinite(rm) ? rm : 1.0;
 }
 

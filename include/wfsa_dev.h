@@ -138,8 +138,26 @@ int wfsa_dev_set_path_blocks(wfsa_dev* h, const wfsa_path_blocks* blocks);
  *   - segmented kernel (6) without blocks: blocks and per-string minima from the compiled region types, the overflow
  *     strings by the sweep; when a region type has more than 2^20 paths an rmin-only call sweeps every string, a call
  *     with Hf returns WFSA_ERR_LIMIT.
- * Without blocks a call with Hf != NULL returns WFSA_ERR_STATE on the other kernels.  Collective with a communicator. */
+ * Without blocks a call with Hf != NULL returns WFSA_ERR_STATE on the other kernels.  Collective with a communicator.
+ * The (min, +) sweep gives the weight of the least probable path; the most probable path itself, of every string, comes
+ * from wfsa_dev_viterbi below. */
 int wfsa_dev_hessian(wfsa_dev* h, const double* x, double* Hf /* n*n, or NULL: only rmin is computed */, double* rmin /* or NULL */);
+
+/* Most probable accepting path of every string of this shard (Viterbi), at x (trimmed parameters, as wfsa_dev_eval):
+ *   logw[s] = max over accepting paths pi of s of the summed log weights of pi's edges  (-inf: no accepting path under
+ *             the parameter map and x, or the string does not take part in evaluations);
+ *   path_off[s]..path_off[s+1]: the steps of that path (path_off: n_strings + 1 entries; 0 steps when logw[s] = -inf).
+ * logw[s] is the left-to-right sum of the log weights of the steps (transition, then emission, ..., final transition), bit
+ * for bit.  Ties are broken deterministically (same bits on every call).  The paths stay on the device until the next
+ * wfsa_dev_viterbi or wfsa_dev_destroy.  Local to the shard: no collective, also with a communicator attached.  The call
+ * keeps its own copy of x: it changes nothing an evaluation returns, also between wfsa_dev_eval_launch and
+ * wfsa_dev_eval_fetch.  WFSA_ERR_STATE before wfsa_dev_set_param_map. */
+int wfsa_dev_viterbi(wfsa_dev* h, const double* x, double* logw, int64_t* path_off);
+/* Steps of the last wfsa_dev_viterbi, path_off[n_strings] of each, in string order:
+ * trans_edge = index of the transition edge in the descriptor (trans_dst order); emis_edge = index of the emission edge
+ * of its target state (emis_tok_off order), -1 for the final transition into the end state.  WFSA_ERR_STATE before any
+ * wfsa_dev_viterbi. */
+int wfsa_dev_viterbi_paths(wfsa_dev* h, int32_t* trans_edge, int32_t* emis_edge);
 
 /* Multi-GPU: one handle per process/GPU; results of eval/structure/hessian are all-reduced as exact integer
  * sums, so every rank holds the same bits (the evaluation through an all-reduce over NVLink peer memory fused

@@ -23,7 +23,8 @@ constexpr int kRowCntBitsD = 8;
 constexpr int kRescaleEvery = 4;       // positions between exponent checks
 constexpr int kRescaleBand = 300;      // rescale when the largest entry leaves 2^(+-300)
 
-enum { MODE_EVAL = 0, MODE_STRUCT = 1, MODE_MINPATH = 2 /* generic kernel: forward only, in (min, +) */ };
+enum { MODE_EVAL = 0, MODE_STRUCT = 1, MODE_MINPATH = 2 /* generic kernel: forward only, in (min, +) */,
+       MODE_VITERBI = 3 /* generic kernel: forward in (max, +) with backpointers, traceback */ };
 enum { ACC_SMEM_CAS = 0, ACC_SMEM_SPLIT = 1, ACC_GLOBAL = 2, ACC_NONE = 3 /* timing experiments only */ };
 
 struct FastTablesD {
@@ -836,6 +837,12 @@ struct GenericParams {
     double* scratch;                   // [n_threads][2][(max_len+1)*n_states]
     int max_len;
     long long first, count;            // slice of C.order handled by this launch
+    // MODE_VITERBI: without vit_off the step count of every string goes to vit_cnt; with vit_off ([n_strings+1] step
+    // offsets) the steps go to vit_trans / vit_emis
+    int32_t* vit_cnt;
+    const int64_t* vit_off;
+    int32_t* vit_trans;
+    int32_t* vit_emis;
 };
 
 __device__ __forceinline__ double logaddexp_d(double a, double b)
@@ -872,6 +879,7 @@ __global__ void __launch_bounds__(128) kg_fwdbwd(const GenericParams P)
     for (size_t k = 0; k < (size_t)(len + 1) * S; ++k) { la[k] = ZERO; lb[k] = ZERO; }
     la[G.start_state] = (MODE == MODE_STRUCT) ? 1.0 : 0.0;
     double lq = ZERO;
+    int fin_t = -1, fin_u = -1;                  // MODE_VITERBI: the winning transition into the end state
     // forward
     for (int pos = 0; pos <= len; ++pos) {
         for (int oi = 0; oi < S; ++oi) {
@@ -883,7 +891,8 @@ __global__ void __launch_bounds__(128) kg_fwdbwd(const GenericParams P)
                 const double w = (MODE == MODE_STRUCT) ? au : au + P.ltw[t];
                 if (w == ZERO) continue;
                 if (v == G.end_state) {
-                    if (pos == len) lq = sr_plus<MODE>(lq, w);
+                    if (MODE == MODE_VITERBI) { if (pos == len && w > lq) { lq = w; fin_t = t; fin_u = u; } }
+                    else if (pos == len) lq = sr_plus<MODE>(lq, w);
                     continue;
                 }
                 for (int e = G.emis_row[v]; e < G.emis_row[v + 1]; ++e) {
@@ -893,13 +902,39 @@ __global__ void __launch_bounds__(128) kg_fwdbwd(const GenericParams P)
                     for (int k = 0; k < el; ++k) if (tok[pos + k] != G.emis_tok[e0 + k]) { m = false; break; }
                     if (!m) continue;
                     double* dst = la + (size_t)(pos + el) * S + v;
-                    *dst = sr_plus<MODE>(*dst, (MODE == MODE_STRUCT) ? w : w + P.lew[e]);
+                    if (MODE == MODE_VITERBI) {          // the first strictly larger candidate wins; backpointer (t, e)
+                        const double val = w + P.lew[e];
+                        if (val > *dst) {
+                            *dst = val;
+                            reinterpret_cast<unsigned long long*>(lb)[(size_t)(pos + el) * S + v] = ((unsigned long long)t << 32) | (unsigned)e;
+                        }
+                    } else *dst = sr_plus<MODE>(*dst, (MODE == MODE_STRUCT) ? w : w + P.lew[e]);
                 }
             }
         }
     }
     if (MODE == MODE_MINPATH) {                  // lq = m_s, the smallest log weight of a path (+inf: none); no backward
         P.O.logq[sid] = lq;
+        return;
+    }
+    if (MODE == MODE_VITERBI) {                  // lq = the largest log weight of a path (-inf: none); traceback, no backward
+        P.O.logq[sid] = lq;
+        const bool found = lq > -INFINITY;
+        const unsigned long long* bp = reinterpret_cast<const unsigned long long*>(lb);
+        int64_t o = found && P.vit_off ? P.vit_off[sid + 1] - 1 : 0;
+        if (found && P.vit_off) { P.vit_trans[o] = fin_t; P.vit_emis[o] = -1; }
+        int n = found ? 1 : 0, p = len, v = fin_u;
+        while (found && v != G.start_state) {
+            const unsigned long long b = bp[(size_t)p * S + v];
+            const int t = (int)(b >> 32), e = (int)(unsigned)b;
+            if (P.vit_off) { --o; P.vit_trans[o] = t; P.vit_emis[o] = e; }
+            p -= G.emis_tok_off[e + 1] - G.emis_tok_off[e];
+            int lo = 0, hi = S;                  // source state of t: the last state whose transitions start at or before t
+            while (hi - lo > 1) { const int mid = (lo + hi) >> 1; if (G.trans_row[mid] <= t) lo = mid; else hi = mid; }
+            v = lo;
+            ++n;
+        }
+        if (!P.vit_off) P.vit_cnt[sid] = n;
         return;
     }
     if (MODE == MODE_STRUCT) {

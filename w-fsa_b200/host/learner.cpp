@@ -235,6 +235,19 @@ const std::vector<double>& Learner::LogQ()
     return logq_cache;
 }
 
+void Learner::Decode(Decoding& d)
+{
+    const size_t ns = shard_words.size();
+    d.logw.assign(std::max<size_t>(ns, 1), 0.0); d.logq.assign(std::max<size_t>(ns, 1), 0.0); d.path_off.assign(ns + 1, 0);
+    double ll = 0.0;
+    std::vector<double> g(std::max(GetNumberOfParameters(), 1));
+    check(wfsa_dev_eval(dev, _x.data(), &ll, d.logq.data(), g.data()), "wfsa_dev_eval");
+    check(wfsa_dev_viterbi(dev, _x.data(), d.logw.data(), d.path_off.data()), "wfsa_dev_viterbi");
+    d.trans_edge.assign(std::max<int64_t>(d.path_off[ns], 1), 0); d.emis_edge.assign(d.trans_edge.size(), 0);
+    check(wfsa_dev_viterbi_paths(dev, d.trans_edge.data(), d.emis_edge.data()), "wfsa_dev_viterbi_paths");
+    d.logw.resize(ns); d.logq.resize(ns); d.trans_edge.resize(d.path_off[ns]); d.emis_edge.resize(d.path_off[ns]);
+}
+
 // ---------------------------------------------------------------------------------------------
 // Route A of SURVEY.md section 7: enumerate the paths of AMBIGUOUS strings only (structure,
 // once), ship dense count blocks; the numeric contraction runs on the device.

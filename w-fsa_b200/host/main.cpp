@@ -6,6 +6,7 @@
 // backend has no P/M matrices to cache.  -r only orders the -p/-pr path listing (BFS/DFS).  Added: --device N, --full (dump weights with 17 digits),
 // --gpus N: one process per GPU (forked before anything touches CUDA), corpus cut into N ranges of equal symbol count, the
 // same optimiser loop on every rank with loglik / gradient / H_f summed over the ranks inside the backend; rank 0 reports.
+// --viterbi FILE: the most probable path of every corpus string with the final weights (write_viterbi).
 #include <cfloat>
 #include <cmath>
 #include <cstdio>
@@ -77,6 +78,43 @@ static void print_paths(const Fsa& fsa, const Corpus& corpus, bool bfs)
     }
 }
 
+// --viterbi FILE: one line per corpus string, in corpus order,  word TAB ln w(pi) TAB w(pi)/q_s TAB path,  pi the most
+// probable path of the word (wfsa_dev_viterbi), the path in the format of -p without its "text: " prefix; "-inf", 0 and an
+// empty path for a word without a path.
+static void write_viterbi(const std::string& filename, const Fsa& fsa, const Corpus& corpus, Learner& learner)
+{
+    Learner::Decoding d;
+    learner.Decode(d);
+    FILE* out = fopen(filename.c_str(), "w");
+    if (!out) throw MyError("Unable to open output file \"" + filename + "\" for writing!");
+    const auto& st = fsa.States();
+    const LoweredFsa& L = learner.Lowered();
+    std::string line;
+    for (size_t s = 0; s < corpus.size(); ++s) {
+        line = corpus[s].first;
+        if (!(d.logw[s] > -INFINITY)) {
+            line += "\t-inf\t0\t\n";
+        } else {
+            char num[64];
+            snprintf(num, sizeof num, "\t%.17g", d.logw[s]); line += num;
+            snprintf(num, sizeof num, "\t%.17g\t", std::exp(d.logw[s] - d.logq[s])); line += num;
+            line += fsa.GetStartState();
+            for (int64_t k = d.path_off[s]; k < d.path_off[s + 1]; ++k) {
+                const auto& te = L.trans_edge[d.trans_edge[k]];
+                line += " -> " + st[st[te.first].transitions[te.second].next].name;
+                if (d.emis_edge[k] >= 0) {
+                    const auto& ee = L.emis_edge[d.emis_edge[k]];
+                    const std::string& e = st[ee.first].emissions[ee.second].str;
+                    if (!e.empty()) line += '"' + e + '"';
+                }
+            }
+            line += '\n';
+        }
+        fwrite(line.data(), 1, line.size(), out);
+    }
+    if (fclose(out) != 0) throw MyError("Unable to write \"" + filename + "\"!");
+}
+
 // --gpus: the ranks meet in collectives (communicator set-up, all-reduces).  A rank that dies would leave the others waiting
 // there for ever, so rank 0 ends the whole run as soon as a child ends with an error, and the children end with their parent.
 static volatile sig_atomic_t g_children_left = 0;
@@ -118,12 +156,15 @@ static void usage()
         "                             16 reorder (no-op: dense solve), 32 exponential multipliers\n"
         "  --device N                 CUDA device ordinal (0); with --gpus the first of N consecutive devices\n"
         "  --gpus N                   shard the corpus over N GPUs of this node (one process per GPU, 1)\n"
-        "  --full                     dump weights with 17 significant digits\n";
+        "  --full                     dump weights with 17 significant digits\n"
+        "  --viterbi FILE             after the optimization, write the most probable path of every corpus string with the\n"
+        "                             final weights (after -n) to FILE: word, ln w(path), w(path)/q(word), path (one GPU);\n"
+        "                             -e 0 -s decodes with the automaton file's own weights\n";
 }
 
 int main(int argc, const char* argv[])
 {
-    std::string automaton_filename, corpus_filename, output_filename, optimizer = "Hessian";
+    std::string automaton_filename, corpus_filename, output_filename, viterbi_filename, optimizer = "Hessian";
     int epochs = 20, initflags = 0, device = 0, gpus = 1;
     bool normalize = false, print = false, print_recognize = false, suppress = false, evaluate = false, initx = false, full = false;
     int recognize = 0;
@@ -158,8 +199,13 @@ int main(int argc, const char* argv[])
         else if (is(a, {"--device"})) device = atoi(next());
         else if (is(a, {"--gpus"})) { gpus = atoi(next()); if (gpus < 1 || gpus > 8) { std::cerr << "--gpus must be between 1 and 8" << std::endl; return 1; } }
         else if (is(a, {"--full"})) full = true;
+        else if (is(a, {"--viterbi"})) viterbi_filename = next();
         else if (is(a, {"-m", "--matrices", "--matrix"})) { next(); std::cerr << "-m is not supported: the DP backend has no path matrices to cache" << std::endl; return 1; }
         else { std::cerr << "Unknown argument \"" << a << "\"!" << std::endl; return 1; }
+    }
+    if (!viterbi_filename.empty() && gpus > 1) {
+        std::cerr << "--viterbi decodes on one GPU: it cannot be combined with --gpus " << gpus << std::endl;
+        return 1;
     }
     // --gpus N: fork the other ranks before CUDA is touched.  Rank 0 (this process) creates the communicator id and hands
     // it to every child through a pipe; the children run the same program with their output discarded (their errors still
@@ -282,6 +328,7 @@ int main(int argc, const char* argv[])
             for (double x : results) std::cerr << ' ' << x;
             std::cerr << std::endl;
         }
+        if (!viterbi_filename.empty()) write_viterbi(viterbi_filename, fsa, corpus, *learner);
         if (!suppress && rank == 0) {
             FILE* outf = output_filename.empty() ? stdout : fopen(output_filename.c_str(), "w");
             if (!outf) throw MyError("Unable to open output file \"" + output_filename + "\" for writing!");

@@ -18,6 +18,7 @@ UNIQUE_ID_BYTES = 128
 DEV_SYMBOLS = [
     "wfsa_dev_create", "wfsa_dev_structure", "wfsa_dev_set_param_map", "wfsa_dev_eval", "wfsa_dev_upload_x",
     "wfsa_dev_eval_launch", "wfsa_dev_eval_fetch", "wfsa_dev_sync", "wfsa_dev_set_path_blocks", "wfsa_dev_hessian",
+    "wfsa_dev_viterbi", "wfsa_dev_viterbi_paths",
     "wfsa_dev_comm_unique_id", "wfsa_dev_comm_init", "wfsa_dev_allreduce_f64", "wfsa_dev_timer_begin", "wfsa_dev_timer_begin_steps",
     "wfsa_dev_timer_end", "wfsa_dev_timer_kernel_ms", "wfsa_dev_timer_split_ms", "wfsa_dev_timer_step_ms", "wfsa_dev_timer_phase_ms", "wfsa_dev_eval6_phases", "wfsa_dev_l2_flush", "wfsa_dev_rank_barrier", "wfsa_dev_get_info", "wfsa_dev_destroy", "wfsa_dev_held_bytes", "wfsa_dev_last_error",
     "wfsa_dev_version", "wfsa_lattice_compile", "wfsa_segmented_compile", "wfsa_segmented_get",
@@ -132,6 +133,8 @@ def lib():
         L.wfsa_dev_sync.argtypes = [C.c_void_p]
         L.wfsa_dev_set_path_blocks.argtypes = [C.c_void_p, C.POINTER(PathBlocks)]
         L.wfsa_dev_hessian.argtypes = [C.c_void_p, F64P, F64P, F64P]
+        L.wfsa_dev_viterbi.argtypes = [C.c_void_p, F64P, F64P, I64P]
+        L.wfsa_dev_viterbi_paths.argtypes = [C.c_void_p, I32P, I32P]
         L.wfsa_dev_comm_unique_id.argtypes = [C.c_void_p]
         L.wfsa_dev_comm_init.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int]
         L.wfsa_dev_allreduce_f64.argtypes = [C.c_void_p, F64P, C.c_int, C.c_int]
@@ -367,6 +370,11 @@ class Device:
             return ll.value, logq[:self.n_strings], grad[:self.n]
         return ll.value, grad[:self.n]
 
+    def viterbi(self, x):
+        """Most probable path of every string at x: (logw, path_off, trans_edge, emis_edge); the steps of string s are
+        [path_off[s], path_off[s+1]) (descriptor edge ids; emis_edge -1 on the final transition), logw[s] = -inf: none."""
+        return _viterbi(self.L, self.h, x, self.n_strings)
+
     def timer_begin(self):
         self._ck(self.L.wfsa_dev_timer_begin(self.h))
 
@@ -431,6 +439,21 @@ class Device:
             self.close()
         except Exception:
             pass
+
+
+def _viterbi(L, h, x, n_strings):
+    def ck(rc):
+        if rc != 0:
+            raise WfsaError(rc, L.wfsa_dev_last_error(h).decode())
+    x = np.ascontiguousarray(x, dtype=np.float64)
+    logw = np.zeros(max(n_strings, 1))
+    off = np.zeros(n_strings + 1, dtype=np.int64)
+    ck(L.wfsa_dev_viterbi(h, _p(x, F64P), _p(logw, F64P), _p(off, I64P)))
+    steps = max(int(off[-1]), 1)
+    tr = np.zeros(steps, dtype=np.int32)
+    em = np.zeros(steps, dtype=np.int32)
+    ck(L.wfsa_dev_viterbi_paths(h, _p(tr, I32P), _p(em, I32P)))
+    return logw[:n_strings], off, tr[:off[-1]], em[:off[-1]]
 
 
 class Session:
@@ -505,6 +528,10 @@ class Session:
 
     def dump(self, full_precision=True):
         return self.L.wfsa_session_dump(self.h, 1 if full_precision else 0).decode("latin-1")
+
+    def viterbi(self, x=None):
+        """Device.viterbi on the session's backend, at x or the current weights, for every string of this shard."""
+        return _viterbi(self.L, self.L.wfsa_session_backend(self.h), self.x() if x is None else x, self.backend_info()["n_strings"])
 
     def backend_info(self):
         i = DevInfo()

@@ -149,14 +149,30 @@ int wfsa_dev_hessian(wfsa_dev* h, const double* x, double* Hf /* n*n, or NULL: o
  *   path_off[s]..path_off[s+1]: the steps of that path (path_off: n_strings + 1 entries; 0 steps when logw[s] = -inf).
  * logw[s] is the left-to-right sum of the log weights of the steps (transition, then emission, ..., final transition), bit
  * for bit.  Ties are broken deterministically (same bits on every call).  The paths stay on the device until the next
- * wfsa_dev_viterbi or wfsa_dev_destroy.  Local to the shard: no collective, also with a communicator attached.  The call
+ * wfsa_dev_viterbi, wfsa_dev_nbest or wfsa_dev_destroy.  Local to the shard: no collective, also with a communicator attached.  The call
  * keeps its own copy of x: it changes nothing an evaluation returns, also between wfsa_dev_eval_launch and
  * wfsa_dev_eval_fetch.  WFSA_ERR_STATE before wfsa_dev_set_param_map. */
 int wfsa_dev_viterbi(wfsa_dev* h, const double* x, double* logw, int64_t* path_off);
-/* Steps of the last wfsa_dev_viterbi, path_off[n_strings] of each, in string order:
+/* The k most probable accepting paths of every string of this shard (N-best), 1 <= k <= 16, at x; path i = s * k + r is the
+ * r-th most probable path of string s (r = 0: the best):
+ *   logw[i] = summed log weight of that path (-inf, and 0 steps, when s has at most r paths, or none under the parameter
+ *             map and x, or does not take part in evaluations); non-increasing in r;
+ *   path_off[i]..path_off[i+1]: its steps (path_off: n_strings * k + 1 entries).
+ * The k paths of a string are pairwise distinct step sequences.  Summation order is wfsa_dev_viterbi's, so logw[i] is the
+ * left-to-right sum of the log weights of the steps, bit for bit, and the values do not depend on the kernel.  Ties: a
+ * node keeps the first strictly larger candidates, in the order (fent entry, source rank) with fast tables and (source
+ * state in eps_order, transition, emission, source rank) otherwise; the end in the order (candidate slot, rank),
+ * respectively (source state, transition, rank).  So rank 0 is the path and value of wfsa_dev_viterbi, bit for bit, and k = 1
+ * is wfsa_dev_viterbi.  Same bits on every call.  Local to the shard and without effect on evaluations, as
+ * wfsa_dev_viterbi.  WFSA_ERR_INVALID: k outside 1..16 or a null pointer; WFSA_ERR_STATE before wfsa_dev_set_param_map;
+ * WFSA_ERR_LIMIT when the handle decodes a CTA per string (more than 32 candidates per symbol) and the lists of its
+ * candidates at this k do not fit a CTA: 2 * K * G doubles of shared memory (K the power of two >= k, G the candidates
+ * rounded up to 32) over the device's opt-in limit, or, at K = 16, G over 768 threads; a smaller k may fit. */
+int wfsa_dev_nbest(wfsa_dev* h, const double* x, int32_t k, double* logw /* [n_strings*k] */, int64_t* path_off /* [n_strings*k + 1] */);
+/* Steps of the last wfsa_dev_viterbi or wfsa_dev_nbest, path_off[n_paths] of them, in path order:
  * trans_edge = index of the transition edge in the descriptor (trans_dst order); emis_edge = index of the emission edge
  * of its target state (emis_tok_off order), -1 for the final transition into the end state.  WFSA_ERR_STATE before any
- * wfsa_dev_viterbi. */
+ * wfsa_dev_viterbi or wfsa_dev_nbest. */
 int wfsa_dev_viterbi_paths(wfsa_dev* h, int32_t* trans_edge, int32_t* emis_edge);
 
 /* Multi-GPU: one handle per process/GPU; results of eval/structure/hessian are all-reduced as exact integer

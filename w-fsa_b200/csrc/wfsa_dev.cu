@@ -30,6 +30,7 @@
 #include "kernels_k7.cuh"
 #include "kernels_rmin.cuh"
 #include "kernels_viterbi.cuh"
+#include "kernels_nbest.cuh"
 #include "layout.hpp"
 #include "lattice.hpp"
 
@@ -227,14 +228,17 @@ struct wfsa_dev {
     int hb_fx_log2 = 40;
     // rmin without path blocks (rmin_sweep): per string m_s - log q_s, log q and (generic kernel) m_s, (min, +) weights, rmin
     DevBuf<double> d_rterm, d_mlq, d_mpath, d_mtw, d_mew, d_msw, d_mfw, d_rsweep;
-    // Viterbi (wfsa_dev_viterbi): its own x and (max, +) weights, so that an evaluation in flight keeps its x; per string
-    // logw and (generic kernel) step counts and offsets; backpointer slabs; the steps of the last call
-    DevBuf<double> d_vx, d_vtw, d_vew, d_vsw, d_vfw, d_vlogw;
+    // Viterbi and N-best (wfsa_dev_viterbi, wfsa_dev_nbest): their own x and (max, +) weights, so that an evaluation in
+    // flight keeps its x; per path (string s, rank r: s * k + r) logw and (generic kernel) step counts and offsets;
+    // backpointer slabs; kg_nbest's lists when the generic scratch holds fewer than k strings' lists; the steps of the last call
+    DevBuf<double> d_vx, d_vtw, d_vew, d_vsw, d_vfw, d_vlogw, d_nscratch;
     DevBuf<int32_t> d_vcnt, d_vtrans, d_vemis;
     DevBuf<int64_t> d_voff;
     DevBuf<uint16_t> d_vbp;
-    std::vector<int64_t> h_vpath_off;          // steps of string s: h_vpath_off[s]..[s+1], at d_vtrans + h_vsrc(s)
-    bool v_done = false, v_padded = false;     // padded: string s starts at offs[s] + s (fast tables), else at h_vpath_off[s]
+    std::vector<int64_t> h_vpath_off;          // steps of path i: h_vpath_off[i]..[i+1]
+    int v_k = 1;                               // paths per string of the last call
+    bool v_done = false, v_padded = false;     // padded: rank r of string s starts at k * (offs[s] + s) + r * (len_s + 1)
+                                               // (fast tables), else at h_vpath_off[s * k + r]
     // comm
     ncclComm_t comm = nullptr; int rank = 0, nranks = 1;
     // NVLink peer memory for the exchange inside k_eval6 (and the rank barrier of the benchmark); without it ncclAllReduce
@@ -1989,7 +1993,7 @@ static int rmin_sweep(wfsa_dev* h, bool all)
 }
 
 // Backpointer slabs of k3_viterbi: a group (warp or CTA) holds max_len x pitch uint16; the grid shrinks when the slabs
-// of all groups would take more than this (very long strings)
+// of all groups would take more than this (very long strings).  k3_nbest's slabs are k times as large, its budget K times.
 constexpr size_t kViterbiSlabBudget = (size_t)256 << 20;
 
 // k3_viterbi over one order list (fast tables): a warp per string when every symbol has at most 32 candidates, else a CTA
@@ -2023,51 +2027,110 @@ static int viterbi_fast_list(wfsa_dev* h, const int32_t* d_ord, int64_t n_ord)
     return WFSA_OK;
 }
 
-// kg_fwdbwd<MODE_VITERBI> over one order list in g_batch batches: step counts (d_voff == nullptr) or the steps
-static void viterbi_generic_list(wfsa_dev* h, const int32_t* d_ord, int64_t n_ord, const int64_t* d_voff)
+// k3_nbest<WARP, K> over one order list (fast tables), K the power of two >= k: a warp per string as k3_viterbi, else a
+// CTA.  The lists take 2 * K * G doubles of shared memory per group; WFSA_ERR_LIMIT when a CTA's do not fit, or when the
+// CTA would need more threads than k3_nbest<false, K> allows.
+static int nbest_fast_list(wfsa_dev* h, const int32_t* d_ord, int64_t n_ord, int k)
+{
+    if (n_ord <= 0) return WFSA_OK;
+    const HostFsa& F = h->fsa;
+    const FastLayout& L = h->fast;
+    K3NbestParams P{};
+    P.T = FastTablesD{h->d_cand_off.p, h->d_slot_state.p, h->d_frow.p, h->d_fent.p, h->d_brow.p, h->d_bent.p,
+                      F.n_sym, F.n_states, L.n_arcs, L.n_slots, F.start, L.start_final_tid};
+    P.vtw = h->d_vtw.p; P.vsw = h->d_vsw.p; P.vfw = h->d_vfw.p; P.slot_emis = h->d_slot_emis.p; P.slot_final = h->d_slot_final.p;
+    P.C = CorpusD{h->d_tokens.p, h->d_offs.p, h->d_p.p, d_ord, n_ord};
+    P.max_len = std::max(h->max_len, 1);
+    P.k = k;
+    P.logw = h->d_vlogw.p; P.trans_edge = h->d_vtrans.p; P.emis_edge = h->d_vemis.p;
+    const int K = k <= 2 ? 2 : k <= 4 ? 4 : k <= 8 ? 8 : 16;
+    const bool warp = L.max_cand <= 32;
+    const int nt = warp ? 256 : std::max(64, (L.max_cand + 31) / 32 * 32);
+    const size_t smem = (size_t)2 * K * nt * 8 + 32 * 8 + 32 * 4 + 32 * kNbestMax * 4;
+    int optin = 0;
+    CK(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, h->device));
+    if (smem > (size_t)optin || nt > nbest_cta_threads(K))
+        return set_err(h, WFSA_ERR_LIMIT, "nbest: the lists of " + std::to_string(nt) + " candidates at k = " + std::to_string(k) +
+                                              " need " + std::to_string(smem) + " bytes of shared memory per CTA (at most " +
+                                              std::to_string(optin) + ") and " + std::to_string(nt) + " threads (at most " +
+                                              std::to_string(nbest_cta_threads(K)) + "); use a smaller k");
+    const int per_cta = warp ? nt / 32 : 1;                                   // strings in flight per CTA
+    P.pitch = warp ? 32 : nt;
+    const size_t slab_bytes = (size_t)P.max_len * P.pitch * k * 2 * per_cta; // per CTA
+    long long grid = (long long)h->sm_count * (warp ? 8 : std::max(1, std::min(4, 1024 / nt)));
+    grid = std::min<long long>(grid, (n_ord + per_cta - 1) / per_cta);
+    grid = std::max<long long>(1, std::min<long long>(grid, (long long)(kViterbiSlabBudget * K / slab_bytes)));
+    const size_t need = (size_t)grid * per_cta * P.max_len * P.pitch * k;
+    if (h->d_vbp.n < need) CK(h->d_vbp.alloc(need));
+    P.bp = h->d_vbp.p;
+    auto launch = [&](auto kern) {
+        CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        kern<<<(unsigned)grid, nt, smem, h->stream>>>(P);
+        return WFSA_OK;
+    };
+    int rc;
+    switch (K) {
+    case 2: rc = warp ? launch(k3_nbest<true, 2>) : launch(k3_nbest<false, 2>); break;
+    case 4: rc = warp ? launch(k3_nbest<true, 4>) : launch(k3_nbest<false, 4>); break;
+    case 8: rc = warp ? launch(k3_nbest<true, 8>) : launch(k3_nbest<false, 8>); break;
+    default: rc = warp ? launch(k3_nbest<true, 16>) : launch(k3_nbest<false, 16>); break;
+    }
+    h->launches++;
+    return rc;
+}
+
+// Over one order list without fast tables, step counts (d_voff == nullptr) or the steps: kg_fwdbwd<MODE_VITERBI> in g_batch
+// batches (k = 1), else kg_nbest in batches of g_batch / k strings, whose lists take k times a string's scratch
+static void viterbi_generic_list(wfsa_dev* h, const int32_t* d_ord, int64_t n_ord, const int64_t* d_voff, int k)
 {
     const HostFsa& F = h->fsa;
     GenericParams P{};
     P.G = GenericTablesD{h->d_emis_row.p, h->d_emis_tok_off.p, h->d_emis_tok.p, h->d_trans_row.p, h->d_trans_dst.p,
                          h->d_eps_order.p, F.n_states, F.n_trans(), F.start, F.end};
     P.C = CorpusD{h->d_tokens.p, h->d_offs.p, h->d_p.p, d_ord, n_ord};
-    P.scratch = h->d_gscratch.p; P.max_len = h->max_len;
+    P.scratch = k > 1 && h->g_batch < k ? h->d_nscratch.p : h->d_gscratch.p; P.max_len = h->max_len;
     P.ltw = h->d_vtw.p; P.lew = h->d_vew.p; P.O.logq = h->d_vlogw.p;
     P.vit_cnt = h->d_vcnt.p; P.vit_off = d_voff; P.vit_trans = h->d_vtrans.p; P.vit_emis = h->d_vemis.p;
-    for (long long first = 0; first < n_ord; first += h->g_batch) {
-        P.first = first; P.count = std::min<long long>(h->g_batch, n_ord - first);
-        kg_fwdbwd<MODE_VITERBI><<<(unsigned)((P.count + 127) / 128), 128, 0, h->stream>>>(P);
+    const long long batch = std::max<long long>(1, h->g_batch / k);
+    for (long long first = 0; first < n_ord; first += batch) {
+        P.first = first; P.count = std::min<long long>(batch, n_ord - first);
+        if (k == 1) kg_fwdbwd<MODE_VITERBI><<<(unsigned)((P.count + 127) / 128), 128, 0, h->stream>>>(P);
+        else kg_nbest<<<(unsigned)((P.count + 127) / 128), 128, 0, h->stream>>>(P, k);
         h->launches++;
     }
 }
 
-extern "C" int wfsa_dev_viterbi(wfsa_dev* h, const double* x, double* logw, int64_t* path_off)
+// wfsa_dev_viterbi (k = 1: k3_viterbi, kg_fwdbwd<MODE_VITERBI>) and wfsa_dev_nbest (k3_nbest, kg_nbest); path i = s * k + r
+static int decode_paths(wfsa_dev* h, const double* x, int k, double* logw, int64_t* path_off)
 {
-    if (!h || !logw || !path_off) return set_err(h, WFSA_ERR_INVALID, "viterbi: bad arguments");
-    if (h->n < 0) return set_err(h, WFSA_ERR_STATE, "viterbi before set_param_map");
-    if (!x && h->n > 0) return set_err(h, WFSA_ERR_INVALID, "viterbi: bad arguments");
     CK(cudaSetDevice(h->device));
     h->v_done = false;
     const HostFsa& F = h->fsa;
     const FastLayout& L = h->fast;
     cudaStream_t st = h->stream;
-    const int64_t ns = h->n_strings;
+    const int64_t ns = h->n_strings, np = ns * k;
     const int n_slots = L.ok ? L.n_slots : 0;
     if (h->d_vx.n < (size_t)h->n + 1) CK(h->d_vx.alloc((size_t)h->n + 1));
-    if (!h->d_vlogw.p) {
+    if (!h->d_vtw.p) {
         CK(h->d_vtw.alloc(std::max(F.n_trans(), 1))); CK(h->d_vew.alloc(std::max(F.n_emis(), 1)));
         CK(h->d_vsw.alloc(std::max(n_slots, 1))); CK(h->d_vfw.alloc(std::max(n_slots, 1)));
-        CK(h->d_vlogw.alloc((size_t)std::max<int64_t>(ns, 1)));
-        if (!L.ok) { CK(h->d_vcnt.alloc((size_t)std::max<int64_t>(ns, 1))); CK(h->d_voff.alloc((size_t)ns + 1)); }
     }
-    if (L.ok && h->d_vtrans.n < (size_t)(h->n_tokens + ns)) {             // fast tables: len + 1 steps, at offs[s] + s
-        CK(h->d_vtrans.alloc((size_t)std::max<int64_t>(h->n_tokens + ns, 1)));
-        CK(h->d_vemis.alloc((size_t)std::max<int64_t>(h->n_tokens + ns, 1)));
+    if (h->d_vlogw.n < (size_t)std::max<int64_t>(np, 1)) {
+        CK(h->d_vlogw.alloc((size_t)std::max<int64_t>(np, 1)));
+        if (!L.ok) { CK(h->d_vcnt.alloc((size_t)std::max<int64_t>(np, 1))); CK(h->d_voff.alloc((size_t)np + 1)); }
+    }
+    if (L.ok && h->d_vtrans.n < (size_t)(k * (h->n_tokens + ns))) {       // fast tables: len + 1 steps per path, padded
+        CK(h->d_vtrans.alloc((size_t)std::max<int64_t>(k * (h->n_tokens + ns), 1)));
+        CK(h->d_vemis.alloc((size_t)std::max<int64_t>(k * (h->n_tokens + ns), 1)));
+    }
+    if (!L.ok && k > 1 && h->g_batch < k) {                                 // kg_nbest needs room for one string's k lists
+        const size_t per = (size_t)2 * (h->max_len + 1) * F.n_states * k;
+        if (h->d_nscratch.n < per) CK(h->d_nscratch.alloc(per));
     }
     if (h->n > 0) CK(cudaMemcpyAsync(h->d_vx.p, x, (size_t)h->n * 8, cudaMemcpyHostToDevice, st));
-    const long long total = (long long)F.n_trans() + F.n_emis() + n_slots + ns;
+    const long long total = (long long)F.n_trans() + F.n_emis() + n_slots + np;
     if (total > 0) {
-        k_maxplus_weights<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(F.n_trans(), F.n_emis(), n_slots, (long long)ns,
+        k_maxplus_weights<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(F.n_trans(), F.n_emis(), n_slots, (long long)np,
                                                                          h->d_trans_tp.p, h->d_emis_tp.p, h->d_slot_emis.p,
                                                                          h->d_slot_final.p, h->d_vx.p, h->d_vtw.p, h->d_vew.p,
                                                                          h->d_vsw.p, h->d_vfw.p, h->d_vlogw.p);
@@ -2079,47 +2142,69 @@ extern "C" int wfsa_dev_viterbi(wfsa_dev* h, const double* x, double* logw, int6
     if (h->kernel == 6 || h->kernel == 7) { counts[0] = h->n_active + h->n_active_w; counts[1] = 0; }
     std::vector<int32_t> cnt;
     if (L.ok) {
-        for (int i = 0; i < 2; ++i) { const int rc = viterbi_fast_list(h, lists[i], counts[i]); if (rc != WFSA_OK) return rc; }
+        for (int i = 0; i < 2; ++i) {
+            const int rc = k == 1 ? viterbi_fast_list(h, lists[i], counts[i]) : nbest_fast_list(h, lists[i], counts[i], k);
+            if (rc != WFSA_OK) return rc;
+        }
     } else {
         // step counts first (they vary with empty and multi-token emissions), then their prefix sum, then the steps
-        if (ns) CK(cudaMemsetAsync(h->d_vcnt.p, 0, (size_t)ns * 4, st));
-        for (int i = 0; i < 2; ++i) if (counts[i] > 0) viterbi_generic_list(h, lists[i], counts[i], nullptr);
-        cnt.resize((size_t)ns);
-        if (ns) CK(cudaMemcpyAsync(cnt.data(), h->d_vcnt.p, (size_t)ns * 4, cudaMemcpyDeviceToHost, st));
+        if (np) CK(cudaMemsetAsync(h->d_vcnt.p, 0, (size_t)np * 4, st));
+        for (int i = 0; i < 2; ++i) if (counts[i] > 0) viterbi_generic_list(h, lists[i], counts[i], nullptr, k);
+        cnt.resize((size_t)np);
+        if (np) CK(cudaMemcpyAsync(cnt.data(), h->d_vcnt.p, (size_t)np * 4, cudaMemcpyDeviceToHost, st));
         CK(cudaStreamSynchronize(st));
         CK(cudaGetLastError());
     }
-    if (ns) CK(cudaMemcpyAsync(logw, h->d_vlogw.p, (size_t)ns * 8, cudaMemcpyDeviceToHost, st));
+    if (np) CK(cudaMemcpyAsync(logw, h->d_vlogw.p, (size_t)np * 8, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
     CK(cudaGetLastError());
     path_off[0] = 0;
-    for (int64_t s = 0; s < ns; ++s)
-        path_off[s + 1] = path_off[s] + (L.ok ? (logw[s] > -INFINITY ? h->h_offs[s + 1] - h->h_offs[s] + 1 : 0) : cnt[(size_t)s]);
-    h->h_vpath_off.assign(path_off, path_off + ns + 1);
+    for (int64_t i = 0; i < np; ++i) {
+        const int64_t s = i / k;
+        path_off[i + 1] = path_off[i] + (L.ok ? (logw[i] > -INFINITY ? h->h_offs[s + 1] - h->h_offs[s] + 1 : 0) : cnt[(size_t)i]);
+    }
+    h->h_vpath_off.assign(path_off, path_off + np + 1);
     if (!L.ok) {
-        const int64_t steps = path_off[ns];
+        const int64_t steps = path_off[np];
         if (h->d_vtrans.n < (size_t)std::max<int64_t>(steps, 1)) {
             CK(h->d_vtrans.alloc((size_t)std::max<int64_t>(steps, 1))); CK(h->d_vemis.alloc((size_t)std::max<int64_t>(steps, 1)));
         }
-        CK(cudaMemcpyAsync(h->d_voff.p, path_off, (size_t)(ns + 1) * 8, cudaMemcpyHostToDevice, st));
-        for (int i = 0; i < 2; ++i) if (counts[i] > 0) viterbi_generic_list(h, lists[i], counts[i], h->d_voff.p);
+        CK(cudaMemcpyAsync(h->d_voff.p, path_off, (size_t)(np + 1) * 8, cudaMemcpyHostToDevice, st));
+        for (int i = 0; i < 2; ++i) if (counts[i] > 0) viterbi_generic_list(h, lists[i], counts[i], h->d_voff.p, k);
         CK(cudaStreamSynchronize(st));
         CK(cudaGetLastError());
     }
+    h->v_k = k;
     h->v_padded = L.ok;
     h->v_done = true;
     return WFSA_OK;
 }
 
+extern "C" int wfsa_dev_viterbi(wfsa_dev* h, const double* x, double* logw, int64_t* path_off)
+{
+    if (!h || !logw || !path_off) return set_err(h, WFSA_ERR_INVALID, "viterbi: bad arguments");
+    if (h->n < 0) return set_err(h, WFSA_ERR_STATE, "viterbi before set_param_map");
+    if (!x && h->n > 0) return set_err(h, WFSA_ERR_INVALID, "viterbi: bad arguments");
+    return decode_paths(h, x, 1, logw, path_off);
+}
+
+extern "C" int wfsa_dev_nbest(wfsa_dev* h, const double* x, int32_t k, double* logw, int64_t* path_off)
+{
+    if (!h || !logw || !path_off || k < 1 || k > kNbestMax) return set_err(h, WFSA_ERR_INVALID, "nbest: bad arguments (k: 1..16)");
+    if (h->n < 0) return set_err(h, WFSA_ERR_STATE, "nbest before set_param_map");
+    if (!x && h->n > 0) return set_err(h, WFSA_ERR_INVALID, "nbest: bad arguments");
+    return decode_paths(h, x, k, logw, path_off);
+}
+
 extern "C" int wfsa_dev_viterbi_paths(wfsa_dev* h, int32_t* trans_edge, int32_t* emis_edge)
 {
     if (!h || !trans_edge || !emis_edge) return set_err(h, WFSA_ERR_INVALID, "viterbi_paths: bad arguments");
-    if (!h->v_done) return set_err(h, WFSA_ERR_STATE, "viterbi_paths before viterbi");
+    if (!h->v_done) return set_err(h, WFSA_ERR_STATE, "viterbi_paths before viterbi or nbest");
     CK(cudaSetDevice(h->device));
-    const int64_t ns = h->n_strings;
+    const int64_t ns = h->n_strings, k = h->v_k, np = ns * k;
     const std::vector<int64_t>& po = h->h_vpath_off;
     if (!h->v_padded) {
-        const size_t steps = (size_t)po[ns];
+        const size_t steps = (size_t)po[np];
         if (steps) {
             CK(cudaMemcpyAsync(trans_edge, h->d_vtrans.p, steps * 4, cudaMemcpyDeviceToHost, h->stream));
             CK(cudaMemcpyAsync(emis_edge, h->d_vemis.p, steps * 4, cudaMemcpyDeviceToHost, h->stream));
@@ -2127,19 +2212,20 @@ extern "C" int wfsa_dev_viterbi_paths(wfsa_dev* h, int32_t* trans_edge, int32_t*
         CK(cudaStreamSynchronize(h->stream));
         return WFSA_OK;
     }
-    // string s was written at offs[s] + s: copy the whole range, keep the strings that have a path
-    const size_t padded = (size_t)(h->n_tokens + ns);
+    // rank r of string s was written at k * (offs[s] + s) + r * (len_s + 1): copy the whole range, keep the paths found
+    const size_t padded = (size_t)(k * (h->n_tokens + ns));
     std::vector<int32_t> tr(padded), em(padded);
     if (padded) {
         CK(cudaMemcpyAsync(tr.data(), h->d_vtrans.p, padded * 4, cudaMemcpyDeviceToHost, h->stream));
         CK(cudaMemcpyAsync(em.data(), h->d_vemis.p, padded * 4, cudaMemcpyDeviceToHost, h->stream));
     }
     CK(cudaStreamSynchronize(h->stream));
-    for (int64_t s = 0; s < ns; ++s) {
-        const int64_t k = po[s + 1] - po[s], src = h->h_offs[s] + s;
-        if (k) {
-            std::memcpy(trans_edge + po[s], tr.data() + src, (size_t)k * 4);
-            std::memcpy(emis_edge + po[s], em.data() + src, (size_t)k * 4);
+    for (int64_t i = 0; i < np; ++i) {
+        const int64_t s = i / k, r = i % k, m = po[i + 1] - po[i];
+        const int64_t src = k * (h->h_offs[s] + s) + r * (h->h_offs[s + 1] - h->h_offs[s] + 1);
+        if (m) {
+            std::memcpy(trans_edge + po[i], tr.data() + src, (size_t)m * 4);
+            std::memcpy(emis_edge + po[i], em.data() + src, (size_t)m * 4);
         }
     }
     return WFSA_OK;

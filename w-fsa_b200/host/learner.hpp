@@ -83,10 +83,11 @@ public:
     // dense H_f (n x n, row major) at the current x; builds the path blocks on first use
     void ComputeHfDense(std::vector<double>& Hf, double* rmin = nullptr);
     double ComputeRmin();
-    // most probable path of every string of this shard at the current x (wfsa_dev_viterbi), with log q_s at the same x;
-    // local to the shard (the evaluation inside is collective with several ranks)
-    struct Decoding { std::vector<double> logw, logq; std::vector<int64_t> path_off; std::vector<int32_t> trans_edge, emis_edge; };
-    void Decode(Decoding& d);
+    // the k most probable paths of every string of this shard at the current x (k = 1: wfsa_dev_viterbi, else
+    // wfsa_dev_nbest; path s * k + r is rank r of string s), with log q_s at the same x; local to the shard (the evaluation
+    // inside is collective with several ranks)
+    struct Decoding { int k = 1; std::vector<double> logw, logq; std::vector<int64_t> path_off; std::vector<int32_t> trans_edge, emis_edge; };
+    void Decode(Decoding& d, int k = 1);
 
 protected:
     virtual void FinalizeCallback() {}

@@ -6,7 +6,8 @@
 // backend has no P/M matrices to cache.  -r only orders the -p/-pr path listing (BFS/DFS).  Added: --device N, --full (dump weights with 17 digits),
 // --gpus N: one process per GPU (forked before anything touches CUDA), corpus cut into N ranges of equal symbol count, the
 // same optimiser loop on every rank with loglik / gradient / H_f summed over the ranks inside the backend; rank 0 reports.
-// --viterbi FILE: the most probable path of every corpus string with the final weights (write_viterbi).
+// --viterbi FILE: the most probable path of every corpus string with the final weights; --nbest K FILE: the K most
+// probable paths (write_paths).
 #include <cfloat>
 #include <cmath>
 #include <cstdio>
@@ -81,36 +82,45 @@ static void print_paths(const Fsa& fsa, const Corpus& corpus, bool bfs)
 // --viterbi FILE: one line per corpus string, in corpus order,  word TAB ln w(pi) TAB w(pi)/q_s TAB path,  pi the most
 // probable path of the word (wfsa_dev_viterbi), the path in the format of -p without its "text: " prefix; "-inf", 0 and an
 // empty path for a word without a path.
-static void write_viterbi(const std::string& filename, const Fsa& fsa, const Corpus& corpus, Learner& learner)
+// --nbest K FILE (nbest = K): min(K, paths) lines per corpus string, in corpus order and by rank,
+// word TAB rank TAB ln w(pi) TAB w(pi)/q_s TAB path,  rank from 1 (wfsa_dev_nbest); "0", "-inf", 0 and an empty path for a
+// word without a path.
+static void write_paths(const std::string& filename, const Fsa& fsa, const Corpus& corpus, Learner& learner, int nbest = 0)
 {
     Learner::Decoding d;
-    learner.Decode(d);
+    learner.Decode(d, nbest ? nbest : 1);
+    const size_t k = (size_t)d.k;
     FILE* out = fopen(filename.c_str(), "w");
     if (!out) throw MyError("Unable to open output file \"" + filename + "\" for writing!");
     const auto& st = fsa.States();
     const LoweredFsa& L = learner.Lowered();
     std::string line;
     for (size_t s = 0; s < corpus.size(); ++s) {
-        line = corpus[s].first;
-        if (!(d.logw[s] > -INFINITY)) {
-            line += "\t-inf\t0\t\n";
-        } else {
+        if (!(d.logw[s * k] > -INFINITY)) {
+            line = corpus[s].first + (nbest ? "\t0" : "") + "\t-inf\t0\t\n";
+            fwrite(line.data(), 1, line.size(), out);
+            continue;
+        }
+        for (size_t r = 0; r < k && d.logw[s * k + r] > -INFINITY; ++r) {
+            const size_t i = s * k + r;
+            line = corpus[s].first;
+            if (nbest) line += "\t" + std::to_string(r + 1);
             char num[64];
-            snprintf(num, sizeof num, "\t%.17g", d.logw[s]); line += num;
-            snprintf(num, sizeof num, "\t%.17g\t", std::exp(d.logw[s] - d.logq[s])); line += num;
+            snprintf(num, sizeof num, "\t%.17g", d.logw[i]); line += num;
+            snprintf(num, sizeof num, "\t%.17g\t", std::exp(d.logw[i] - d.logq[s])); line += num;
             line += fsa.GetStartState();
-            for (int64_t k = d.path_off[s]; k < d.path_off[s + 1]; ++k) {
-                const auto& te = L.trans_edge[d.trans_edge[k]];
+            for (int64_t j = d.path_off[i]; j < d.path_off[i + 1]; ++j) {
+                const auto& te = L.trans_edge[d.trans_edge[j]];
                 line += " -> " + st[st[te.first].transitions[te.second].next].name;
-                if (d.emis_edge[k] >= 0) {
-                    const auto& ee = L.emis_edge[d.emis_edge[k]];
+                if (d.emis_edge[j] >= 0) {
+                    const auto& ee = L.emis_edge[d.emis_edge[j]];
                     const std::string& e = st[ee.first].emissions[ee.second].str;
                     if (!e.empty()) line += '"' + e + '"';
                 }
             }
             line += '\n';
+            fwrite(line.data(), 1, line.size(), out);
         }
-        fwrite(line.data(), 1, line.size(), out);
     }
     if (fclose(out) != 0) throw MyError("Unable to write \"" + filename + "\"!");
 }
@@ -159,13 +169,16 @@ static void usage()
         "  --full                     dump weights with 17 significant digits\n"
         "  --viterbi FILE             after the optimization, write the most probable path of every corpus string with the\n"
         "                             final weights (after -n) to FILE: word, ln w(path), w(path)/q(word), path (one GPU);\n"
-        "                             -e 0 -s decodes with the automaton file's own weights\n";
+        "                             -e 0 -s decodes with the automaton file's own weights\n"
+        "  --nbest K FILE             as --viterbi, the K (1..16) most probable paths of every corpus string, best first:\n"
+        "                             word, rank, ln w(path), w(path)/q(word), path; a word without a path gets one line\n"
+        "                             with rank 0 (one GPU)\n";
 }
 
 int main(int argc, const char* argv[])
 {
-    std::string automaton_filename, corpus_filename, output_filename, viterbi_filename, optimizer = "Hessian";
-    int epochs = 20, initflags = 0, device = 0, gpus = 1;
+    std::string automaton_filename, corpus_filename, output_filename, viterbi_filename, nbest_filename, optimizer = "Hessian";
+    int epochs = 20, initflags = 0, device = 0, gpus = 1, nbest = 0;
     bool normalize = false, print = false, print_recognize = false, suppress = false, evaluate = false, initx = false, full = false;
     int recognize = 0;
     double eta = 1.0, tolerance = 1e-6;
@@ -200,11 +213,23 @@ int main(int argc, const char* argv[])
         else if (is(a, {"--gpus"})) { gpus = atoi(next()); if (gpus < 1 || gpus > 8) { std::cerr << "--gpus must be between 1 and 8" << std::endl; return 1; } }
         else if (is(a, {"--full"})) full = true;
         else if (is(a, {"--viterbi"})) viterbi_filename = next();
+        else if (is(a, {"--nbest"})) {
+            const char* v = next();
+            char* end = nullptr;
+            const long K = std::strtol(v, &end, 10);
+            if (end == v || *end || K < 1 || K > 16) { std::cerr << "--nbest K must be between 1 and 16" << std::endl; return 1; }
+            nbest = (int)K;
+            nbest_filename = next();
+        }
         else if (is(a, {"-m", "--matrices", "--matrix"})) { next(); std::cerr << "-m is not supported: the DP backend has no path matrices to cache" << std::endl; return 1; }
         else { std::cerr << "Unknown argument \"" << a << "\"!" << std::endl; return 1; }
     }
     if (!viterbi_filename.empty() && gpus > 1) {
         std::cerr << "--viterbi decodes on one GPU: it cannot be combined with --gpus " << gpus << std::endl;
+        return 1;
+    }
+    if (nbest && gpus > 1) {
+        std::cerr << "--nbest decodes on one GPU: it cannot be combined with --gpus " << gpus << std::endl;
         return 1;
     }
     // --gpus N: fork the other ranks before CUDA is touched.  Rank 0 (this process) creates the communicator id and hands
@@ -328,7 +353,8 @@ int main(int argc, const char* argv[])
             for (double x : results) std::cerr << ' ' << x;
             std::cerr << std::endl;
         }
-        if (!viterbi_filename.empty()) write_viterbi(viterbi_filename, fsa, corpus, *learner);
+        if (!viterbi_filename.empty()) write_paths(viterbi_filename, fsa, corpus, *learner);
+        if (nbest) write_paths(nbest_filename, fsa, corpus, *learner, nbest);
         if (!suppress && rank == 0) {
             FILE* outf = output_filename.empty() ? stdout : fopen(output_filename.c_str(), "w");
             if (!outf) throw MyError("Unable to open output file \"" + output_filename + "\" for writing!");

@@ -18,7 +18,7 @@ UNIQUE_ID_BYTES = 128
 DEV_SYMBOLS = [
     "wfsa_dev_create", "wfsa_dev_structure", "wfsa_dev_set_param_map", "wfsa_dev_eval", "wfsa_dev_upload_x",
     "wfsa_dev_eval_launch", "wfsa_dev_eval_fetch", "wfsa_dev_sync", "wfsa_dev_set_path_blocks", "wfsa_dev_hessian",
-    "wfsa_dev_viterbi", "wfsa_dev_viterbi_paths",
+    "wfsa_dev_viterbi", "wfsa_dev_viterbi_paths", "wfsa_dev_nbest",
     "wfsa_dev_comm_unique_id", "wfsa_dev_comm_init", "wfsa_dev_allreduce_f64", "wfsa_dev_timer_begin", "wfsa_dev_timer_begin_steps",
     "wfsa_dev_timer_end", "wfsa_dev_timer_kernel_ms", "wfsa_dev_timer_split_ms", "wfsa_dev_timer_step_ms", "wfsa_dev_timer_phase_ms", "wfsa_dev_eval6_phases", "wfsa_dev_l2_flush", "wfsa_dev_rank_barrier", "wfsa_dev_get_info", "wfsa_dev_destroy", "wfsa_dev_held_bytes", "wfsa_dev_last_error",
     "wfsa_dev_version", "wfsa_lattice_compile", "wfsa_segmented_compile", "wfsa_segmented_get",
@@ -135,6 +135,7 @@ def lib():
         L.wfsa_dev_hessian.argtypes = [C.c_void_p, F64P, F64P, F64P]
         L.wfsa_dev_viterbi.argtypes = [C.c_void_p, F64P, F64P, I64P]
         L.wfsa_dev_viterbi_paths.argtypes = [C.c_void_p, I32P, I32P]
+        L.wfsa_dev_nbest.argtypes = [C.c_void_p, F64P, C.c_int32, F64P, I64P]
         L.wfsa_dev_comm_unique_id.argtypes = [C.c_void_p]
         L.wfsa_dev_comm_init.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int]
         L.wfsa_dev_allreduce_f64.argtypes = [C.c_void_p, F64P, C.c_int, C.c_int]
@@ -375,6 +376,13 @@ class Device:
         [path_off[s], path_off[s+1]) (descriptor edge ids; emis_edge -1 on the final transition), logw[s] = -inf: none."""
         return _viterbi(self.L, self.h, x, self.n_strings)
 
+    def nbest(self, x, k):
+        """The k most probable paths of every string at x: (logw [n_strings, k], path_off, trans_edge, emis_edge); path
+        i = s * k + r is the r-th most probable path of string s, its steps [path_off[i], path_off[i+1]) as in viterbi,
+        logw[s, r] = -inf: string s has at most r paths."""
+        logw, off, tr, em = _viterbi(self.L, self.h, x, self.n_strings, k)
+        return logw.reshape(self.n_strings, k), off, tr, em
+
     def timer_begin(self):
         self._ck(self.L.wfsa_dev_timer_begin(self.h))
 
@@ -441,19 +449,24 @@ class Device:
             pass
 
 
-def _viterbi(L, h, x, n_strings):
+def _viterbi(L, h, x, n_strings, k=None):
+    """wfsa_dev_viterbi (k None) or wfsa_dev_nbest, then the steps: (logw, path_off, trans_edge, emis_edge) per path."""
     def ck(rc):
         if rc != 0:
             raise WfsaError(rc, L.wfsa_dev_last_error(h).decode())
     x = np.ascontiguousarray(x, dtype=np.float64)
-    logw = np.zeros(max(n_strings, 1))
-    off = np.zeros(n_strings + 1, dtype=np.int64)
-    ck(L.wfsa_dev_viterbi(h, _p(x, F64P), _p(logw, F64P), _p(off, I64P)))
+    n_paths = n_strings * (k or 1)
+    logw = np.zeros(max(n_paths, 1))
+    off = np.zeros(n_paths + 1, dtype=np.int64)
+    if k is None:
+        ck(L.wfsa_dev_viterbi(h, _p(x, F64P), _p(logw, F64P), _p(off, I64P)))
+    else:
+        ck(L.wfsa_dev_nbest(h, _p(x, F64P), k, _p(logw, F64P), _p(off, I64P)))
     steps = max(int(off[-1]), 1)
     tr = np.zeros(steps, dtype=np.int32)
     em = np.zeros(steps, dtype=np.int32)
     ck(L.wfsa_dev_viterbi_paths(h, _p(tr, I32P), _p(em, I32P)))
-    return logw[:n_strings], off, tr[:off[-1]], em[:off[-1]]
+    return logw[:n_paths], off, tr[:off[-1]], em[:off[-1]]
 
 
 class Session:
@@ -532,6 +545,12 @@ class Session:
     def viterbi(self, x=None):
         """Device.viterbi on the session's backend, at x or the current weights, for every string of this shard."""
         return _viterbi(self.L, self.L.wfsa_session_backend(self.h), self.x() if x is None else x, self.backend_info()["n_strings"])
+
+    def nbest(self, k, x=None):
+        """Device.nbest on the session's backend, at x or the current weights, for every string of this shard."""
+        ns = self.backend_info()["n_strings"]
+        logw, off, tr, em = _viterbi(self.L, self.L.wfsa_session_backend(self.h), self.x() if x is None else x, ns, k)
+        return logw.reshape(ns, k), off, tr, em
 
     def backend_info(self):
         i = DevInfo()

@@ -149,7 +149,7 @@ int wfsa_dev_hessian(wfsa_dev* h, const double* x, double* Hf /* n*n, or NULL: o
  *   path_off[s]..path_off[s+1]: the steps of that path (path_off: n_strings + 1 entries; 0 steps when logw[s] = -inf).
  * logw[s] is the left-to-right sum of the log weights of the steps (transition, then emission, ..., final transition), bit
  * for bit.  Ties are broken deterministically (same bits on every call).  The paths stay on the device until the next
- * wfsa_dev_viterbi, wfsa_dev_nbest or wfsa_dev_destroy.  Local to the shard: no collective, also with a communicator attached.  The call
+ * wfsa_dev_viterbi, wfsa_dev_nbest, wfsa_dev_sample or wfsa_dev_destroy.  Local to the shard: no collective, also with a communicator attached.  The call
  * keeps its own copy of x: it changes nothing an evaluation returns, also between wfsa_dev_eval_launch and
  * wfsa_dev_eval_fetch.  WFSA_ERR_STATE before wfsa_dev_set_param_map. */
 int wfsa_dev_viterbi(wfsa_dev* h, const double* x, double* logw, int64_t* path_off);
@@ -169,10 +169,31 @@ int wfsa_dev_viterbi(wfsa_dev* h, const double* x, double* logw, int64_t* path_o
  * candidates at this k do not fit a CTA: 2 * K * G doubles of shared memory (K the power of two >= k, G the candidates
  * rounded up to 32) over the device's opt-in limit, or, at K = 16, G over 768 threads; a smaller k may fit. */
 int wfsa_dev_nbest(wfsa_dev* h, const double* x, int32_t k, double* logw /* [n_strings*k] */, int64_t* path_off /* [n_strings*k + 1] */);
-/* Steps of the last wfsa_dev_viterbi or wfsa_dev_nbest, path_off[n_paths] of them, in path order:
+/* n independent draws from p(pi | s) = w(pi) / q_s for every string of this shard, 1 <= n <= 256, at x; path i = s * n + r is
+ * draw r of string s:
+ *   logw[i] = summed log weight of the draw's steps, the left-to-right sum (acc + log a) + log b of wfsa_dev_viterbi, bit
+ *             for bit, so a draw that is also an N-best path has that path's wfsa_dev_nbest value (-inf, and 0 steps, for
+ *             every draw of a string without a path under the parameter map and x, or that does not take part in
+ *             evaluations);
+ *   logq[s] = log q_s from the sampler's own forward sweep, as the evaluation's log q (logq may be NULL);
+ *   path_off[i]..path_off[i+1]: the draw's steps (path_off: n_strings * n + 1 entries), through wfsa_dev_viterbi_paths.
+ * Randomness: Philox4x32-10 (wfsa_philox4x32_10 of wfsa_host.h) under the key (seed & 0xffffffff, seed >> 32); choice d of
+ * draw r of string s (s the shard's string index, d counted from 0 within the draw) uses the counter (d, r, s, 0) and
+ * u = ((o0 << 32 | o1) >> 11) * 2^-53.  At a node the draw takes the first entry, in table order, whose running sum exceeds
+ * u * total; when rounding leaves none, the last entry of positive weight.  Draw r of string s is therefore a function of
+ * (automaton, parameter map, x, seed, s, r) only: the first m draws of a call with n > m are the draws of a call with
+ * n = m, and every handle with fast tables (kernels 1, 2, 4, 6, 7, a warp or a CTA per string) returns the same bits.
+ * Handles without fast tables choose in another order (forward from the start state instead of back from the end): their
+ * draws differ but follow the same distribution.  Same bits on every call.  Local to the shard and without effect on
+ * evaluations, as wfsa_dev_viterbi.  WFSA_ERR_INVALID: n outside 1..256 or a null pointer (other than logq);
+ * WFSA_ERR_STATE before wfsa_dev_set_param_map; WFSA_ERR_NOMEM, with a message, when the padded step buffer of
+ * n * (symbols + strings) steps cannot be allocated (checked before any launch). */
+int wfsa_dev_sample(wfsa_dev* h, const double* x, int32_t n, uint64_t seed, double* logw /* [n_strings*n] */,
+                    double* logq /* [n_strings] or NULL */, int64_t* path_off /* [n_strings*n + 1] */);
+/* Steps of the last wfsa_dev_viterbi, wfsa_dev_nbest or wfsa_dev_sample, path_off[n_paths] of them, in path order:
  * trans_edge = index of the transition edge in the descriptor (trans_dst order); emis_edge = index of the emission edge
  * of its target state (emis_tok_off order), -1 for the final transition into the end state.  WFSA_ERR_STATE before any
- * wfsa_dev_viterbi or wfsa_dev_nbest. */
+ * wfsa_dev_viterbi, wfsa_dev_nbest or wfsa_dev_sample. */
 int wfsa_dev_viterbi_paths(wfsa_dev* h, int32_t* trans_edge, int32_t* emis_edge);
 
 /* Multi-GPU: one handle per process/GPU; results of eval/structure/hessian are all-reduced as exact integer

@@ -30,6 +30,10 @@ const char* wfsa_host_last_error(void);
 int wfsa_host_kkt_solve(int32_t n, int32_t k, const double* expx, const double* lambda, const int32_t* ccol, const double* rhs,
                         double* sol_schur, double* sol_dense, int32_t* inertia4);
 
+/* Host-only: the Philox4x32-10 block function (10 rounds, Random123's constants) that wfsa_dev_sample draws with, from the
+ * same source as the kernels: out = philox(ctr, key). */
+void wfsa_philox4x32_10(const uint32_t ctr[4], const uint32_t key[2], uint32_t out[4]);
+
 typedef struct wfsa_session wfsa_session;
 typedef struct {
     int32_t device, force_kernel, accum_mode, accum_variant;

@@ -31,6 +31,7 @@
 #include "kernels_rmin.cuh"
 #include "kernels_viterbi.cuh"
 #include "kernels_nbest.cuh"
+#include "kernels_sample.cuh"
 #include "layout.hpp"
 #include "lattice.hpp"
 
@@ -232,11 +233,14 @@ struct wfsa_dev {
     // flight keeps its x; per path (string s, rank r: s * k + r) logw and (generic kernel) step counts and offsets;
     // backpointer slabs; kg_nbest's lists when the generic scratch holds fewer than k strings' lists; the steps of the last call
     DevBuf<double> d_vx, d_vtw, d_vew, d_vsw, d_vfw, d_vlogw, d_nscratch;
+    // sampling (wfsa_dev_sample) besides: its linear weights (k_weights of its own x) and k3_sample's alpha slabs; d_vlogw
+    // holds the logw of its n_strings * n draws and then log q of every string
+    DevBuf<double> d_stw, d_ssw, d_sfw, d_sslab;
     DevBuf<int32_t> d_vcnt, d_vtrans, d_vemis;
     DevBuf<int64_t> d_voff;
     DevBuf<uint16_t> d_vbp;
     std::vector<int64_t> h_vpath_off;          // steps of path i: h_vpath_off[i]..[i+1]
-    int v_k = 1;                               // paths per string of the last call
+    int v_k = 1;                               // paths per string of the last call (draws for wfsa_dev_sample)
     bool v_done = false, v_padded = false;     // padded: rank r of string s starts at k * (offs[s] + s) + r * (len_s + 1)
                                                // (fast tables), else at h_vpath_off[s * k + r]
     // comm
@@ -2079,29 +2083,75 @@ static int nbest_fast_list(wfsa_dev* h, const int32_t* d_ord, int64_t n_ord, int
     return rc;
 }
 
+// wfsa_dev_sample's arguments, for decode_paths
+struct SampleSpec {
+    uint64_t seed;
+    double* logq;                            // [n_strings], on the host
+};
+
+// k3_sample over one order list (fast tables): k3_viterbi's groups and grid; its alpha slabs take four times the bytes of
+// k3_viterbi's backpointer slabs, within four times their budget
+static int sample_fast_list(wfsa_dev* h, const int32_t* d_ord, int64_t n_ord, int n, uint64_t seed)
+{
+    if (n_ord <= 0) return WFSA_OK;
+    const HostFsa& F = h->fsa;
+    const FastLayout& L = h->fast;
+    K3SampleParams P{};
+    P.T = FastTablesD{h->d_cand_off.p, h->d_slot_state.p, h->d_frow.p, h->d_fent.p, h->d_brow.p, h->d_bent.p,
+                      F.n_sym, F.n_states, L.n_arcs, L.n_slots, F.start, L.start_final_tid};
+    P.W = EvalWeightsD{h->d_stw.p, h->d_ssw.p, h->d_sfw.p};
+    P.vtw = h->d_vtw.p; P.vew = h->d_vew.p; P.slot_emis = h->d_slot_emis.p; P.slot_final = h->d_slot_final.p;
+    P.C = CorpusD{h->d_tokens.p, h->d_offs.p, h->d_p.p, d_ord, n_ord};
+    P.max_len = std::max(h->max_len, 1);
+    P.n = n; P.key0 = (uint32_t)seed; P.key1 = (uint32_t)(seed >> 32);
+    P.logw = h->d_vlogw.p; P.logq = h->d_vlogw.p + (size_t)h->n_strings * n;
+    P.trans_edge = h->d_vtrans.p; P.emis_edge = h->d_vemis.p;
+    const bool warp = L.max_cand <= 32;
+    const int nt = warp ? 256 : std::max(64, (L.max_cand + 31) / 32 * 32);
+    const int per_cta = warp ? nt / 32 : 1;                                   // strings in flight per CTA
+    P.pitch = warp ? 32 : nt;
+    const size_t slab_bytes = (size_t)P.max_len * P.pitch * 8 * per_cta;     // per CTA
+    long long grid = (long long)h->sm_count * (warp ? 8 : std::max(1, std::min(4, 1024 / nt)));
+    grid = std::min<long long>(grid, (n_ord + per_cta - 1) / per_cta);
+    grid = std::max<long long>(1, std::min<long long>(grid, (long long)(4 * kViterbiSlabBudget / slab_bytes)));
+    const size_t need = (size_t)grid * per_cta * P.max_len * P.pitch;
+    if (h->d_sslab.n < need) CK(h->d_sslab.alloc(need));
+    P.slab = h->d_sslab.p;
+    const size_t smem = (size_t)2 * nt * 8 + 32 * 8 + 32 * 4;
+    if (warp) k3_sample<true><<<(unsigned)grid, nt, smem, h->stream>>>(P);
+    else k3_sample<false><<<(unsigned)grid, nt, smem, h->stream>>>(P);
+    h->launches++;
+    return WFSA_OK;
+}
+
 // Over one order list without fast tables, step counts (d_voff == nullptr) or the steps: kg_fwdbwd<MODE_VITERBI> in g_batch
-// batches (k = 1), else kg_nbest in batches of g_batch / k strings, whose lists take k times a string's scratch
-static void viterbi_generic_list(wfsa_dev* h, const int32_t* d_ord, int64_t n_ord, const int64_t* d_voff, int k)
+// batches (k = 1), else kg_nbest in batches of g_batch / k strings, whose lists take k times a string's scratch; with smp
+// kg_sample in g_batch batches (k draws per string)
+static void viterbi_generic_list(wfsa_dev* h, const int32_t* d_ord, int64_t n_ord, const int64_t* d_voff, int k,
+                                 const SampleSpec* smp = nullptr)
 {
     const HostFsa& F = h->fsa;
     GenericParams P{};
     P.G = GenericTablesD{h->d_emis_row.p, h->d_emis_tok_off.p, h->d_emis_tok.p, h->d_trans_row.p, h->d_trans_dst.p,
                          h->d_eps_order.p, F.n_states, F.n_trans(), F.start, F.end};
     P.C = CorpusD{h->d_tokens.p, h->d_offs.p, h->d_p.p, d_ord, n_ord};
-    P.scratch = k > 1 && h->g_batch < k ? h->d_nscratch.p : h->d_gscratch.p; P.max_len = h->max_len;
+    P.scratch = !smp && k > 1 && h->g_batch < k ? h->d_nscratch.p : h->d_gscratch.p; P.max_len = h->max_len;
     P.ltw = h->d_vtw.p; P.lew = h->d_vew.p; P.O.logq = h->d_vlogw.p;
     P.vit_cnt = h->d_vcnt.p; P.vit_off = d_voff; P.vit_trans = h->d_vtrans.p; P.vit_emis = h->d_vemis.p;
-    const long long batch = std::max<long long>(1, h->g_batch / k);
+    const long long batch = smp ? h->g_batch : std::max<long long>(1, h->g_batch / k);
     for (long long first = 0; first < n_ord; first += batch) {
         P.first = first; P.count = std::min<long long>(batch, n_ord - first);
-        if (k == 1) kg_fwdbwd<MODE_VITERBI><<<(unsigned)((P.count + 127) / 128), 128, 0, h->stream>>>(P);
+        if (smp) kg_sample<<<(unsigned)((P.count + 127) / 128), 128, 0, h->stream>>>(P, k, (uint32_t)smp->seed, (uint32_t)(smp->seed >> 32),
+                                                                                    h->d_vlogw.p + (size_t)h->n_strings * k);
+        else if (k == 1) kg_fwdbwd<MODE_VITERBI><<<(unsigned)((P.count + 127) / 128), 128, 0, h->stream>>>(P);
         else kg_nbest<<<(unsigned)((P.count + 127) / 128), 128, 0, h->stream>>>(P, k);
         h->launches++;
     }
 }
 
-// wfsa_dev_viterbi (k = 1: k3_viterbi, kg_fwdbwd<MODE_VITERBI>) and wfsa_dev_nbest (k3_nbest, kg_nbest); path i = s * k + r
-static int decode_paths(wfsa_dev* h, const double* x, int k, double* logw, int64_t* path_off)
+// wfsa_dev_viterbi (k = 1: k3_viterbi, kg_fwdbwd<MODE_VITERBI>), wfsa_dev_nbest (k3_nbest, kg_nbest) and, with smp,
+// wfsa_dev_sample (k draws: k3_sample, kg_sample); path i = s * k + r
+static int decode_paths(wfsa_dev* h, const double* x, int k, double* logw, int64_t* path_off, const SampleSpec* smp = nullptr)
 {
     CK(cudaSetDevice(h->device));
     h->v_done = false;
@@ -2115,25 +2165,43 @@ static int decode_paths(wfsa_dev* h, const double* x, int k, double* logw, int64
         CK(h->d_vtw.alloc(std::max(F.n_trans(), 1))); CK(h->d_vew.alloc(std::max(F.n_emis(), 1)));
         CK(h->d_vsw.alloc(std::max(n_slots, 1))); CK(h->d_vfw.alloc(std::max(n_slots, 1)));
     }
-    if (h->d_vlogw.n < (size_t)std::max<int64_t>(np, 1)) {
-        CK(h->d_vlogw.alloc((size_t)std::max<int64_t>(np, 1)));
-        if (!L.ok) { CK(h->d_vcnt.alloc((size_t)std::max<int64_t>(np, 1))); CK(h->d_voff.alloc((size_t)np + 1)); }
+    const int64_t nw = np + (smp ? ns : 0);                                 // sampling: log q behind the draws' logw
+    if (h->d_vlogw.n < (size_t)std::max<int64_t>(nw, 1)) CK(h->d_vlogw.alloc((size_t)std::max<int64_t>(nw, 1)));
+    if (!L.ok && h->d_vcnt.n < (size_t)std::max<int64_t>(np, 1)) {
+        CK(h->d_vcnt.alloc((size_t)std::max<int64_t>(np, 1))); CK(h->d_voff.alloc((size_t)np + 1));
     }
-    if (L.ok && h->d_vtrans.n < (size_t)(k * (h->n_tokens + ns))) {       // fast tables: len + 1 steps per path, padded
-        CK(h->d_vtrans.alloc((size_t)std::max<int64_t>(k * (h->n_tokens + ns), 1)));
-        CK(h->d_vemis.alloc((size_t)std::max<int64_t>(k * (h->n_tokens + ns), 1)));
+    if (smp && !h->d_stw.p) {
+        CK(h->d_stw.alloc(std::max(F.n_trans(), 1)));
+        CK(h->d_ssw.alloc(std::max(n_slots, 1))); CK(h->d_sfw.alloc(std::max(n_slots, 1)));
     }
-    if (!L.ok && k > 1 && h->g_batch < k) {                                 // kg_nbest needs room for one string's k lists
+    const int64_t padded = k * (h->n_tokens + ns);
+    if (L.ok && h->d_vtrans.n < (size_t)padded) {                           // fast tables: len + 1 steps per path, padded
+        if (h->d_vtrans.alloc((size_t)padded) != cudaSuccess || h->d_vemis.alloc((size_t)padded) != cudaSuccess) {
+            h->d_vtrans.release(); h->d_vemis.release();
+            cudaGetLastError();
+            return set_err(h, WFSA_ERR_NOMEM, "cannot allocate the step buffer of " + std::to_string(k) + " x (" +
+                                                  std::to_string(h->n_tokens) + " symbols + " + std::to_string(ns) +
+                                                  " strings) = " + std::to_string(padded) + " steps (8 bytes each)");
+        }
+    }
+    if (!L.ok && !smp && k > 1 && h->g_batch < k) {                         // kg_nbest needs room for one string's k lists
         const size_t per = (size_t)2 * (h->max_len + 1) * F.n_states * k;
         if (h->d_nscratch.n < per) CK(h->d_nscratch.alloc(per));
     }
     if (h->n > 0) CK(cudaMemcpyAsync(h->d_vx.p, x, (size_t)h->n * 8, cudaMemcpyHostToDevice, st));
-    const long long total = (long long)F.n_trans() + F.n_emis() + n_slots + np;
+    const long long total = (long long)F.n_trans() + F.n_emis() + n_slots + nw;
     if (total > 0) {
-        k_maxplus_weights<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(F.n_trans(), F.n_emis(), n_slots, (long long)np,
+        k_maxplus_weights<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(F.n_trans(), F.n_emis(), n_slots, (long long)nw,
                                                                          h->d_trans_tp.p, h->d_emis_tp.p, h->d_slot_emis.p,
                                                                          h->d_slot_final.p, h->d_vx.p, h->d_vtw.p, h->d_vew.p,
                                                                          h->d_vsw.p, h->d_vfw.p, h->d_vlogw.p);
+        h->launches++;
+    }
+    const long long nlin = (long long)F.n_trans() + F.n_emis() + n_slots;
+    if (smp && nlin > 0) {              // linear weights as the evaluation builds them (its log weights are k_maxplus_weights')
+        k_weights<<<(unsigned)((nlin + 255) / 256), 256, 0, st>>>(F.n_trans(), F.n_emis(), n_slots, h->d_trans_tp.p, h->d_emis_tp.p,
+                                                                  h->d_slot_emis.p, h->d_slot_final.p, h->d_vx.p, 0, h->d_stw.p,
+                                                                  h->d_ssw.p, h->d_sfw.p, h->d_vtw.p, h->d_vew.p);
         h->launches++;
     }
     // the strings that take part, as in the rmin sweep: the segmented and the batched kernel keep all of them in d_order
@@ -2143,19 +2211,21 @@ static int decode_paths(wfsa_dev* h, const double* x, int k, double* logw, int64
     std::vector<int32_t> cnt;
     if (L.ok) {
         for (int i = 0; i < 2; ++i) {
-            const int rc = k == 1 ? viterbi_fast_list(h, lists[i], counts[i]) : nbest_fast_list(h, lists[i], counts[i], k);
+            const int rc = smp ? sample_fast_list(h, lists[i], counts[i], k, smp->seed)
+                         : k == 1 ? viterbi_fast_list(h, lists[i], counts[i]) : nbest_fast_list(h, lists[i], counts[i], k);
             if (rc != WFSA_OK) return rc;
         }
     } else {
         // step counts first (they vary with empty and multi-token emissions), then their prefix sum, then the steps
         if (np) CK(cudaMemsetAsync(h->d_vcnt.p, 0, (size_t)np * 4, st));
-        for (int i = 0; i < 2; ++i) if (counts[i] > 0) viterbi_generic_list(h, lists[i], counts[i], nullptr, k);
+        for (int i = 0; i < 2; ++i) if (counts[i] > 0) viterbi_generic_list(h, lists[i], counts[i], nullptr, k, smp);
         cnt.resize((size_t)np);
         if (np) CK(cudaMemcpyAsync(cnt.data(), h->d_vcnt.p, (size_t)np * 4, cudaMemcpyDeviceToHost, st));
         CK(cudaStreamSynchronize(st));
         CK(cudaGetLastError());
     }
     if (np) CK(cudaMemcpyAsync(logw, h->d_vlogw.p, (size_t)np * 8, cudaMemcpyDeviceToHost, st));
+    if (smp && smp->logq && ns) CK(cudaMemcpyAsync(smp->logq, h->d_vlogw.p + np, (size_t)ns * 8, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
     CK(cudaGetLastError());
     path_off[0] = 0;
@@ -2170,7 +2240,7 @@ static int decode_paths(wfsa_dev* h, const double* x, int k, double* logw, int64
             CK(h->d_vtrans.alloc((size_t)std::max<int64_t>(steps, 1))); CK(h->d_vemis.alloc((size_t)std::max<int64_t>(steps, 1)));
         }
         CK(cudaMemcpyAsync(h->d_voff.p, path_off, (size_t)(np + 1) * 8, cudaMemcpyHostToDevice, st));
-        for (int i = 0; i < 2; ++i) if (counts[i] > 0) viterbi_generic_list(h, lists[i], counts[i], h->d_voff.p, k);
+        for (int i = 0; i < 2; ++i) if (counts[i] > 0) viterbi_generic_list(h, lists[i], counts[i], h->d_voff.p, k, smp);
         CK(cudaStreamSynchronize(st));
         CK(cudaGetLastError());
     }
@@ -2196,10 +2266,19 @@ extern "C" int wfsa_dev_nbest(wfsa_dev* h, const double* x, int32_t k, double* l
     return decode_paths(h, x, k, logw, path_off);
 }
 
+extern "C" int wfsa_dev_sample(wfsa_dev* h, const double* x, int32_t n, uint64_t seed, double* logw, double* logq, int64_t* path_off)
+{
+    if (!h || !logw || !path_off || n < 1 || n > kSampleMax) return set_err(h, WFSA_ERR_INVALID, "sample: bad arguments (n: 1..256)");
+    if (h->n < 0) return set_err(h, WFSA_ERR_STATE, "sample before set_param_map");
+    if (!x && h->n > 0) return set_err(h, WFSA_ERR_INVALID, "sample: bad arguments");
+    const SampleSpec smp{seed, logq};
+    return decode_paths(h, x, n, logw, path_off, &smp);
+}
+
 extern "C" int wfsa_dev_viterbi_paths(wfsa_dev* h, int32_t* trans_edge, int32_t* emis_edge)
 {
     if (!h || !trans_edge || !emis_edge) return set_err(h, WFSA_ERR_INVALID, "viterbi_paths: bad arguments");
-    if (!h->v_done) return set_err(h, WFSA_ERR_STATE, "viterbi_paths before viterbi or nbest");
+    if (!h->v_done) return set_err(h, WFSA_ERR_STATE, "viterbi_paths before viterbi, nbest or sample");
     CK(cudaSetDevice(h->device));
     const int64_t ns = h->n_strings, k = h->v_k, np = ns * k;
     const std::vector<int64_t>& po = h->h_vpath_off;

@@ -6,6 +6,7 @@
 #include <memory>
 #include <sstream>
 
+#include "../csrc/philox.hpp"
 #include "fsa.hpp"
 #include "learner.hpp"
 
@@ -55,6 +56,11 @@ static void describe_fsa(std::ostringstream& o, const Fsa& fsa, const std::vecto
         }
     }
     o << ']';
+}
+
+extern "C" void wfsa_philox4x32_10(const uint32_t ctr[4], const uint32_t key[2], uint32_t out[4])
+{
+    wfsa::philox4x32_10(ctr, key, out);
 }
 
 extern "C" int wfsa_host_kkt_solve(int32_t n, int32_t k, const double* expx, const double* lambda, const int32_t* ccol, const double* rhs,

@@ -235,16 +235,23 @@ const std::vector<double>& Learner::LogQ()
     return logq_cache;
 }
 
-void Learner::Decode(Decoding& d, int k)
+void Learner::Decode(Decoding& d, int k) { DecodePaths(d, k, false, 0); }
+
+void Learner::Sample(Decoding& d, int n, uint64_t seed) { DecodePaths(d, n, true, seed); }
+
+void Learner::DecodePaths(Decoding& d, int k, bool sample, uint64_t seed)
 {
     const size_t ns = shard_words.size(), np = ns * (size_t)k;
     d.k = k;
     d.logw.assign(std::max<size_t>(np, 1), 0.0); d.logq.assign(std::max<size_t>(ns, 1), 0.0); d.path_off.assign(np + 1, 0);
-    double ll = 0.0;
-    std::vector<double> g(std::max(GetNumberOfParameters(), 1));
-    check(wfsa_dev_eval(dev, _x.data(), &ll, d.logq.data(), g.data()), "wfsa_dev_eval");
-    if (k == 1) check(wfsa_dev_viterbi(dev, _x.data(), d.logw.data(), d.path_off.data()), "wfsa_dev_viterbi");
-    else check(wfsa_dev_nbest(dev, _x.data(), k, d.logw.data(), d.path_off.data()), "wfsa_dev_nbest");
+    if (sample) check(wfsa_dev_sample(dev, _x.data(), k, seed, d.logw.data(), d.logq.data(), d.path_off.data()), "wfsa_dev_sample");
+    else {
+        double ll = 0.0;
+        std::vector<double> g(std::max(GetNumberOfParameters(), 1));
+        check(wfsa_dev_eval(dev, _x.data(), &ll, d.logq.data(), g.data()), "wfsa_dev_eval");
+        if (k == 1) check(wfsa_dev_viterbi(dev, _x.data(), d.logw.data(), d.path_off.data()), "wfsa_dev_viterbi");
+        else check(wfsa_dev_nbest(dev, _x.data(), k, d.logw.data(), d.path_off.data()), "wfsa_dev_nbest");
+    }
     d.trans_edge.assign(std::max<int64_t>(d.path_off[np], 1), 0); d.emis_edge.assign(d.trans_edge.size(), 0);
     check(wfsa_dev_viterbi_paths(dev, d.trans_edge.data(), d.emis_edge.data()), "wfsa_dev_viterbi_paths");
     d.logw.resize(np); d.logq.resize(ns); d.trans_edge.resize(d.path_off[np]); d.emis_edge.resize(d.path_off[np]);

@@ -88,9 +88,13 @@ public:
     // inside is collective with several ranks)
     struct Decoding { int k = 1; std::vector<double> logw, logq; std::vector<int64_t> path_off; std::vector<int32_t> trans_edge, emis_edge; };
     void Decode(Decoding& d, int k = 1);
+    // n independent draws from the path posterior of every string of this shard at the current x (wfsa_dev_sample; path
+    // s * n + r is draw r of string s), with log q_s from the sampler; local to the shard, no evaluation
+    void Sample(Decoding& d, int n, uint64_t seed);
 
 protected:
     virtual void FinalizeCallback() {}
+    void DecodePaths(Decoding& d, int k, bool sample, uint64_t seed);
     virtual void InitCallback(int) {}
     void LambdaUpdate(double* lstep, double* l, double eta, bool exponential) const;   // src/Learner.cpp:438-462
     void EvalAt(const double* x);            // device evaluation: loglik, grad

@@ -7,7 +7,7 @@
 // --gpus N: one process per GPU (forked before anything touches CUDA), corpus cut into N ranges of equal symbol count, the
 // same optimiser loop on every rank with loglik / gradient / H_f summed over the ranks inside the backend; rank 0 reports.
 // --viterbi FILE: the most probable path of every corpus string with the final weights; --nbest K FILE: the K most
-// probable paths (write_paths).
+// probable paths; --sample N FILE [--seed S]: N draws from the path posterior of every corpus string (write_paths).
 #include <cfloat>
 #include <cmath>
 #include <cstdio>
@@ -84,11 +84,14 @@ static void print_paths(const Fsa& fsa, const Corpus& corpus, bool bfs)
 // empty path for a word without a path.
 // --nbest K FILE (nbest = K): min(K, paths) lines per corpus string, in corpus order and by rank,
 // word TAB rank TAB ln w(pi) TAB w(pi)/q_s TAB path,  rank from 1 (wfsa_dev_nbest); "0", "-inf", 0 and an empty path for a
-// word without a path.
-static void write_paths(const std::string& filename, const Fsa& fsa, const Corpus& corpus, Learner& learner, int nbest = 0)
+// word without a path.  --sample N FILE (nbest = N, sample): the same columns with the draw (from 1) in place of the rank,
+// N lines per corpus string (wfsa_dev_sample with seed).
+static void write_paths(const std::string& filename, const Fsa& fsa, const Corpus& corpus, Learner& learner, int nbest = 0,
+                        bool sample = false, uint64_t seed = 0)
 {
     Learner::Decoding d;
-    learner.Decode(d, nbest ? nbest : 1);
+    if (sample) learner.Sample(d, nbest, seed);
+    else learner.Decode(d, nbest ? nbest : 1);
     const size_t k = (size_t)d.k;
     FILE* out = fopen(filename.c_str(), "w");
     if (!out) throw MyError("Unable to open output file \"" + filename + "\" for writing!");
@@ -172,13 +175,18 @@ static void usage()
         "                             -e 0 -s decodes with the automaton file's own weights\n"
         "  --nbest K FILE             as --viterbi, the K (1..16) most probable paths of every corpus string, best first:\n"
         "                             word, rank, ln w(path), w(path)/q(word), path; a word without a path gets one line\n"
-        "                             with rank 0 (one GPU)\n";
+        "                             with rank 0 (one GPU)\n"
+        "  --sample N FILE            N (1..256) independent draws from the posterior w(path)/q(word) of the paths of every\n"
+        "                             corpus string with the final weights: word, draw, ln w(path), w(path)/q(word), path;\n"
+        "                             a word without a path gets one line with draw 0 (one GPU)\n"
+        "  --seed S                   seed of --sample (default 0): the same seed gives the same draws\n";
 }
 
 int main(int argc, const char* argv[])
 {
-    std::string automaton_filename, corpus_filename, output_filename, viterbi_filename, nbest_filename, optimizer = "Hessian";
-    int epochs = 20, initflags = 0, device = 0, gpus = 1, nbest = 0;
+    std::string automaton_filename, corpus_filename, output_filename, viterbi_filename, nbest_filename, sample_filename, optimizer = "Hessian";
+    int epochs = 20, initflags = 0, device = 0, gpus = 1, nbest = 0, sample = 0;
+    uint64_t seed = 0;
     bool normalize = false, print = false, print_recognize = false, suppress = false, evaluate = false, initx = false, full = false;
     int recognize = 0;
     double eta = 1.0, tolerance = 1e-6;
@@ -221,6 +229,20 @@ int main(int argc, const char* argv[])
             nbest = (int)K;
             nbest_filename = next();
         }
+        else if (is(a, {"--sample"})) {
+            const char* v = next();
+            char* end = nullptr;
+            const long N = std::strtol(v, &end, 10);
+            if (end == v || *end || N < 1 || N > 256) { std::cerr << "--sample N must be between 1 and 256" << std::endl; return 1; }
+            sample = (int)N;
+            sample_filename = next();
+        }
+        else if (is(a, {"--seed"})) {
+            const char* v = next();
+            char* end = nullptr;
+            seed = std::strtoull(v, &end, 10);
+            if (end == v || *end || *v == '-') { std::cerr << "--seed S must be an integer between 0 and 2^64 - 1" << std::endl; return 1; }
+        }
         else if (is(a, {"-m", "--matrices", "--matrix"})) { next(); std::cerr << "-m is not supported: the DP backend has no path matrices to cache" << std::endl; return 1; }
         else { std::cerr << "Unknown argument \"" << a << "\"!" << std::endl; return 1; }
     }
@@ -230,6 +252,10 @@ int main(int argc, const char* argv[])
     }
     if (nbest && gpus > 1) {
         std::cerr << "--nbest decodes on one GPU: it cannot be combined with --gpus " << gpus << std::endl;
+        return 1;
+    }
+    if (sample && gpus > 1) {
+        std::cerr << "--sample draws on one GPU: it cannot be combined with --gpus " << gpus << std::endl;
         return 1;
     }
     // --gpus N: fork the other ranks before CUDA is touched.  Rank 0 (this process) creates the communicator id and hands
@@ -355,6 +381,7 @@ int main(int argc, const char* argv[])
         }
         if (!viterbi_filename.empty()) write_paths(viterbi_filename, fsa, corpus, *learner);
         if (nbest) write_paths(nbest_filename, fsa, corpus, *learner, nbest);
+        if (sample) write_paths(sample_filename, fsa, corpus, *learner, sample, true, seed);
         if (!suppress && rank == 0) {
             FILE* outf = output_filename.empty() ? stdout : fopen(output_filename.c_str(), "w");
             if (!outf) throw MyError("Unable to open output file \"" + output_filename + "\" for writing!");

@@ -18,14 +18,14 @@ UNIQUE_ID_BYTES = 128
 DEV_SYMBOLS = [
     "wfsa_dev_create", "wfsa_dev_structure", "wfsa_dev_set_param_map", "wfsa_dev_eval", "wfsa_dev_upload_x",
     "wfsa_dev_eval_launch", "wfsa_dev_eval_fetch", "wfsa_dev_sync", "wfsa_dev_set_path_blocks", "wfsa_dev_hessian",
-    "wfsa_dev_viterbi", "wfsa_dev_viterbi_paths", "wfsa_dev_nbest",
+    "wfsa_dev_viterbi", "wfsa_dev_viterbi_paths", "wfsa_dev_nbest", "wfsa_dev_sample",
     "wfsa_dev_comm_unique_id", "wfsa_dev_comm_init", "wfsa_dev_allreduce_f64", "wfsa_dev_timer_begin", "wfsa_dev_timer_begin_steps",
     "wfsa_dev_timer_end", "wfsa_dev_timer_kernel_ms", "wfsa_dev_timer_split_ms", "wfsa_dev_timer_step_ms", "wfsa_dev_timer_phase_ms", "wfsa_dev_eval6_phases", "wfsa_dev_l2_flush", "wfsa_dev_rank_barrier", "wfsa_dev_get_info", "wfsa_dev_destroy", "wfsa_dev_held_bytes", "wfsa_dev_last_error",
     "wfsa_dev_version", "wfsa_lattice_compile", "wfsa_segmented_compile", "wfsa_segmented_get",
     "wfsa_segmented_free",
 ]
 HOST_SYMBOLS = [
-    "wfsa_host_parse", "wfsa_host_last_error", "wfsa_host_kkt_solve", "wfsa_session_create", "wfsa_session_destroy", "wfsa_session_error",
+    "wfsa_host_parse", "wfsa_host_last_error", "wfsa_host_kkt_solve", "wfsa_philox4x32_10", "wfsa_session_create", "wfsa_session_destroy", "wfsa_session_error",
     "wfsa_session_describe", "wfsa_session_n", "wfsa_session_k", "wfsa_session_n_recognised_local", "wfsa_session_init",
     "wfsa_session_eval", "wfsa_session_hessian", "wfsa_session_step", "wfsa_session_halt", "wfsa_session_get_x",
     "wfsa_session_renormalize", "wfsa_session_result", "wfsa_session_dump", "wfsa_session_backend",
@@ -33,6 +33,7 @@ HOST_SYMBOLS = [
 
 I32P = C.POINTER(C.c_int32)
 I64P = C.POINTER(C.c_int64)
+U32P = C.POINTER(C.c_uint32)
 F64P = C.POINTER(C.c_double)
 U8P = C.POINTER(C.c_uint8)
 
@@ -136,6 +137,9 @@ def lib():
         L.wfsa_dev_viterbi.argtypes = [C.c_void_p, F64P, F64P, I64P]
         L.wfsa_dev_viterbi_paths.argtypes = [C.c_void_p, I32P, I32P]
         L.wfsa_dev_nbest.argtypes = [C.c_void_p, F64P, C.c_int32, F64P, I64P]
+        L.wfsa_dev_sample.argtypes = [C.c_void_p, F64P, C.c_int32, C.c_uint64, F64P, F64P, I64P]
+        L.wfsa_philox4x32_10.argtypes = [U32P, U32P, U32P]
+        L.wfsa_philox4x32_10.restype = None
         L.wfsa_dev_comm_unique_id.argtypes = [C.c_void_p]
         L.wfsa_dev_comm_init.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int]
         L.wfsa_dev_allreduce_f64.argtypes = [C.c_void_p, F64P, C.c_int, C.c_int]
@@ -383,6 +387,12 @@ class Device:
         logw, off, tr, em = _viterbi(self.L, self.h, x, self.n_strings, k)
         return logw.reshape(self.n_strings, k), off, tr, em
 
+    def sample(self, x, n, seed=0):
+        """n independent draws from the path posterior of every string at x: (logw [n_strings, n], logq, path_off,
+        trans_edge, emis_edge); path i = s * n + r is draw r of string s, its steps [path_off[i], path_off[i+1]) as in viterbi,
+        logw[s, r] = -inf: string s has no path; logq[s] = log q_s from the sampler's forward sweep."""
+        return _sample(self.L, self.h, x, self.n_strings, n, seed)
+
     def timer_begin(self):
         self._ck(self.L.wfsa_dev_timer_begin(self.h))
 
@@ -447,6 +457,32 @@ class Device:
             self.close()
         except Exception:
             pass
+
+
+def _sample(L, h, x, n_strings, n, seed):
+    """wfsa_dev_sample, then the steps: (logw [n_strings, n], logq, path_off, trans_edge, emis_edge)."""
+    def ck(rc):
+        if rc != 0:
+            raise WfsaError(rc, L.wfsa_dev_last_error(h).decode())
+    x = np.ascontiguousarray(x, dtype=np.float64)
+    logw = np.zeros(max(n_strings * n, 1))
+    logq = np.zeros(max(n_strings, 1))
+    off = np.zeros(n_strings * n + 1, dtype=np.int64)
+    ck(L.wfsa_dev_sample(h, _p(x, F64P), n, seed, _p(logw, F64P), _p(logq, F64P), _p(off, I64P)))
+    steps = max(int(off[-1]), 1)
+    tr = np.zeros(steps, dtype=np.int32)
+    em = np.zeros(steps, dtype=np.int32)
+    ck(L.wfsa_dev_viterbi_paths(h, _p(tr, I32P), _p(em, I32P)))
+    return logw[:n_strings * n].reshape(n_strings, n), logq[:n_strings], off, tr[:off[-1]], em[:off[-1]]
+
+
+def philox4x32_10(ctr, key):
+    """The Philox4x32-10 block function of wfsa_dev_sample (wfsa_philox4x32_10): 4 words out of a 4-word counter and a 2-word
+    key."""
+    c = np.ascontiguousarray(ctr, dtype=np.uint32); k = np.ascontiguousarray(key, dtype=np.uint32)
+    out = np.zeros(4, dtype=np.uint32)
+    lib().wfsa_philox4x32_10(_p(c, U32P), _p(k, U32P), _p(out, U32P))
+    return out
 
 
 def _viterbi(L, h, x, n_strings, k=None):
@@ -551,6 +587,11 @@ class Session:
         ns = self.backend_info()["n_strings"]
         logw, off, tr, em = _viterbi(self.L, self.L.wfsa_session_backend(self.h), self.x() if x is None else x, ns, k)
         return logw.reshape(ns, k), off, tr, em
+
+    def sample(self, n, seed=0, x=None):
+        """Device.sample on the session's backend, at x or the current weights, for every string of this shard."""
+        return _sample(self.L, self.L.wfsa_session_backend(self.h), self.x() if x is None else x,
+                       self.backend_info()["n_strings"], n, seed)
 
     def backend_info(self):
         i = DevInfo()

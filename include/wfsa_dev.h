@@ -135,9 +135,12 @@ int wfsa_dev_set_path_blocks(wfsa_dev* h, const wfsa_path_blocks* blocks);
  *   - blocks set by wfsa_dev_set_path_blocks: from the blocks (Hf needs them on every kernel but the segmented one);
  *   - no blocks, Hf == NULL, any kernel: no enumeration -- a forward sweep in the (min, +) semiring over the lattice of the
  *     evaluation gives m_s = min_pi log w(pi), and r_s = exp(m_s - log q_s);
- *   - segmented kernel (6) without blocks: blocks and per-string minima from the compiled region types, the overflow
- *     strings by the sweep; when a region type has more than 2^20 paths an rmin-only call sweeps every string, a call
- *     with Hf returns WFSA_ERR_LIMIT.
+ *   - segmented kernel (6) without blocks: blocks and per-string minima from the compiled region types; the strings
+ *     that no type covers (more live lattice nodes than pool slots) add one block per segment of their lattice to H and
+ *     are taken into rmin by the sweep.  When a region type or such a segment has more than 2^20 paths an rmin-only call
+ *     sweeps every string, a call with Hf returns WFSA_ERR_LIMIT (never a partial H).
+ * H is summed in 64-bit fixed point whose range is sized from sum_b p_b * cmax_b^2 over the blocks of all ranks (cmax_b =
+ * largest |count| of block b); WFSA_ERR_LIMIT when that sum reaches 2^50.
  * Without blocks a call with Hf != NULL returns WFSA_ERR_STATE on the other kernels.  Collective with a communicator.
  * The (min, +) sweep gives the weight of the least probable path; the most probable path itself, of every string, comes
  * from wfsa_dev_viterbi below. */
@@ -285,9 +288,11 @@ int wfsa_lattice_compile(const wfsa_fsa_desc* fsa, const int32_t* trimmed, const
  * which: 0 rwords(u32) 1 rgoff(i64) 2 rgrows(i32) 3 typeW(f64) 4 swords(u32) 5 sgoff(i64) 6 sgref(i32)
  *        7 ksid(i32) 8 kp(f64) 9 overflow(i32) 10 rejected(i32) 11 const_acc(i64)
  *        12 stats(i64): types, region instances, instance edges, type edges, bridges, strings, host microseconds,
- *           path blocks omitted (1: a region type has more than 2^20 paths, so arrays 13-19 describe zero blocks)
+ *           path blocks omitted (1: a region type, or a segment of an overflow string, has more than 2^20 paths, so
+ *           arrays 13-19 describe zero blocks)
  *        13 path_off(i64) 14 col_off(i64) 15 val_off(i64) 16 cols(i32) 17 counts(f64) 18 p(f64) 19 type slot(i32): the path blocks
- *           wfsa_dev_hessian derives from the region types (layout of wfsa_path_blocks, p = weight of the type).  The
+ *           wfsa_dev_hessian derives from the region types (layout of wfsa_path_blocks, p = weight of the type), then one
+ *           block per segment with a choice of every overflow string (p = p_s, type slot -1).  The
  *           evaluation does not need them: a shard whose blocks cannot be built still compiles (wfsa_dev_hessian of such
  *           a shard returns WFSA_ERR_LIMIT).
  *        20 pwords(u32) 21 pgoff(i64): the reduction plan of the path-form groups (lattice.hpp, SegmentedCorpus::pwords) */

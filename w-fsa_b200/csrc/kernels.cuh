@@ -1114,7 +1114,7 @@ struct HessParams {
     double* rmin;                    // [1] smallest path posterior (atomicMin on bits)
     int n;
     double fx_scale;
-    const int32_t* __restrict__ blk_slot;   // blocks = region types: type slot of block b, or nullptr
+    const int32_t* __restrict__ blk_slot;   // blocks = region types: type slot of block b (-1: no type), or nullptr
     double* slot_lrmin;              // [type slots] log of the smallest path posterior of the type
 };
 
@@ -1157,8 +1157,10 @@ __global__ void __launch_bounds__(256) k5_hessian(const HessParams P)
         for (int l = lane; l < L; l += 32) { const double v = r[l] / z; r[l] = v; rm = fmin(rm, v); }
 #pragma unroll
         for (int o = 16; o; o >>= 1) rm = fmin(rm, __shfl_xor_sync(FULL, rm, o));
-        if (lane == 0 && P.rmin) atomicMin(reinterpret_cast<unsigned long long*>(P.rmin), (unsigned long long)__double_as_longlong(rm));
-        if (lane == 0 && P.blk_slot) P.slot_lrmin[P.blk_slot[b]] = log(rm);
+        // a block without a type slot (a segment of a string that no region type covers) leaves rmin to the caller's sweep
+        const int slot = P.blk_slot ? P.blk_slot[b] : 0;
+        if (lane == 0 && P.rmin && slot >= 0) atomicMin(reinterpret_cast<unsigned long long*>(P.rmin), (unsigned long long)__double_as_longlong(rm));
+        if (lane == 0 && P.blk_slot && slot >= 0) P.slot_lrmin[slot] = log(rm);
         __syncwarp();
         if (!P.H_fx) continue;                                 // rmin only (QuasiNewtonLearner's diagnostic column)
         // 8x8 output tiles; DMMA fragment layout (m8n8k4): A[row=lane/4][k=lane%4],

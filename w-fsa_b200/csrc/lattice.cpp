@@ -386,6 +386,72 @@ int compile_segments(const HostFsa& f, const LatticeArcs& A, const uint8_t* aliv
     return 1;
 }
 
+int segment_paths(const HostFsa& f, const LatticeArcs& A, const uint8_t* alive, const int32_t* tok, int len,
+                  size_t max_paths, LatticeScratch& S, const std::function<void(const std::vector<std::vector<int32_t>>&)>& emit)
+{
+    const int end_node = build_and_trim(f, A, alive, tok, len, S);
+    if (end_node < 0) return 0;
+    const int n_nodes = (int)S.npos.size(), n_e = (int)S.esrc.size();
+    S.kept.clear();
+    S.topo.assign(n_nodes, -1);
+    int nt = 0;
+    for (int e = 0; e < n_e; ++e) {
+        if (!S.coreach[S.edst[e]]) continue;
+        S.kept.push_back(e);
+        if (S.topo[S.esrc[e]] < 0) S.topo[S.esrc[e]] = nt++;
+    }
+    S.topo[end_node] = nt;
+    std::vector<int32_t>& first_out = S.nout;               // first kept edge of a node (the edges of a node are contiguous)
+    first_out.assign(n_nodes, -1);
+    for (int i = (int)S.kept.size() - 1; i >= 0; --i) first_out[S.esrc[S.kept[i]]] = i;
+    std::vector<std::vector<int32_t>> paths;
+    std::vector<int32_t>& stk = S.per_pos;                  // the current path as kept[] positions
+    // kept edges [b, e) between two consecutive cut nodes: every path from the entry to the exit (the dst of the last edge)
+    auto segment = [&](int b, int e) -> bool {
+        if (e - b == 1) return true;                        // a bridge: one path
+        const int exitn = S.edst[S.kept[e - 1]];
+        paths.clear();
+        stk.clear();
+        int node = S.esrc[S.kept[b]], next_edge = b;
+        for (;;) {
+            if (node == exitn) {
+                paths.emplace_back();
+                for (int i : stk) paths.back().push_back(S.earc[S.kept[i]]);
+                if (paths.size() > max_paths) return false;
+                next_edge = -1;                             // backtrack
+            }
+            if (next_edge >= 0 && next_edge < e && S.esrc[S.kept[next_edge]] == node) {
+                stk.push_back(next_edge);
+                node = S.edst[S.kept[next_edge]];
+                next_edge = node == exitn ? -1 : first_out[node];
+                continue;
+            }
+            if (stk.empty()) break;
+            const int last = stk.back();
+            stk.pop_back();
+            node = S.esrc[S.kept[last]];
+            next_edge = last + 1;
+        }
+        if (paths.size() >= 2) emit(paths);
+        return true;
+    };
+    const int nk = (int)S.kept.size();
+    int seg_begin = 0, maxdst = 0, cur = -1;
+    for (int i = 0; i < nk; ++i) {                          // the cut of compile_segments
+        const int ed = S.kept[i], sN = S.esrc[ed];
+        if (sN != cur) {
+            cur = sN;
+            if (S.topo[sN] == maxdst && i > seg_begin) {
+                if (!segment(seg_begin, i)) return -1;
+                seg_begin = i;
+            }
+        }
+        maxdst = std::max(maxdst, S.topo[S.edst[ed]]);
+    }
+    if (nk > seg_begin && !segment(seg_begin, nk)) return -1;
+    return 1;
+}
+
 namespace {
 inline uint64_t fnv1a(const uint32_t* w, size_t n)
 {

@@ -29,6 +29,7 @@
 //   PAD   0
 #pragma once
 #include <cstdint>
+#include <functional>
 #include <string>
 #include <memory>
 #include <vector>
@@ -109,6 +110,13 @@ struct SegString {                         // one string, compiled
 };
 int compile_segments(const HostFsa& f, const LatticeArcs& A, const uint8_t* arc_alive, const int32_t* tok, int len,
                      int n_slots, LatticeScratch& S, SegString& out);
+
+// The paths of every segment of one string, without a pool-slot limit: the trimmed lattice is cut at its cut nodes as
+// compile_segments cuts it, and `emit` receives, for each segment with at least two paths, the arcs of all its paths (in
+// DFS order).  Returns 1, 0 when the string has no accepting path, -1 when a segment has more than max_paths paths (the
+// segments before it have been emitted).  For the H_f blocks of strings that no region type covers.
+int segment_paths(const HostFsa& f, const LatticeArcs& A, const uint8_t* arc_alive, const int32_t* tok, int len,
+                  size_t max_paths, LatticeScratch& S, const std::function<void(const std::vector<std::vector<int32_t>>&)>& emit);
 
 struct SegmentedCorpus {
     // KR: region types in groups of 32 (one warp), word j of lane l of group g at rgoff[g] + j*32 + l;

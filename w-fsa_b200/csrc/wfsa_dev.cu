@@ -222,6 +222,7 @@ struct wfsa_dev {
     int64_t hb_blocks = -1, hb_paths = 0;
     // H_f from the compiled region types (no path enumeration per string): host copy of the KR arrays, kept by set_param_map
     std::vector<uint32_t> hrw; std::vector<int64_t> hrgoff; std::vector<int32_t> hrgrows; std::vector<double> hrW;
+    std::vector<int32_t> h_seg_overflow;       // strings that no region type covers: H_f blocks of their own segments
     std::vector<int32_t> h_ttp, h_etp;
     bool hb_from_types = false, hb_user = false;
     bool hb_types_failed = false;              // the region types of this parameter map have too many paths for blocks
@@ -1245,6 +1246,7 @@ extern "C" int wfsa_dev_set_param_map(wfsa_dev* h, const int32_t* trimmed, int32
         CK(cudaStreamSynchronize(h->stream));
         // the region types stay on the host as well: wfsa_dev_hessian derives its path blocks from them
         h->hrw = std::move(sc.rwords); h->hrgoff = std::move(sc.rgoff); h->hrgrows = std::move(sc.rgrows); h->hrW = std::move(sc.typeW);
+        h->h_seg_overflow = std::move(sc.overflow);
         h->h_ttp = ttp; h->h_etp = etp;
         if (!h->hb_user) h->hb_blocks = -1;
         h->hb_from_types = false; h->hb_types_failed = false;
@@ -1703,21 +1705,37 @@ static int upload_path_blocks(wfsa_dev* h, const std::vector<int64_t>& po, const
     CK(h->d_H.alloc(std::max<size_t>((size_t)h->n * h->n, 1)));
     CK(h->d_rmin.alloc(1));
     CK(cudaStreamSynchronize(h->stream));
-    // fixed-point scale of H: |H_jk| <= sum_s p_s * cmax^2 <= cmax^2 (p sums to <= 1 over all ranks)
-    double cmax = 1.0;
-    for (double c : counts) cmax = std::max(cmax, std::fabs(c));
-    long long v[2] = {(long long)std::ceil(cmax * cmax) + 1, (long long)local_error};
+    // fixed-point scale of H: a block adds p_b * Cov_b(c_j, c_k) to an entry, |Cov_b| <= cmax_b^2 (cmax_b = largest |count|
+    // of the block), so every single contribution and every entry of the sum over all blocks of all ranks is bounded by
+    // sum_b |p_b| cmax_b^2.  The block weights need not sum to 1: a type weighs all its instances, a string with several
+    // regions counts once per region.  The range 2^63 / fx = 2^(bits+2) is at least 4 (cmax^2 + 1), cmax over all blocks,
+    // as for blocks of one string each (p summing to at most 1), and at least twice that bound.
+    constexpr long long kRangeCap = 1ll << 50;
+    double bound = 0.0, cmax_all = 1.0;
+    for (int64_t b = 0; b < nb; ++b) {
+        double cmax = 0.0;
+        for (int64_t i = vo[b]; i < vo[b + 1]; ++i) cmax = std::max(cmax, std::fabs(counts[i]));
+        bound += std::fabs(p[b]) * cmax * cmax;
+        cmax_all = std::max(cmax_all, cmax);
+    }
+    long long v[3] = {bound < (double)kRangeCap ? (long long)std::ceil(bound) + 1 : kRangeCap, (long long)local_error,
+                      cmax_all * cmax_all < (double)kRangeCap ? (long long)std::ceil(cmax_all * cmax_all) + 1 : kRangeCap};
     if (h->comm) {         // every rank must see a failure of any rank BEFORE the all-reduce of H (a rank that returned early would leave the others waiting)
         long long* d = reinterpret_cast<long long*>(h->d_red.p);
-        CK(cudaMemcpyAsync(d, v, 16, cudaMemcpyHostToDevice, h->stream));
-        int rc = nccl_allreduce(h, d, 2, ncclInt64, ncclMax);
+        CK(cudaMemcpyAsync(d, v, 24, cudaMemcpyHostToDevice, h->stream));
+        int rc = nccl_allreduce(h, d, 2, ncclInt64, ncclSum);
+        if (rc == WFSA_OK) rc = nccl_allreduce(h, d + 2, 1, ncclInt64, ncclMax);
         if (rc != WFSA_OK) return rc;
-        CK(cudaMemcpyAsync(v, d, 16, cudaMemcpyDeviceToHost, h->stream));
+        CK(cudaMemcpyAsync(v, d, 24, cudaMemcpyDeviceToHost, h->stream));
         CK(cudaStreamSynchronize(h->stream));
     }
-    if (v[1]) return set_err(h, WFSA_ERR_LIMIT, local_error ? h->err : "H_f blocks: another rank could not build its path blocks");
+    if (v[1]) { h->hb_blocks = -1; return set_err(h, WFSA_ERR_LIMIT, local_error ? h->err : "H_f blocks: another rank could not build its path blocks"); }
     int bits = 1;
-    while ((1ll << bits) <= v[0] && bits < 50) ++bits;
+    while (bits <= 50 && ((1ll << bits) <= v[2] || (1ll << (bits + 1)) <= v[0])) ++bits;
+    if (bits > 50 || v[0] >= kRangeCap) {
+        h->hb_blocks = -1;
+        return set_err(h, WFSA_ERR_LIMIT, "H_f blocks: the sum over the blocks of p * (largest count)^2 reaches 2^50, beyond the fixed-point range of H");
+    }
     h->hb_fx_log2 = 61 - bits;
     h->hb_blocks = nb; h->hb_paths = po[nb];
     return WFSA_OK;
@@ -1747,6 +1765,8 @@ extern "C" int wfsa_dev_set_path_blocks(wfsa_dev* h, const wfsa_path_blocks* b)
 //     H_f = - sum_types W_type * Cov_type(c_j, c_k):
 // the blocks of k5_hessian are the distinct region types of the compiled corpus.  Path-form types are their own path
 // list; the paths of a DAG-form type are enumerated from its words (a region, not a string: bounded by max_paths).
+// Strings that no type covers add one block per segment (OverflowStrings below), under the same bound.  Past the bound
+// the blocks fail as a whole (B.fail): never a partial H.
 // Replaces the per-string BFS of Learner::BuildPaths feeding HessianLearner::ComputeHf (src/HessianLearner.cpp:498-547).
 struct TypeBlocks {
     std::vector<int64_t> po{0}, co{0}, vo{0};
@@ -1755,35 +1775,57 @@ struct TypeBlocks {
     std::string fail;
 };
 
+// Strings that no region type covers (more live nodes than pool slots: SegmentedCorpus::overflow) have blocks of their own:
+// one per segment with a choice, its paths enumerated from the string's trimmed lattice (segment_paths), weight p_s and no
+// type slot (-1).
+struct OverflowStrings {
+    const HostFsa* f;
+    const uint8_t* alive;                                 // [n_arcs]
+    const int32_t* tokens;
+    const int64_t* offs;
+    const double* p;
+    const std::vector<int32_t>* ids;
+};
+
 static void make_type_blocks(const LatticeArcs& A, const std::vector<int32_t>& ttp, const std::vector<int32_t>& etp,
                              const std::vector<uint32_t>& rw, const std::vector<int64_t>& rgoff, const std::vector<int32_t>& rgrows,
-                             const std::vector<double>& typeW, TypeBlocks& B)
+                             const std::vector<double>& typeW, const OverflowStrings& ov, TypeBlocks& B)
 {
     const int64_t n_rg = (int64_t)rgrows.size();
     const size_t max_paths = 1u << 20;
     std::vector<std::vector<int32_t>> paths;              // arcs of every path of the current type
-    auto emit = [&](int64_t slot, double W) {
-        std::map<int, int> colset;
-        std::vector<std::map<int, double>> hist(paths.size());
-        for (size_t q = 0; q < paths.size(); ++q)
-            for (int32_t a : paths[q]) {
-                const int tp = ttp[A.arc_tid[a]], ep = A.arc_eid[a] < 0 ? -1 : etp[A.arc_eid[a]];
-                if (tp >= 0) { hist[q][tp] += 1.0; colset[tp] = 0; }
-                if (ep >= 0) { hist[q][ep] += 1.0; colset[ep] = 0; }
-            }
-        std::vector<int> keep;                             // columns whose count differs between the paths (src/HessianLearner.cpp:409-443)
-        for (const auto& kv : colset) {
-            const int j = kv.first;
-            auto f0 = hist[0].find(j);
-            const double c0 = f0 == hist[0].end() ? 0.0 : f0->second;
+    std::vector<int32_t> col_of, bcols;                  // parameter -> column of the current block (-1: none), its columns
+    std::vector<double> dense;                            // paths x columns of the current block
+    auto emit = [&](const std::vector<std::vector<int32_t>>& pl, int64_t slot, double W) {
+        auto each_param = [&](int32_t a, auto&& fn) {
+            const int tp = ttp[A.arc_tid[a]], ep = A.arc_eid[a] < 0 ? -1 : etp[A.arc_eid[a]];
+            if (tp >= 0) fn(tp);
+            if (ep >= 0) fn(ep);
+        };
+        bcols.clear();
+        for (const auto& pa : pl)
+            for (int32_t a : pa)
+                each_param(a, [&](int j) {
+                    if (j >= (int)col_of.size()) col_of.resize((size_t)j + 1, -1);
+                    if (col_of[j] < 0) { col_of[j] = 0; bcols.push_back(j); }
+                });
+        std::sort(bcols.begin(), bcols.end());
+        const size_t D = bcols.size();
+        for (size_t k = 0; k < D; ++k) col_of[bcols[k]] = (int32_t)k;
+        dense.assign(pl.size() * D, 0.0);
+        for (size_t q = 0; q < pl.size(); ++q)
+            for (int32_t a : pl[q]) each_param(a, [&](int j) { dense[q * D + col_of[j]] += 1.0; });
+        std::vector<size_t> keep;                          // columns whose count differs between the paths (src/HessianLearner.cpp:409-443)
+        for (size_t k = 0; k < D; ++k) {
             bool same = true;
-            for (const auto& hq : hist) { auto f = hq.find(j); if ((f == hq.end() ? 0.0 : f->second) != c0) { same = false; break; } }
-            if (!same) keep.push_back(j);
+            for (size_t q = 1; q < pl.size() && same; ++q) same = dense[q * D + k] == dense[k];
+            if (!same) keep.push_back(k);
         }
-        for (int j : keep) B.cols.push_back(j);
-        for (const auto& hq : hist)
-            for (int j : keep) { auto f = hq.find(j); B.counts.push_back(f == hq.end() ? 0.0 : f->second); }
-        B.po.push_back(B.po.back() + (int64_t)paths.size());
+        for (int j : bcols) col_of[j] = -1;
+        for (size_t k : keep) B.cols.push_back(bcols[k]);
+        for (size_t q = 0; q < pl.size(); ++q)
+            for (size_t k : keep) B.counts.push_back(dense[q * D + k]);
+        B.po.push_back(B.po.back() + (int64_t)pl.size());
         B.co.push_back((int64_t)B.cols.size());
         B.vo.push_back((int64_t)B.counts.size());
         B.bp.push_back(W);
@@ -1842,15 +1884,28 @@ static void make_type_blocks(const LatticeArcs& A, const std::vector<int32_t>& t
                     stack.push_back({ed.first, 0});
                 }
             }
-            if (B.fail.empty() && paths.size() >= 2) emit(g * 32 + l, W);
+            if (B.fail.empty() && paths.size() >= 2) emit(paths, g * 32 + l, W);
         }
+    }
+    LatticeScratch S;
+    for (size_t i = 0; i < ov.ids->size() && B.fail.empty(); ++i) {
+        const int32_t s = (*ov.ids)[i];
+        if (!(ov.p[s] > 0.0)) continue;
+        const int rc = segment_paths(*ov.f, A, ov.alive, ov.tokens + ov.offs[s], (int)(ov.offs[s + 1] - ov.offs[s]), max_paths, S,
+                                     [&](const std::vector<std::vector<int32_t>>& seg) { emit(seg, -1, ov.p[s]); });
+        if (rc < 0) B.fail = "H_f blocks: a segment of string " + std::to_string(s) + " (more live nodes than pool slots) has more than 2^20 paths";
     }
 }
 
 static int build_type_blocks(wfsa_dev* h)
 {
+    const LatticeArcs& A = h->larcs;
+    std::vector<uint8_t> alive((size_t)A.n_arcs);          // as wfsa_dev_set_param_map compiled the strings
+    for (int a = 0; a < A.n_arcs; ++a)
+        alive[a] = h->h_ttp[A.arc_tid[a]] != -2 && (A.arc_eid[a] < 0 || h->h_etp[A.arc_eid[a]] != -2);
+    const OverflowStrings ov{&h->fsa, alive.data(), h->h_tokens.data(), h->h_offs.data(), h->h_p.data(), &h->h_seg_overflow};
     TypeBlocks B;
-    make_type_blocks(h->larcs, h->h_ttp, h->h_etp, h->hrw, h->hrgoff, h->hrgrows, h->hrW, B);
+    make_type_blocks(A, h->h_ttp, h->h_etp, h->hrw, h->hrgoff, h->hrgrows, h->hrW, ov, B);
     if (!B.fail.empty()) h->err = B.fail;
     CK(h->d_type_lrmin.alloc(h->hrgrows.size() * 32 + 1));
     CK(cudaMemsetAsync(h->d_type_lrmin.p, 0, h->d_type_lrmin.n * 8, h->stream));
@@ -2703,7 +2758,8 @@ extern "C" int wfsa_segmented_compile(const wfsa_fsa_desc* fd, const wfsa_corpus
         std::vector<int32_t> ttp(f.n_trans()), etp(f.n_emis());
         for (int t = 0; t < f.n_trans(); ++t) ttp[t] = f.trans_param[t] < 0 ? -1 : (trimmed ? trimmed[f.trans_param[t]] : f.trans_param[t]);
         for (int e = 0; e < f.n_emis(); ++e) etp[e] = f.emis_param[e] < 0 ? -1 : (trimmed ? trimmed[f.emis_param[e]] : f.emis_param[e]);
-        make_type_blocks(A, ttp, etp, s->sc.rwords, s->sc.rgoff, s->sc.rgrows, s->sc.typeW, s->blocks);
+        const OverflowStrings ov{&f, alive.data(), cd->tokens, cd->offsets, cd->p, &s->sc.overflow};
+        make_type_blocks(A, ttp, etp, s->sc.rwords, s->sc.rgoff, s->sc.rgrows, s->sc.typeW, ov, s->blocks);
         // the evaluation does not need the blocks: a region type with too many paths leaves them out (zero blocks), not the shard
         if (!s->blocks.fail.empty()) { s->blocks = TypeBlocks(); blocks_omitted = 1; }
     }
